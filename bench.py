@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - LQR fwd+bwd solves/s (DiffLqr.apply + .backward) on B200, one JSON line.
 
-    python bench.py --gpus N --steps K --warmup W [--workload c5|c2|c3s] [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--workload c5|c2|c3s] [--impl reference] [--dump-outputs DIR]
 
 Metric (BASELINE.json): "LQR fwd+bwd solves/sec"; one solve = one batch element's full
 horizon through forward (Riccati + rollout) and the KKT-adjoint backward.
@@ -21,6 +21,9 @@ import threading
 import time
 
 import numpy as np
+
+# the benchmark may run from a read-only tree and must not leave __pycache__ in it
+sys.dont_write_bytecode = True
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 PKG = os.path.join(ROOT, "chainer-differentiable-mpc_b200")
@@ -209,6 +212,30 @@ def parity_vs_oracle(chunk, n, m, T, k=16):
             "oracle": "oracle/lqr.py (numpy restatement pinned to the live reference by tests/golden/make_golden.py)"}
 
 
+# --dump-outputs: what DiffLqr.apply (x, u) and .backward (dx0, dC, dc, dF, df) return to a caller -> batch axis
+LQR_OUTPUTS = {"x": 1, "u": 1, "dx0": 0, "dC": 1, "dc": 1, "dF": 1, "df": 1}
+DUMP_BYTES = 63 * 10 ** 6
+
+
+def dump_outputs(path, chunks, B):
+    """Writes the outputs the last timed step left in HBM to path/<name>.npy (float64), so that two builds can be
+    compared output for output.  The full outputs exceed DUMP_BYTES at most workloads (10 GB of dC alone at c5), so a
+    fixed seeded sample of batch elements is written, each with its whole horizon; the inputs are seeded too."""
+    import torch
+    os.makedirs(path, exist_ok=True)
+    Bc = chunks[0][1]["x"].shape[1]
+    per_elem = sum(chunks[0][1][k].numel() // Bc * 8 for k in LQR_OUTPUTS)
+    idx = np.sort(np.random.RandomState(0).choice(B, min(B, DUMP_BYTES // per_elem), replace=False))
+    for name, axis in LQR_OUTPUTS.items():
+        parts = []
+        for i, (_, out) in enumerate(chunks):
+            sel = idx[(idx >= i * Bc) & (idx < (i + 1) * Bc)] - i * Bc
+            if sel.size:
+                t = out[name].index_select(axis, torch.as_tensor(sel, device=out[name].device))
+                parts.append(t.cpu().numpy())
+        np.save(os.path.join(path, name + ".npy"), np.concatenate(parts, axis=axis))
+
+
 # ------------------------------------------------------------------------------------- CPU port timing
 def cpu_lqr_fwd_bwd(n, m, T, Bc, seed=0):
     """One DiffLqr.apply + .backward with the oracle port (numpy, all BLAS threads)."""
@@ -305,14 +332,14 @@ def run_reference_c1(args):
     ts = []
     with warnings.catch_warnings():
         warnings.simplefilter("ignore")
-        for _ in range(max(args.warmup, 1) + max(args.steps, 5)):
+        for _ in range(max(args.warmup, 1) + args.steps):
             t0 = time.perf_counter()
             ompc.step_forward(pr["C"], pr["c"], pr["F"], pr["f"], pr["x_nom"], pr["u"], pr["lo"], pr["hi"], (pr["C"], pr["c"]),
                               ("pendulum", (10.0, 1.0, 1.0)), 0.2, 5, n, m, need_expand=True, coupling="batch")
             ts.append(time.perf_counter() - t0)
     p50 = float(np.median(ts[max(args.warmup, 1):])) * 1e3
     emit({"impl": "reference", "metric": "mpc_step_p50_latency_ms", "value": p50, "unit": "ms", "n_gpus": args.gpus,
-          "steps": max(args.steps, 5), "warmup": max(args.warmup, 1), "ms_per_step": p50, "higher_is_better": False,
+          "steps": args.steps, "warmup": max(args.warmup, 1), "ms_per_step": p50, "higher_is_better": False,
           "scaling": "weak", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
           "config": {"workload": "c1", "desc": desc, "n_state": n, "n_ctrl": m, "T": T, "batch": B, "coupling": "batch"},
           "cpu_baseline": {"value": p50, "unit": "ms", "cores": 1, "kind": "port",
@@ -592,6 +619,8 @@ def run_b200(args):
     ms_step = ms_total / args.steps
     value = world * B / (ms_step * 1e-3)
     ok = all(bool(torch.isfinite(o["x"]).all().item() and torch.isfinite(o["dF"]).all().item()) for _, o in chunks)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, chunks, B)
     parity = None
     if rank == 0:
         try:
@@ -906,9 +935,10 @@ def run_e2e_shared(args, torch, ctx, n, m, T, world, dist, dev, rank):
                    "device, (T,B)-summed parameter gradients back (pinned host buffers, %d host worker threads)" % W}
 
 
-def mpc_step_latency(ctx, n_calls=200, cpu_calls=10, with_cpu=True, kernel_events=None):
+def mpc_step_latency(ctx, n_calls=200, cpu_calls=10, with_cpu=True, kernel_events=None, dump=None):
     """Second half of BASELINE's metric: batch-64 MPC-step p50 latency on the pendulum
-    (config 1: n=3, m=1, T=20, B=64, bounds +-2, as env_dx/il_exp.py wires it)."""
+    (config 1: n=3, m=1, T=20, B=64, bounds +-2, as env_dx/il_exp.py wires it).  With `dump`, the x, u the last
+    device-resident call computed (what MPCstep.apply returns) are written to dump/<name>.npy."""
     import _native
     from mpc_step import MPCstep
     from util import QuadCost
@@ -957,6 +987,10 @@ def mpc_step_latency(ctx, n_calls=200, cpu_calls=10, with_cpu=True, kernel_event
     ts = []
     for _ in range(n_calls):
         t0 = time.perf_counter(); dev_call(); ts.append(time.perf_counter() - t0)
+    if dump:
+        os.makedirs(dump, exist_ok=True)
+        for name in ("x", "u"):
+            np.save(os.path.join(dump, name + ".npy"), o[name].download())
     out = {"config": "c1 pendulum n=3 m=1 T=20 B=64 (one MPCstep.apply, need_expand, batch coupling)",
            "p50_ms": p50_facade, "p50_ms_device_resident": float(np.median(ts)) * 1e3, "calls": n_calls,
            "kernel": "mpc_forward_tpe_kernel" if os.environ.get("DMPC_MPC_GROUP") != "1" else "mpc_forward_kernel",
@@ -1016,7 +1050,8 @@ def run_c1(args):
         dist.init_process_group("nccl", device_id=dev)
     ctx = _native.Context(local)
     sampler = ClockSampler(local); sampler.start()
-    lat = mpc_step_latency(ctx, n_calls=max(200, args.steps), cpu_calls=10, with_cpu=(rank == 0 and not args.no_cpu), kernel_events=torch)
+    lat = mpc_step_latency(ctx, n_calls=args.steps, cpu_calls=10, with_cpu=(rank == 0 and not args.no_cpu), kernel_events=torch,
+                           dump=args.dump_outputs if rank == 0 else None)
     clocks = sampler.stop()
     vals = torch.tensor([lat["p50_ms_device_resident"], lat["p50_ms"], lat["kernel_ms"]], dtype=torch.float64, device=dev)
     if dist is not None:
@@ -1224,7 +1259,14 @@ def main():
     ap.add_argument("--chunks", type=int, default=1, help="sub-batches per GPU; >1 overlaps fwd(i+1) with bwd(i)")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-latency", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (seeded inputs, a fixed sample of the "
+                         "batch, under 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the CUDA path computed; the reference arm runs other inputs")
     if args.impl == "reference":
         run_reference(args)
     elif args.workload == "c1":

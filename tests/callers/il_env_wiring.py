@@ -1,8 +1,8 @@
 """How the reference's imitation-learning environment calls the solver (env_dx/il_env.py:104-158), restated in a few
-lines for boxes without /root/reference (the GPU box): the cost vectors q, p become chainer Variables broadcast to
+lines for runs without the original project at hand: the cost vectors q, p become chainer Variables broadcast to
 [T, B, 4, 4] / [T, B, 4] with util.chainer_diag + F.expand_dims + F.repeat, the solver is BoxDDP with the pendulum's own
 settings and float bounds, and the dynamics object is passed as is.  TEST INFRASTRUCTURE: tests/callers/run_callers.py uses
-the reference's unmodified il_env.py instead whenever /root/reference exists."""
+the reference's unmodified il_env.py instead when DIFFMPC_REFERENCE names a checkout of it."""
 from box_ddp import BoxDDP
 from chainer import functions as F
 from util import QuadCost, chainer_diag

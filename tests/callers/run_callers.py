@@ -4,10 +4,11 @@ under the forward-only Chainer stub and writes their results to an .npz.
 
     python tests/callers/run_callers.py OUT.npz
 
-sys.path order = [chainer stub, package dirs, (reference env_dx / mpc dirs when /root/reference exists)], so `box_ddp`,
-`mpc_step`, `util`, ... resolve to THIS package while `il_env`, `pendulum`, `mpc_net` are the reference's unmodified
-files when they are present (build container) and tests/callers' restatement / the package's own classes otherwise
-(GPU box).  The fixtures it is compared with come from the unmodified reference (tests/golden/make_golden_callers.py).
+sys.path order = [chainer stub, package dirs, (reference env_dx / mpc dirs when DIFFMPC_REFERENCE names a checkout of
+the original chainer-differentiable-mpc)], so `box_ddp`, `mpc_step`, `util`, ... resolve to THIS package while `il_env`,
+`pendulum`, `mpc_net` are the reference's unmodified files when that checkout is given and tests/callers' restatement /
+the package's own classes otherwise.  The fixtures it is compared with come from the unmodified reference
+(tests/golden/make_golden_callers.py).
 """
 import contextlib
 import io
@@ -22,8 +23,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 TESTS = os.path.dirname(HERE)
 ROOT = os.path.dirname(TESTS)
 PKG = os.path.join(ROOT, "chainer-differentiable-mpc_b200")
-REF = os.environ.get("DIFFMPC_REFERENCE", "/root/reference")
-USE_REF = os.path.isdir(os.path.join(REF, "env_dx")) and os.environ.get("DIFFMPC_NO_REFERENCE") != "1"
+REF = os.environ.get("DIFFMPC_REFERENCE", "")
+USE_REF = bool(REF) and os.path.isdir(os.path.join(REF, "env_dx")) and os.environ.get("DIFFMPC_NO_REFERENCE") != "1"
 
 sys.path[:0] = [os.path.join(TESTS, "_chainer_stub"), PKG, os.path.join(PKG, "lqr"), os.path.join(PKG, "mpc"),
                 os.path.join(PKG, "env_dx"), TESTS, HERE]

@@ -1,6 +1,7 @@
-"""Import the UNMODIFIED reference modules from /root/reference under the chainer stub.
+"""Import the UNMODIFIED reference modules under the chainer stub from the checkout of the original
+chainer-differentiable-mpc that DIFFMPC_REFERENCE names.
 
-Container-only helper (the GPU box has no /root/reference).  Used by
+Not part of the test suite.  Used by
 tests/golden/make_golden.py to produce the committed fixtures and to pin the
 numpy oracle (oracle/) against the live reference.
 
@@ -16,18 +17,18 @@ import sys
 
 import numpy as np
 
-REF = os.environ.get("DIFFMPC_REFERENCE", "/root/reference")
+REF = os.environ.get("DIFFMPC_REFERENCE", "")
 HERE = os.path.dirname(os.path.abspath(__file__))
 STUB = os.path.join(os.path.dirname(HERE), "_chainer_stub")
 
 
 def available():
-    return os.path.isdir(os.path.join(REF, "lqr"))
+    return bool(REF) and os.path.isdir(os.path.join(REF, "lqr"))
 
 
 def load(lu_fp32=True):
     """Returns a dict of the reference modules."""
-    assert available(), "reference not present"
+    assert available(), "set DIFFMPC_REFERENCE to a checkout of the original chainer-differentiable-mpc"
     for p in (STUB, REF, os.path.join(REF, "lqr"), os.path.join(REF, "mpc")):
         if p not in sys.path:
             sys.path.insert(0, p)

@@ -1,8 +1,8 @@
 #!/usr/bin/env python
 """Generate tests/golden/*.npz from the UNMODIFIED reference and pin the oracle to it.
 
-Run in the build container only (needs /root/reference):
-    python tests/golden/make_golden.py
+Needs a checkout of the original chainer-differentiable-mpc:
+    DIFFMPC_REFERENCE=<checkout> python tests/golden/make_golden.py
 
 For every case the reference modules (imported unmodified under
 tests/_chainer_stub, see _ref_loader.py) and the numpy oracle (oracle/) are run

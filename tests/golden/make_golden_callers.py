@@ -13,7 +13,7 @@ approximate.linearize_dynamics (n_state chainer.grad calls per step) is replaced
 linearisation of oracle/pendulum.py exactly as tests/golden/make_golden.py does (SURVEY.md H3), and the literal
 float32 lu_solve is replaced by the fp64-clean shim (SURVEY.md H1).
 
-    python tests/golden/make_golden_callers.py
+    DIFFMPC_REFERENCE=<checkout of the original chainer-differentiable-mpc> python tests/golden/make_golden_callers.py
 """
 import contextlib
 import io

@@ -5,6 +5,9 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 BASE_KEYS = {"metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling",
@@ -29,7 +32,26 @@ def test_reference_arm_runs_on_host_cores_and_prints_one_line():
     cb = d["cpu_baseline"]
     assert cb["kind"] == "port" and cb["cores"] >= 1 and cb["value"] == d["value"] and cb["sample"]
     assert d["e2e"] == {"value": d["value"], "unit": d["unit"], "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
-    assert d["config"]["workload"] == "c2"
+    assert d["config"]["workload"] == "c2" and d["steps"] == 1
+
+
+@pytest.mark.gpu
+def test_dump_outputs_writes_what_the_timed_steps_computed(tmp_path):
+    T, B, n, m = 50, 256, 4, 2
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "c2", "--batch", str(B), "--steps", "2",
+                          "--warmup", "1", "--no-cpu", "--no-latency", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert out.returncode == 0, out.stderr[-2000:]
+    d = _last_json_line(out.stdout)
+    assert d["steps"] == 2 and d["parity_max_rel"] < 1e-9
+    s = n + m
+    # 256 elements fit the size cap: the whole batch is written
+    shapes = {"x": (T, B, n), "u": (T, B, m), "dx0": (B, n), "dC": (T, B, s, s), "dc": (T, B, s), "dF": (T - 1, B, n, s),
+              "df": (T - 1, B, n)}
+    assert sorted(p.name for p in tmp_path.iterdir()) == sorted(k + ".npy" for k in shapes)
+    for name, shape in shapes.items():
+        a = np.load(tmp_path / (name + ".npy"))
+        assert a.dtype == np.float64 and a.shape == shape and np.isfinite(a).all(), name
 
 
 def test_b200_arm_refuses_to_run_without_a_gpu():

@@ -2,8 +2,8 @@
 
 tests/callers/run_callers.py (a child process with the forward-only Chainer stub first on sys.path) drives
   * IL_Env.mpc exactly as env_dx/il_env.py:94 (data generation) and env_dx/il_exp.py:249 (training step, warm start,
-    update_dynamics=False) do, B=64 - through the reference's own unmodified il_env.py + pendulum.py when /root/reference
-    exists, through the few-line restatement tests/callers/il_env_wiring.py on the GPU box - and the backward of the final
+    update_dynamics=False) do, B=64 - through the reference's own unmodified il_env.py + pendulum.py when DIFFMPC_REFERENCE
+    names a checkout of it, through the few-line restatement tests/callers/il_env_wiring.py otherwise - and the backward of the final
     MPCstep for the imitation loss, reduced to d loss / d q, d loss / d p;
   * MpcNet_dx.forward + backward as experiment_mpc/MpcNet.py:44-104 wires it.
 Results are compared with fixtures produced by the UNMODIFIED reference (tests/golden/make_golden_callers.py).
