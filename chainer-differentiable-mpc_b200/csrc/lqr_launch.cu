@@ -55,8 +55,8 @@ static bool lqr_tpe_enabled() {
 // elements per warp of the thread-per-element kernels (lqr_tpe_kernel.cuh).  32 is the measured default.
 // DMPC_LQR_TPE_EPW=auto spreads a small batch over thin warps (8 elements per warp up to B = 148 SMs x 4 schedulers x 8,
 // 16 up to twice that), which shortens each warp's operand staging (about 30 % of its instruction stream at config 2;
-// the recursion itself does not shrink); it is parity-checked on the GPU (profiles/tools/epw_check.py: 1.7e-12 against the oracle on four shapes) but the
-// round's GPU budget ended before it could be timed, so it stays opt-in.  DMPC_LQR_TPE_EPW=8|16|32 forces a value.
+// the recursion itself does not shrink); tests/test_gpu_dispatch_matrix.py checks every setting against the oracle, but it
+// has not been timed, so it stays opt-in.  DMPC_LQR_TPE_EPW=8|16|32 forces a value.
 static int tpe_elems_per_warp(int B) {
   static int forced = -2;
   if (forced == -2) {

@@ -54,8 +54,8 @@ __device__ __forceinline__ void tpe_solve(R (&H)[M][M], R (&X)[M][NC]) {
 // 3.2 cycles, `wait` the top stall, DRAM at 15 %, 1.6 % of the warp slots in use), and ~30 % of that stream is this
 // staging.  A batch that leaves most of the GPU's 592 warp schedulers idle anyway can be spread thinner - 16 or 8 elements
 // per warp, the other lanes shadow the last element - so that each warp stages half or a quarter as much; the recursion's
-// own instructions do not shrink, so the gain is bounded by ~1.3x.  Opt-in (DMPC_LQR_TPE_EPW, lqr_launch.cu):
-// parity-checked on the GPU, not yet timed.
+// own instructions do not shrink, so the gain is bounded by ~1.3x.  Opt-in (DMPC_LQR_TPE_EPW, lqr_launch.cu): checked
+// against the oracle by tests/test_gpu_dispatch_matrix.py, not yet timed.
 template <typename R>
 __device__ __forceinline__ void tpe_cp(R* sdst, const R* g) {
   if (sizeof(R) == 8) cp_async8(sdst, g); else cp_async4(sdst, g);

@@ -1,7 +1,7 @@
 """GPU, torch-free, ~3 s: the thread-per-element LQR kernels (csrc/lqr_tpe_kernel.cuh) launched with thin warps (8 / 16 elements
 per warp, DMPC_LQR_TPE_EPW=auto) against the oracle: forward + adjoint on four shapes, slices at both ends and in the middle of
-the batch.  Prints EPW_CHECK PASS|FAIL.  Run by tests/test_gpu_lqr.py::test_tpe_kernels_thin_warps in a subprocess (the
-launcher reads the variable once per process)."""
+the batch.  Prints EPW_CHECK PASS|FAIL.  A quick profiling-side check; the test suite covers the same shapes in
+tests/test_gpu_dispatch_matrix.py (setting epw_auto)."""
 import os, sys, time
 os.environ.setdefault("DMPC_LQR_TPE_EPW", "auto")
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))

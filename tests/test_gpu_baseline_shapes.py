@@ -85,42 +85,6 @@ def test_c5_T100_vs_oracle(ctx, B, dtype):
     assert not bad, (bad, errs)
 
 
-def _child_paths():
-    import os
-    here = os.path.dirname(os.path.abspath(__file__))
-    root = os.path.dirname(here)
-    pkg = os.path.join(root, "chainer-differentiable-mpc_b200")
-    return [root, pkg, os.path.join(pkg, "lqr"), os.path.join(pkg, "mpc"), here]
-
-
-def test_c5_T100_matches_generic_kernel(ctx):
-    """Same inputs through the generic shared-memory kernel (all four V terms kept, LU with back substitution) and
-    through the DMMA warp kernel: two independent CUDA implementations agree at T=100 (B=33, ragged)."""
-    import os
-    import subprocess
-    import sys
-    # DMPC_DISABLE_DMMA is read once per process -> run the generic path in a child process
-    T, B, n, m = 100, 33, 32, 8
-    code = (
-        "import sys, numpy as np; sys.path[:0]=%r; import _native; from _helpers import lqr_problem\n"
-        "ctx=_native.default_context(0); pr=lqr_problem(77,%d,%d,%d,%d)\n"
-        "d={k:ctx.to_device(pr[k]) for k in ('x0','C','c','F','f')}\n"
-        "x=ctx.empty((%d,%d,%d)); u=ctx.empty((%d,%d,%d)); K=ctx.empty((%d,%d,%d,%d)); k=ctx.empty((%d,%d,%d))\n"
-        "ctx.lqr_solve(np.float64,%d,%d,%d,%d,d['x0'],d['C'],d['c'],d['F'],%d,d['f'],x,u,K,k,None,3); ctx.sync()\n"
-        "np.savez(sys.argv[1], x=x.download(), u=u.download(), K=K.download(), k=k.download())\n"
-    ) % (_child_paths(), T, B, n, m, T, B, n, T, B, m, T, B, m, n, T, B, m, T, B, n, m, T - 1)
-    import tempfile
-    outs = {}
-    for mode in ("0", "1"):
-        with tempfile.NamedTemporaryFile(suffix=".npz") as tf:
-            env = dict(os.environ, DMPC_DISABLE_DMMA=mode)
-            subprocess.check_call([sys.executable, "-c", code, tf.name], env=env)
-            d = np.load(tf.name)
-            outs[mode] = {k: d[k] for k in d.files}
-    for k in ("x", "u", "K", "k"):
-        assert rel_err(outs["0"][k], outs["1"][k]) < 1e-10, k
-
-
 # ------------------------------------------------------------------------------------------------- config 2
 def test_c2_full_batch_slice_vs_oracle(ctx):
     """n=4, m=2, T=50, B=4096 (BASELINE config 2) fwd+bwd on the GPU at the full batch; the oracle solves a strided

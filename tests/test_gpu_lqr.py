@@ -131,20 +131,6 @@ def test_tpe_kernels_other_launch_geometries(ctx, B, n, m):
             assert rel_err(a[:, sl], b) < 1e-10, k
 
 
-def test_tpe_kernels_thin_warps():
-    """DMPC_LQR_TPE_EPW=auto (8 / 16 elements per warp for small batches, csrc/lqr_launch.cu) is read once per process, so the
-    check runs in its own: profiles/tools/epw_check.py compares forward + adjoint with the oracle on four shapes."""
-    import os
-    import subprocess
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    env = dict(os.environ, DMPC_LQR_TPE_EPW="auto")
-    r = subprocess.run([sys.executable, os.path.join(root, "profiles", "tools", "epw_check.py")], env=env, capture_output=True,
-                       text=True, timeout=300)
-    assert r.returncode == 0, r.stderr[-2000:]
-    assert "EPW_CHECK PASS" in r.stdout, r.stdout[-2000:]
-
-
 def test_factor_then_rollout_split(ctx):
     """LqrRecursion.backward() then .forward(Ks, ks) as two calls == solve_recursion()."""
     pr = lqr_problem(5, 15, 40, 4, 2)

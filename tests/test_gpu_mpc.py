@@ -63,7 +63,7 @@ def test_pnqp_batch_golden(ctx, name):
         assert rel_err(LU, g["Hf"]) < 1e-10
 
 
-@pytest.mark.parametrize("m,B", [(1, 300), (2, 257), (4, 1000), (6, 64), (8, 129), (12, 33)])
+@pytest.mark.parametrize("m,B", [(1, 300), (2, 257), (4, 1000), (6, 64), (8, 129), (12, 33), (20, 40), (32, 17)])
 def test_pnqp_random_vs_oracle(ctx, m, B):
     rs = np.random.RandomState(100 + m)
     L = rs.randn(B, m, m)
