@@ -597,7 +597,7 @@ __global__ void mpc_forward_kernel(MpcFwdParams<R> p) {
     {
       const bool worse = cost > old_cost;             // NaN -> accepted, as in the reference
       if (!worse) done = true;
-      else if (trial + 1 >= p.max_ls_trials) { status |= FLAG_LS_CAPPED; ++trial; done = true; }   // alpha stays the one of the
+      else if (trial + 1 >= p.max_ls_trials) { status |= FLAG_LS_CAPPED; done = true; }            // alpha stays the one of the
       else { alpha *= p.ls_decay; ++trial; }                                                        // trajectory just written
     }
   }

@@ -339,7 +339,7 @@ __global__ void __launch_bounds__(MAXT) mpc_forward_tpe_kernel(MpcFwdParams<R> p
     cost = cc;
   };
 
-  int trial = 0;                                            // index of the accepted candidate
+  int trial = 0;                                            // index of the accepted (or, capped, the last) candidate
   if (NA == 1) {
     bool done = false;
     while (!done) {
@@ -349,7 +349,6 @@ __global__ void __launch_bounds__(MAXT) mpc_forward_tpe_kernel(MpcFwdParams<R> p
       else if (trial + 1 >= p.max_ls_trials) { status |= FLAG_LS_CAPPED; done = true; }   // alpha = the one written
       else { alpha *= p.ls_decay; ++trial; }
     }
-    if (status & FLAG_LS_CAPPED) ++trial;
   } else {
     const unsigned full = 0xffffffffu;
     const int qbase = (threadIdx.x & 31) & ~(NA - 1);
@@ -393,7 +392,7 @@ __global__ void __launch_bounds__(MAXT) mpc_forward_tpe_kernel(MpcFwdParams<R> p
         }
       }
     }
-    trial = win + ((status & FLAG_LS_CAPPED) ? 1 : 0);
+    trial = win;
     cost = wcost; alpha = walpha;
   }
   if (writer) {

@@ -178,7 +178,8 @@ int dmpc_pnqp(dmpc_handle h, int dtype, int B, int m,
  * Outputs: d_x[T,B,n] d_u[T,B,m]; gains d_Ks[T,B,m,n] d_ks[T,B,m]; d_u_first[T,B,m] = controls of the
  * alpha=1 pass (for full_du_norm, :260-263); d_objs[T,B]; d_costs[B]; d_old_costs[B] (nullable);
  * d_alphas[B]; d_n_qp[T,B] int32 (1 + PNQP iterations); d_free[T,B,m] uint8; d_n_ls[B] int32
- * (line-search passes); d_flags[B] int32 (dmpc_elem_flag bits).
+ * (line-search passes run: the accepted pass, or max_ls_trials on an element whose line search hit the cap - that one
+ * carries DMPC_FLAG_LS_CAPPED and its alpha is the one of the last pass); d_flags[B] int32 (dmpc_elem_flag bits).
  * max_ls_trials caps the per-element line search (the reference's loop has no effective cap, Q5).
  */
 int dmpc_mpc_step_forward(dmpc_handle h, int dtype, int T, int B, int n, int m,

@@ -6,7 +6,8 @@ step_forward   follows mpc/mpc_step.py:288-328
 lqr_active     follows mpc/active_constrained_lqr.py:67-193
 step_backward  follows mpc/mpc_step.py:330-460
 
-`dynamics` is ('linear', F, f) or ('pendulum', params); `cost` is (C, c) (QuadCost).
+`dynamics` is ('linear', F, f) or ('pendulum', params[, dt, max_torque]) (PendulumDx: params = (g, m, l) or the
+non-`simple` (g, m, l, d, b); dt / max_torque default to 0.05 / 2.0); `cost` is (C, c) (QuadCost).
 """
 from collections import namedtuple
 
@@ -26,7 +27,7 @@ def dyn_step(dynamics, t, x, u):
         if f is not None:
             xn = xn + f[t]
         return xn
-    return _pend.step(x, u, dynamics[1])
+    return _pend.step(x, u, *dynamics[1:])
 
 
 def traj_cost(x, u, cost):
@@ -100,10 +101,33 @@ def backward_rec(C, c, F, f, u_nom, u_lower, u_upper, n, m, lu_fp32=False, coupl
     return Ks, ks, n_qp, free_all
 
 
+def ls_pass(Ks, ks, x_nom, u_nom, u_lower, u_upper, cost, dynamics, alphas):
+    """One line-search pass of forward_rec (mpc_step.py:198-253) at the per-element step lengths alphas[B]:
+    returns (new_x, new_u, objs[T,B], cost[B])."""
+    T = u_nom.shape[0]
+    C, c = cost
+    new_x = [x_nom[0]]
+    new_u = []
+    dx = [np.zeros_like(x_nom[0])]
+    objs = []
+    for t in range(T):
+        nu = bmv(Ks[t], dx[t]) + u_nom[t]
+        nu = nu + alphas[:, None] * ks[t]                             # :213-219 (diagflat(alphas) @ kt)
+        nu = clamp(nu, u_lower[t], u_upper[t])
+        new_u.append(nu)
+        tau = np.concatenate((new_x[t], nu), axis=1)
+        if t < T - 1:
+            xn = dyn_step(dynamics, t, new_x[t], nu)
+            new_x.append(xn)
+            dx.append(xn - x_nom[t + 1])
+        objs.append(0.5 * bquad(tau, C[t]) + bdot(tau, c[t]))         # :251
+    objs = np.stack(objs)
+    return np.stack(new_x), np.stack(new_u), objs, np.sum(objs, axis=0)
+
+
 def forward_rec(Ks, ks, x_nom, u_nom, u_lower, u_upper, cost, dynamics, ls_decay, max_ls_iter,
                 max_trials=200):
     T, B, m = u_nom.shape
-    C, c = cost
     alphas = np.ones(B, dtype=u_nom.dtype)
     old_cost = traj_cost(x_nom, u_nom, cost)                          # :191
     cur = None
@@ -111,25 +135,7 @@ def forward_rec(Ks, ks, x_nom, u_nom, u_lower, u_upper, cost, dynamics, ls_decay
     full_du_norm = None
     u_first = None
     while (n_iter < max_ls_iter and cur is None) or (cur is not None and (cur > old_cost).any()):   # :196 (Q5)
-        new_x = [x_nom[0]]
-        new_u = []
-        dx = [np.zeros_like(x_nom[0])]
-        objs = []
-        for t in range(T):
-            nu = bmv(Ks[t], dx[t]) + u_nom[t]
-            nu = nu + alphas[:, None] * ks[t]                         # :213-219 (diagflat(alphas) @ kt)
-            nu = clamp(nu, u_lower[t], u_upper[t])
-            new_u.append(nu)
-            tau = np.concatenate((new_x[t], nu), axis=1)
-            if t < T - 1:
-                xn = dyn_step(dynamics, t, new_x[t], nu)
-                new_x.append(xn)
-                dx.append(xn - x_nom[t + 1])
-            objs.append(0.5 * bquad(tau, C[t]) + bdot(tau, c[t]))     # :251
-        objs = np.stack(objs)
-        cur = np.sum(objs, axis=0)
-        new_x = np.stack(new_x)
-        new_u = np.stack(new_u)
+        new_x, new_u, objs, cur = ls_pass(Ks, ks, x_nom, u_nom, u_lower, u_upper, cost, dynamics, alphas)
         if full_du_norm is None:
             u_first = new_u.copy()
             full_du_norm = _scrambled_norm(u_nom - new_u, B, T, m)
@@ -143,9 +149,10 @@ def forward_rec(Ks, ks, x_nom, u_nom, u_lower, u_upper, cost, dynamics, ls_decay
 
 
 def step_forward(C, c, F, f, x_nom, u_nom, u_lower, u_upper, cost, dynamics, ls_decay, max_ls_iter,
-                 n, m, need_expand=True, lu_fp32=False, coupling="batch"):
+                 n, m, need_expand=True, lu_fp32=False, coupling="batch", max_trials=200):
     """mpc_step.py:288-328.  coupling='element' runs the reference control flow with
-    n_batch == 1 on every element (SURVEY.md H2) and re-assembles the batch."""
+    n_batch == 1 on every element (SURVEY.md H2) and re-assembles the batch.  max_trials caps the
+    line-search passes (forward_rec); n_ls = passes run (per element under 'element')."""
     T, B = C.shape[0], C.shape[1]
     if coupling == "element" and B > 1:
         outs = []
@@ -157,7 +164,7 @@ def step_forward(C, c, F, f, x_nom, u_nom, u_lower, u_upper, cost, dynamics, ls_
             outs.append(step_forward(C[:, sl], c[:, sl], F[:, sl], None if f is None else f[:, sl],
                                      x_nom[:, sl], u_nom[:, sl], u_lower[:, sl], u_upper[:, sl],
                                      (cost[0][:, sl], cost[1][:, sl]), dyn_b, ls_decay, max_ls_iter,
-                                     n, m, need_expand, lu_fp32, "batch"))
+                                     n, m, need_expand, lu_fp32, "batch", max_trials))
         x = np.concatenate([o[0] for o in outs], axis=1)
         u = np.concatenate([o[1] for o in outs], axis=1)
         u_first = np.concatenate([o[2].u_first for o in outs], axis=1)
@@ -179,7 +186,8 @@ def step_forward(C, c, F, f, x_nom, u_nom, u_lower, u_upper, cost, dynamics, ls_
     else:
         c_hat, f_hat = c, f
     Ks, ks, n_qp, free = backward_rec(C, c_hat, F, f_hat, u_nom, u_lower, u_upper, n, m, lu_fp32, "batch")
-    x, u, fo = forward_rec(Ks, ks, x_nom, u_nom, u_lower, u_upper, cost, dynamics, ls_decay, max_ls_iter)
+    x, u, fo = forward_rec(Ks, ks, x_nom, u_nom, u_lower, u_upper, cost, dynamics, ls_decay, max_ls_iter,
+                           max_trials)
     return x, u, fo, dict(Ks=Ks, ks=ks, n_qp=n_qp, free=free)
 
 

@@ -21,8 +21,18 @@ Launcher branch -> case that reaches it (kernel asserted from the profiler trace
   launch_lqr_dtau     tpe / specialised / runtime G         as above (adjoint of every lqr case)
   launch_adjoint_out  tpe (full) / specialised / runtime    as above; reduced: *-reduced*; adj_group
   launch_adjoint_fused + adjoint_fused_available            (32,8) full and reduced: *-pathdmma*, *-pathfused*; off: adj_unfused
-  launch_mpc_forward  tpe (m = 1) / specialised / runtime   default mpcf cases, mpc_group
+  launch_mpc_forward  tpe (m = 1) / specialised / runtime   default mpcf cases, mpc_group (linear and pendulum <3,1,4>)
   launch_mpc_tpe      4 lanes with / without stash, 1 lane   default mpcf (stash threshold asserted), mpc_no_spec, mpc_no_stash
+MPC step forward contract (mpcf keys, every kernel above in both couplings where the launcher has them):
+  true_cost           separate tC, tc buffers (the oracle asserts they change the line search); elements e % 5 == 2 capped
+  cap = 1 ... 6, 0    max_ls_trials (0 = 64): FLAG_LS_CAPPED exactly on the capped elements, n_ls = the cap, alpha of the
+                      last pass; every cap mod 4 with and without the stash (test_mpcf_four_lane_coverage)
+  decay = 0.7 / 0.9   true control gain 1 - 10 x the model's: winners on every lane and in later rounds of the 4-lane kernel
+  expand / f / FT     need_expand = 0 with the model f (and without: f = False); F with T rows
+  dyn = "pendulum"    g, m, l, dt = 0.03, max_torque = 1.5 off their defaults, bounds +-2 (the torque clip is active)
+Every mpcf case checks n_qp, free, alphas, n_ls and the capped flag bit-exact, x, u, Ks, ks, objs, u_first, costs and
+old costs against the oracle (1e-10; 1e-9 for element-coupled x, u), and that no decisive line-search comparison is within
+1e3 ulp of the old cost.
   launch_pnqp         SG = 32 (17 <= m <= 32), both couplings  default pnqp cases (SG 4 / 8 / 16: tests/test_gpu_mpc.py)
 Not reached here: batch-coupled launches spread over a thread-block cluster (tests/test_gpu_mpc.py covers them), the
 one-lane element-coupled MPC kernel at T >= 454 (an oracle run that long is slow), the m > 32 errors.
@@ -45,7 +55,7 @@ if __name__ == "__main__":                       # child process: the import pat
 
 import _native
 from _helpers import rel_err, lqr_problem, psd_cost, stable_dynamics
-from oracle import lqr as olqr, mpc as ompc, pnqp as opnqp
+from oracle import lqr as olqr, mpc as ompc, pendulum as opend, pnqp as opnqp
 
 pytestmark = pytest.mark.gpu
 
@@ -378,22 +388,68 @@ def tpe_stash(T, n, B, batch, itemsize=8):
     return 16 * ks <= kmax // 3
 
 
+PEND = ((9.5, 1.3, 0.8), 0.03, 1.5)      # PendulumDx (g, m, l), dt, max_torque: none at its default (10, 1, 1), 0.05, 2.0
+CAPPED = 5                               # true_cost: elements e % CAPPED == 2 are capped by construction
+
+
 def mpcf_problem(sp):
+    """Model (C, c, F, f) and true problem of one MPC step case.  Keys (all optional): gain = range of the true control
+    gain over the model's (linear dynamics); dyn = "pendulum" (true dynamics PEND, model = its linearisation at the
+    nominal point, bounds +-2 so that the torque clip at 1.5 is active); expand = False (need_expand = 0: the model c
+    is the Taylor-shifted C tau_nom + c and the model f enters the sweep); f = False (no model f); FT = True (F with T
+    rows, the last one junk); true_cost = True (a true cost that differs from the model's, and the elements
+    e % CAPPED == 2 get 0.5 beta |tau - tau_nom|^2, which every alpha > 0 increases: capped by construction)."""
     T, B, n, m = sp["T"], sp["B"], sp["n"], sp["m"]
     rs = np.random.RandomState(sp["seed"])
     s = n + m
     C, c = psd_cost(rs, T, B, s)
-    bound = 0.5
-    F = stable_dynamics(rs, T, B, n, m, per_t=False)
-    f = 0.1 * rs.randn(T - 1, B, n)
-    tF = F.copy()
-    # the true control gain is 1.5 - 3.5 times the model's: the full step overshoots and the line search picks a shorter one
-    tF[..., n:] *= 1.5 + 2.0 * rs.rand(1, B, 1, 1)
-    x0 = rs.randn(B, n)
-    u_nom = np.clip(0.2 * rs.randn(T, B, m), -bound, bound)
-    x_nom = ompc.get_traj(x0, u_nom, ("linear", tF, f))
-    return dict(C=C, c=c, F=F, f=f, tF=tF, dyn=("linear", tF, f), x_nom=x_nom, u_nom=u_nom,
-                lo=np.full((T, B, m), -bound), hi=np.full((T, B, m), bound))
+    if sp.get("dyn") == "pendulum":
+        assert (n, m) == (3, 1)
+        bound = 2.0
+        th = rs.uniform(-np.pi, np.pi, B)
+        x0 = np.stack((np.cos(th), np.sin(th), 0.5 * rs.randn(B)), axis=1)
+        u_nom = np.clip(1.2 * rs.randn(T, B, m), -bound, bound)
+        dyn = ("pendulum",) + PEND
+        x_nom = ompc.get_traj(x0, u_nom, dyn)
+        F, f = opend.linearize(x0, u_nom, *PEND)
+        tF = None
+        assert ((np.abs(u_nom) > PEND[2]) & (np.abs(u_nom) < bound)).any()
+    else:
+        bound = 0.5
+        F = stable_dynamics(rs, T, B, n, m, per_t=False)
+        f = 0.1 * rs.randn(T - 1, B, n)
+        tF = F.copy()
+        # the true control gain is a multiple of the model's: the full step overshoots and the line search picks a
+        # shorter one (the default 1.5 - 3.5 times; 1 - 10 times spreads the accepted trial over 1 ... 8 at decay 0.7)
+        glo, ghi = sp.get("gain", (1.5, 3.5))
+        tF[..., n:] *= glo + (ghi - glo) * rs.rand(1, B, 1, 1)
+        x0 = rs.randn(B, n)
+        u_nom = np.clip(0.2 * rs.randn(T, B, m), -bound, bound)
+        dyn = ("linear", tF, f)
+        x_nom = ompc.get_traj(x0, u_nom, dyn)
+    tC, tc = C, c
+    capped = np.zeros(B, dtype=bool)
+    if sp.get("true_cost"):
+        tC, tc = psd_cost(rs, T, B, s)
+        tC, tc = 0.5 * (tC + C), 0.5 * (tc + c)
+        capped = np.arange(B) % CAPPED == 2
+        beta = 2.0
+        tau = np.concatenate((x_nom, u_nom), axis=2)
+        tC[:, capped] = beta * np.eye(s)
+        tc[:, capped] = -beta * tau[:, capped]
+    cm, fm = c, f
+    if not sp.get("expand", True):
+        cm = np.einsum("tbij,tbj->tbi", C, np.concatenate((x_nom, u_nom), axis=2)) + c
+        fm = 0.3 * f
+    if not sp.get("f", True):
+        fm = None
+    Fm = np.concatenate((F, 1e3 * rs.randn(1, B, n, s))) if sp.get("FT") else F
+    return dict(C=C, c=cm, F=Fm, f=fm, tC=tC, tc=tc, tF=tF, tf=None if tF is None else f, dyn=dyn, x_nom=x_nom,
+                u_nom=u_nom, lo=np.full((T, B, m), -bound), hi=np.full((T, B, m), bound), capped=capped)
+
+
+def mpcf_cap(sp):
+    return sp.get("cap", 64) or 64          # max_ls_trials = 0 means 64
 
 
 def run_mpcf(ctx, sp):
@@ -401,44 +457,112 @@ def run_mpcf(ctx, sp):
     T, B, n, m = sp["T"], sp["B"], sp["n"], sp["m"]
     npd = np.float64
     b = Bufs(sp.get("off", 0))
-    d = {k: b.put(pr[k], npd) for k in ("C", "c", "F", "f", "tF", "x_nom", "u_nom", "lo", "hi")}
+    d = {k: b.put(pr[k], npd) for k in ("C", "c", "F", "f", "tF", "tf", "x_nom", "u_nom", "lo", "hi") if pr[k] is not None}
+    for k, km in (("tC", "C"), ("tc", "c")):             # the true cost aliases the model's where it is the same array
+        d[k] = d[km] if pr[k] is pr[km] else b.put(pr[k], npd)
     o = dict(x=b.empty((T, B, n), npd), u=b.empty((T, B, m), npd), Ks=b.empty((T, B, m, n), npd), ks=b.empty((T, B, m), npd),
              u_first=b.empty((T, B, m), npd), objs=b.empty((T, B), npd), costs=b.empty((B,), npd), old=b.empty((B,), npd),
              alphas=b.empty((B,), npd), n_qp=b.empty((T, B), np.int32), free=b.empty((T, B, m), np.uint8),
              n_ls=b.empty((B,), np.int32), flags=b.empty((B,), np.int32))
     b.ready()
     coupling = _native.COUPLING_BATCH if sp["batch"] else _native.COUPLING_ELEMENT
+    if sp.get("dyn") == "pendulum":
+        dyn, dynp = _native.DYN_PENDULUM, PEND[0] + PEND[1:]
+    else:
+        dyn, dynp = _native.DYN_LINEAR, None
 
     def go():
-        ctx.mpc_step_forward(npd, T, B, n, m, d["C"], d["c"], d["F"], T - 1, d["f"], d["x_nom"], d["u_nom"], d["lo"], d["hi"],
-                             d["C"], d["c"], _native.DYN_LINEAR, d["tF"], d["f"], None, 0.2, 64, True, coupling, o["x"], o["u"], o["Ks"], o["ks"], o["u_first"],
-                             o["objs"], o["costs"], o["old"], o["alphas"], o["n_qp"], o["free"], o["n_ls"], o["flags"])
+        ctx.mpc_step_forward(npd, T, B, n, m, d["C"], d["c"], d["F"], pr["F"].shape[0], d.get("f"), d["x_nom"], d["u_nom"],
+                             d["lo"], d["hi"], d["tC"], d["tc"], dyn, d.get("tF"), d.get("tf"), dynp,
+                             sp.get("decay", 0.2), sp.get("cap", 64), sp.get("expand", True), coupling, o["x"], o["u"],
+                             o["Ks"], o["ks"], o["u_first"], o["objs"], o["costs"], o["old"], o["alphas"], o["n_qp"],
+                             o["free"], o["n_ls"], o["flags"])
     _, names = profiled(ctx, go)
     return {k: v.get() for k, v in o.items()}, names
 
 
-def check_mpcf(sp, out, names):
+def _pow(decay, k):
+    a = 1.0
+    for _ in range(k):                       # the line search's repeated multiplication, bit for bit
+        a *= decay
+    return a
+
+
+_MPCF_EXPECT = {}
+
+
+def mpcf_expect(sp):
+    """The oracle's step (line search capped at the case's max_ls_trials) and what each output must be, with the checks
+    that make the case discriminating: every decisive line-search comparison clears ~1e3 ulp of the old cost, and a
+    separate true cost changes the oracle's alphas."""
+    key = (case_id(sp), sp["seed"], sp.get("gain"))
+    if key in _MPCF_EXPECT:
+        return _MPCF_EXPECT[key]
     pr = mpcf_problem(sp)
+    T, B, n, m = sp["T"], sp["B"], sp["n"], sp["m"]
+    decay, cap = sp.get("decay", 0.2), mpcf_cap(sp)
+    coupling = "batch" if sp["batch"] else "element"
+
+    def oracle(cost):
+        with warnings.catch_warnings():
+            warnings.simplefilter("ignore")
+            return ompc.step_forward(pr["C"], pr["c"], pr["F"], pr["f"], pr["x_nom"], pr["u_nom"], pr["lo"], pr["hi"],
+                                     cost, pr["dyn"], decay, 10, n, m, need_expand=sp.get("expand", True),
+                                     coupling=coupling, max_trials=cap)
+    cost = (pr["tC"], pr["tc"])
+    ox, ou, fo, aux = oracle(cost)
+    old = ompc.traj_cost(pr["x_nom"], pr["u_nom"], cost)
+    capped = fo.costs > old
+    assert np.array_equal(capped[pr["capped"]], np.ones(pr["capped"].sum(), bool)), "a capped-by-construction element accepted"
+    # passes per element: decays of the oracle's alpha + 1 (a capped element's alpha has one decay more than its last pass)
+    n_ls = np.zeros(B, dtype=np.int64)
+    for e in range(B):
+        k = 0
+        while _pow(decay, k) != fo.alphas[e]:
+            k += 1
+            assert k <= cap, (e, fo.alphas[e])
+        n_ls[e] = cap if capped[e] else k + 1
+    assert (n_ls[capped] == cap).all() and (n_ls <= cap).all()
+    if not sp["batch"]:
+        assert np.array_equal(n_ls, fo.n_ls), (n_ls, fo.n_ls)           # the per-element recursion counts the same
+    alphas = fo.alphas.copy()
+    alphas[capped] = _pow(decay, cap - 1)                              # the alpha of the trajectory the last pass wrote
+    assert (alphas[capped] * decay == fo.alphas[capped]).all()
+    # margins: pass k of element e compares the cost at decay^k with the old cost
+    for k in range(int(n_ls.max())):
+        al = np.full(B, _pow(decay, k))
+        *_, cur = ompc.ls_pass(aux["Ks"], aux["ks"], pr["x_nom"], pr["u_nom"], pr["lo"], pr["hi"], cost, pr["dyn"], al)
+        live = k < n_ls
+        margin = np.abs(cur - old) / np.spacing(np.abs(old))
+        assert (margin[live] > 1e3).all(), ("line-search comparison near a tie", k, margin[live].min())
+        assert ((cur > old) == ((k < n_ls - 1) | capped))[live].all(), k
+    if sp.get("true_cost"):
+        assert (oracle((pr["C"], pr["c"]))[2].alphas != fo.alphas).any(), "the true cost does not change the line search"
+    want = dict(x=ox, u=ou, Ks=aux["Ks"], ks=aux["ks"], objs=fo.objs, u_first=fo.u_first, costs=fo.costs, old=old,
+                alphas=alphas, n_qp=aux["n_qp"], free=aux["free"], n_ls=n_ls, capped=capped)
+    _MPCF_EXPECT[key] = want
+    return want
+
+
+def check_mpcf(sp, out, names):
     T, B, n, m = sp["T"], sp["B"], sp["n"], sp["m"]
     assert_kernels(names, sp["expect"], absent=sp.get("absent", ()))
     if "stash" in sp:
         assert tpe_stash(T, n, B, sp["batch"]) == sp["stash"], (T, n, B, tpe_stash(T, n, B, sp["batch"]))
-    with warnings.catch_warnings():
-        warnings.simplefilter("ignore")
-        ox, ou, fo, aux = ompc.step_forward(pr["C"], pr["c"], pr["F"], pr["f"], pr["x_nom"], pr["u_nom"], pr["lo"], pr["hi"],
-                                            (pr["C"], pr["c"]), pr["dyn"], 0.2, 10, n, m, need_expand=True,
-                                            coupling="batch" if sp["batch"] else "element")
-    assert np.array_equal(out["n_qp"], aux["n_qp"])
-    assert np.array_equal(out["free"].astype(float), aux["free"])
-    assert np.array_equal(out["alphas"], fo.alphas)
+    w = mpcf_expect(sp)
+    assert np.array_equal(out["n_qp"], w["n_qp"])
+    assert np.array_equal(out["free"].astype(float), w["free"])
+    assert np.array_equal(out["alphas"], w["alphas"]), (out["alphas"], w["alphas"])
+    assert np.array_equal(out["n_ls"], w["n_ls"]), ("n_ls", out["n_ls"], w["n_ls"])
+    assert np.array_equal((out["flags"] & _native.FLAG_LS_CAPPED) != 0, w["capped"]), (out["flags"], w["capped"])
+    assert not (out["flags"] & ~_native.FLAG_LS_CAPPED).any(), out["flags"]
     if sp.get("line_search"):
-        assert (fo.alphas < 1).any(), "no element took a shortened step: the candidate selection is not exercised"
-        assert fo.alphas.min() > 1e-6, "an element found no descent: its line search ends on a rounding-level tie"
+        assert (w["alphas"] < 1).any(), "no element took a shortened step: the candidate selection is not exercised"
+        assert w["alphas"].min() > 1e-6, "an element found no descent: its line search ends on a rounding-level tie"
     tx = 1e-10 if sp["batch"] else 1e-9
-    assert rel_err(out["Ks"], aux["Ks"]) < 1e-10 and rel_err(out["ks"], aux["ks"]) < 1e-10
-    assert rel_err(out["x"], ox) < tx and rel_err(out["u"], ou) < tx
-    assert rel_err(out["costs"], fo.costs) < 1e-10
-    assert not out["flags"].any()
+    for k in ("Ks", "ks", "objs", "u_first", "costs", "old"):
+        assert rel_err(out[k], w[k]) < 1e-10, (k, rel_err(out[k], w[k]))
+    assert rel_err(out["x"], w["x"]) < tx and rel_err(out["u"], w["u"]) < tx, (rel_err(out["x"], w["x"]), rel_err(out["u"], w["u"]))
 
 
 # ------------------------------------------------------------------------------------------------ PNQP
@@ -484,11 +608,34 @@ def L(T, B, n, m, dt, path, G=None, **kw):
     return dict(op="lqr", T=T, B=B, n=n, m=m, dt=dt, path=path, G=G, seed=kw.pop("seed", T * 1009 + B * 7 + n * 3 + m), **kw)
 
 
+def MF(T, B, n, m, batch, seed, expect, **kw):
+    """An MPC step forward case; the cases with a line-search decay of their own spread the true control gain over 1 - 10
+    times the model's."""
+    if "decay" in kw and kw.get("dyn") != "pendulum":
+        kw.setdefault("gain", (1.0, 10.0))
+    return dict(op="mpcf", T=T, B=B, n=n, m=m, batch=batch, seed=seed, expect=[expect], **kw)
+
+
+def TPE(n, batch, NA):
+    return "mpc_forward_tpe_kernel<double, %d, %s, 256, %d>" % (n, "true" if batch else "false", NA)
+
+
+def GRP(N, M, G, batch):
+    return "mpc_forward_kernel<double, %d, %d, %d, %s>" % (N, M, G, "true" if batch else "false")
+
+
 def case_id(sp):
     bits = [sp["op"], "T%d" % sp.get("T", 1), "B%d" % sp["B"], "n%dm%d" % (sp["n"], sp["m"]), sp.get("dt", F64)]
-    for k in ("path", "pivot", "off", "reduced", "batch"):
+    for k in ("path", "pivot", "off", "reduced", "batch", "dyn", "true_cost", "decay"):
         if sp.get(k) not in (None, False, 0):
             bits.append(k if sp[k] is True else "%s%s" % (k, sp[k]))
+    for k, v in (("expand", False), ("f", False)):
+        if sp.get(k, True) is v:
+            bits.append("no" + k)
+    if sp.get("FT"):
+        bits.append("FT")
+    if "cap" in sp:
+        bits.append("cap%d" % sp["cap"])
     return "-".join(str(b) for b in bits)
 
 
@@ -531,6 +678,36 @@ DEFAULT = [
     # runtime-shape group MPC kernel with m > n, and the MPC step on misaligned buffers
     dict(op="mpcf", T=8, B=9, n=2, m=3, batch=False, seed=65, expect=["mpc_forward_kernel<double, 0, 0, 8, false>"]),
     dict(op="mpcf", T=8, B=21, n=4, m=2, batch=False, seed=66, off=1, expect=["mpc_forward_kernel<double, 4, 2, 8, false>"]),
+    # MPC step forward, the whole contract: a separate true cost (with elements capped by construction), the line-search
+    # cap (max_ls_trials 1 ... 6 and 0 = 64, every residue mod 4 with and without the stash), decays 0.7 / 0.9 (the
+    # accepted trial spreads over the four candidate lanes and later rounds), need_expand = 0 with / without the model f,
+    # F with T rows, and the pendulum at non-default g, m, l, dt, max_torque.  Four lanes, stash:
+    MF(20, 16, 3, 1, False, 143, TPE(3, False, 4), stash=True, true_cost=True, decay=0.7, cap=1),
+    MF(20, 24, 3, 1, True, 102, TPE(3, True, 4), stash=True, true_cost=True, decay=0.7, cap=2, expand=False),
+    MF(20, 16, 2, 1, False, 103, TPE(2, False, 4), stash=True, true_cost=True, decay=0.7, cap=3),
+    MF(20, 16, 2, 1, True, 104, TPE(2, True, 4), stash=True, true_cost=True, decay=0.9, cap=0),
+    MF(20, 16, 3, 1, False, 105, TPE(3, False, 4), stash=True, true_cost=True, decay=0.9, cap=0, dyn="pendulum"),
+    MF(20, 20, 3, 1, True, 106, TPE(3, True, 4), stash=True, true_cost=True, decay=0.7, cap=6, dyn="pendulum"),
+    # four lanes, no stash
+    MF(40, 16, 3, 1, False, 107, TPE(3, False, 4), stash=False, true_cost=True, decay=0.7, cap=5),
+    MF(30, 64, 3, 1, True, 108, TPE(3, True, 4), stash=False, true_cost=True, decay=0.7, cap=6),
+    MF(45, 16, 2, 1, False, 109, TPE(2, False, 4), stash=False, true_cost=True, decay=0.9, cap=0, expand=False),
+    MF(32, 64, 2, 1, True, 110, TPE(2, True, 4), stash=False, true_cost=True, decay=0.7, cap=3, FT=True),
+    MF(40, 16, 3, 1, False, 111, TPE(3, False, 4), stash=False, true_cost=True, decay=0.7, cap=4, expand=False, f=False),
+    # one lane per element (batch coupling past 64 elements)
+    MF(20, 100, 3, 1, True, 112, TPE(3, True, 1), stash=None, true_cost=True, decay=0.7, cap=5),
+    # group kernels: specialised <4,2,8> <8,4,16>, runtime shape G = 8 / 16 / 32 / 256, both couplings
+    MF(8, 21, 4, 2, True, 113, GRP(4, 2, 8, True), true_cost=True, decay=0.7, cap=3),
+    MF(8, 21, 4, 2, False, 114, GRP(4, 2, 8, False), true_cost=True, decay=0.9, cap=0, expand=False, f=False, FT=True),
+    MF(6, 10, 8, 4, False, 115, GRP(8, 4, 16, False), true_cost=True, decay=0.9, cap=0),
+    MF(6, 10, 8, 4, True, 116, GRP(8, 4, 16, True), true_cost=True, decay=0.7, cap=5, expand=False),
+    MF(8, 9, 2, 3, False, 117, GRP(0, 0, 8, False), true_cost=True, decay=0.7, cap=2, expand=False, FT=True),
+    MF(8, 9, 2, 3, True, 118, GRP(0, 0, 8, True), true_cost=True, decay=0.9, cap=0),
+    MF(6, 9, 6, 5, False, 119, GRP(0, 0, 16, False), true_cost=True, decay=0.7, cap=4),
+    MF(6, 9, 6, 5, True, 120, GRP(0, 0, 16, True), true_cost=True, decay=0.7, cap=6, expand=False),
+    MF(5, 7, 12, 6, False, 121, GRP(0, 0, 32, False), true_cost=True, decay=0.9, cap=0, expand=False, f=False),
+    MF(5, 7, 12, 6, True, 122, GRP(0, 0, 32, True), true_cost=True, decay=0.7, cap=3),
+    MF(6, 3, 32, 8, False, 123, GRP(0, 0, 256, False), true_cost=True, decay=0.7, cap=4, expand=False),
     # PNQP with 17 <= m <= 32: 32 lanes per element
     dict(op="pnqp", B=40, n=0, m=20, batch=False, seed=91, expect=["pnqp_kernel<double, 0, 32, false>"]),
     dict(op="pnqp", B=17, n=0, m=32, batch=False, seed=92, expect=["pnqp_kernel<double, 0, 32, false>"]),
@@ -571,14 +748,22 @@ CHILD = {
     "adj_unfused": (dict(DMPC_ADJ_UNFUSED="1"), [L(8, 21, 32, 8, F64, "unfused", 256, reduced=True)]),
     "mpc_group": (dict(DMPC_MPC_GROUP="1"),
                   [dict(_M1_BATCH, op="mpcf", expect=["mpc_forward_kernel<double, 3, 1, 4, true>"]),
-                   dict(_M1_ELEM, op="mpcf", expect=["mpc_forward_kernel<double, 3, 1, 4, false>"])]),
+                   dict(_M1_ELEM, op="mpcf", expect=["mpc_forward_kernel<double, 3, 1, 4, false>"]),
+                   MF(20, 16, 3, 1, False, 131, GRP(3, 1, 4, False), true_cost=True, decay=0.7, cap=5, dyn="pendulum"),
+                   MF(20, 20, 3, 1, True, 132, GRP(3, 1, 4, True), true_cost=True, decay=0.9, cap=0, dyn="pendulum"),
+                   MF(20, 24, 3, 1, True, 133, GRP(3, 1, 4, True), true_cost=True, decay=0.7, cap=2, expand=False)]),
     "mpc_no_spec": (dict(DMPC_MPC_NO_SPEC="1"),
                     [dict(_M1_BATCH, op="mpcf", expect=["mpc_forward_tpe_kernel<double, 3, true, 256, 1>"]),
-                     dict(_M1_ELEM, op="mpcf", expect=["mpc_forward_tpe_kernel<double, 3, false, 256, 1>"])]),
+                     dict(_M1_ELEM, op="mpcf", expect=["mpc_forward_tpe_kernel<double, 3, false, 256, 1>"]),
+                     MF(20, 16, 3, 1, False, 134, TPE(3, False, 1), true_cost=True, decay=0.7, cap=3, dyn="pendulum"),
+                     MF(20, 24, 2, 1, True, 135, TPE(2, True, 1), true_cost=True, decay=0.9, cap=0, expand=False)]),
     # the default launch would stash at these horizons (stash=True); the switch turns the stash off, same kernel
     "mpc_no_stash": (dict(DMPC_MPC_NO_STASH="1"),
                      [dict(_M1_BATCH, op="mpcf", stash=True, expect=["mpc_forward_tpe_kernel<double, 3, true, 256, 4>"]),
-                      dict(_M1_ELEM, op="mpcf", stash=True, expect=["mpc_forward_tpe_kernel<double, 3, false, 256, 4>"])]),
+                      dict(_M1_ELEM, op="mpcf", stash=True, expect=["mpc_forward_tpe_kernel<double, 3, false, 256, 4>"]),
+                      MF(20, 16, 3, 1, False, 136, TPE(3, False, 4), stash=True, true_cost=True, decay=0.7, cap=3),
+                      MF(20, 24, 3, 1, True, 137, TPE(3, True, 4), stash=True, true_cost=True, decay=0.9, cap=0,
+                         dyn="pendulum")]),
 }
 
 
@@ -620,6 +805,24 @@ def test_ab_switch(setting, sp):
     out = {k[len(cid):]: v for k, v in res.items() if k.startswith(cid)}
     names = list(out.pop("__kernels__"))
     CHECK[sp["op"]](sp, out, names)
+
+
+def test_mpcf_four_lane_coverage():
+    """Together, the cases of the four-lane MPC kernel (mpc_forward_tpe_kernel<..., 4>) have winners on every candidate
+    lane (n_ls mod 4) and in a later round, and line-search caps at every residue mod 4 (the capped winner's lane is
+    (cap - 1) mod 4), both with the candidate stash and without it.  From the oracle."""
+    lanes, late, caps = set(), False, {True: set(), False: set()}
+    for setting, sp in [(None, sp) for sp in DEFAULT] + [(s, sp) for s, (_, cs) in CHILD.items() for sp in cs]:
+        if sp["op"] != "mpcf" or not any(k.startswith("mpc_forward_tpe_kernel") and k.endswith(", 4>") for k in sp["expect"]):
+            continue
+        w = mpcf_expect(sp)
+        won = w["n_ls"][~w["capped"]]
+        lanes |= set((won - 1) % 4)
+        late |= bool((won > 4).any())
+        if w["capped"].any():
+            caps[bool(sp["stash"]) and setting != "mpc_no_stash"].add(mpcf_cap(sp) % 4)
+    assert lanes == {0, 1, 2, 3} and late, (lanes, late)
+    assert caps[True] == {0, 1, 2, 3} and caps[False] == {0, 1, 2, 3}, caps
 
 
 def _child_main(setting, path):

@@ -216,20 +216,26 @@ def test_get_traj_linear_and_pendulum(ctx):
                  ctx.to_device(f), None, x)
     ctx.sync()
     assert rel_err(x.download(), want) < 1e-12
-    # pendulum (env_dx/pendulum.py:65-102) + analytic linearisation
+    # pendulum (env_dx/pendulum.py:65-102) + analytic linearisation: the reference's parameters, (g, m, l, dt,
+    # max_torque) none at its default (the controls reach 7: the torque clip at 1.5 and at 2.0 are both active), and
+    # dt <= 0 / max_torque <= 0, which mean the defaults 0.05 / 2.0
     g = load_golden("pendulum_step")
     B = g["x"].shape[0]
     T = 6
     u = np.repeat(g["u"][None], T, axis=0) * np.linspace(0.2, 1.0, T)[:, None, None]
-    want = ompc.get_traj(g["x"], u, ("pendulum", (10.0, 1.0, 1.0)))
-    wF, wf = opend.linearize(g["x"], u)
-    x = ctx.empty((T, B, 3)); Fo = ctx.empty((T - 1, B, 3, 4)); fo = ctx.empty((T - 1, B, 3))
-    ctx.get_traj(np.float64, T, B, 3, 1, _native.DYN_PENDULUM, ctx.to_device(g["x"]), ctx.to_device(u), None, None,
-                 (10.0, 1.0, 1.0), x, Fo, fo)
-    ctx.sync()
-    assert rel_err(x.download()[1], g["xn"] if False else want[1]) < 1e-13
-    assert rel_err(x.download(), want) < 1e-12
-    assert rel_err(Fo.download(), wF) < 1e-12 and rel_err(fo.download(), wf) < 1e-11
+    assert ((np.abs(u) > 1.5) & (np.abs(u) < 2.0)).any()
+    for dev, par, dt, maxu in (((10.0, 1.0, 1.0), (10.0, 1.0, 1.0), 0.05, 2.0),
+                               ((9.5, 1.3, 0.8, 0.03, 1.5), (9.5, 1.3, 0.8), 0.03, 1.5),
+                               ((9.5, 1.3, 0.8, 0.0, -1.0), (9.5, 1.3, 0.8), 0.05, 2.0)):
+        want = ompc.get_traj(g["x"], u, ("pendulum", par, dt, maxu))
+        wF, wf = opend.linearize(g["x"], u, par, dt, maxu)
+        x = ctx.empty((T, B, 3)); Fo = ctx.empty((T - 1, B, 3, 4)); fo = ctx.empty((T - 1, B, 3))
+        ctx.get_traj(np.float64, T, B, 3, 1, _native.DYN_PENDULUM, ctx.to_device(g["x"]), ctx.to_device(u), None, None,
+                     dev, x, Fo, fo)
+        ctx.sync()
+        assert rel_err(x.download()[1], want[1]) < 1e-13, dev
+        assert rel_err(x.download(), want) < 1e-12, dev
+        assert rel_err(Fo.download(), wF) < 1e-12 and rel_err(fo.download(), wf) < 1e-11, dev
 
 
 def test_bad_bounds_are_reported_through_the_c_abi(ctx):
