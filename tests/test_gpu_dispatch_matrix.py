@@ -35,7 +35,9 @@ old costs against the oracle (1e-10; 1e-9 for element-coupled x, u), and that no
 1e3 ulp of the old cost.
   launch_pnqp         SG = 32 (17 <= m <= 32), both couplings  default pnqp cases (SG 4 / 8 / 16: tests/test_gpu_mpc.py)
 Not reached here: batch-coupled launches spread over a thread-block cluster (tests/test_gpu_mpc.py covers them), the
-one-lane element-coupled MPC kernel at T >= 454 (an oracle run that long is slow), the m > 32 errors.
+one-lane element-coupled MPC kernel at T >= 454 (an oracle run that long is slow), the m > 32 errors.  The MPC step
+backward (full and reduced, every kernel and A/B setting it can select, non-symmetric C, F with T rows, gx or gu NULL,
+the active-set band) is in tests/test_gpu_mpc_backward_matrix.py; the mpcb cases here are its default-path subset.
 """
 import os
 import subprocess
