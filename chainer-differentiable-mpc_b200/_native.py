@@ -61,6 +61,10 @@ SIGNATURES = {
     "dmpc_reduced_grad_elems": (_sz, [_i, _i]),
     "dmpc_lqr_adjoint_reduced": (_i, [_vp, _i, _i, _i, _i, _i] + [_vp] * 13 + [_i, _vp]),
     "dmpc_mpc_step_backward_reduced": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _i] + [_vp] * 13 + [_vp]),
+    "dmpc_lqr_shared_workspace_bytes": (_i, [_i, _i, _i, _i, _i, ctypes.POINTER(_sz)]),
+    "dmpc_lqr_solve_shared": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "dmpc_lqr_adjoint_shared": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _sz]
+                                + [_vp] * 5 + [_i, _vp]),
     "dmpc_boxddp_workspace_bytes": (_i, [_i, _i, _i, _i, _i, ctypes.POINTER(_sz)]),
     "dmpc_boxddp_solve": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _i, _vp, _i, _vp, ctypes.POINTER(_d), _vp,
                                _vp, _vp, _sz] + [_vp] * 7 + [ctypes.POINTER(_i)] * 3 + [_vp]),
@@ -396,6 +400,24 @@ class Context:
         self._check(self.lib.dmpc_lqr_adjoint(self.h, dtype_code(dtype), T, B, n, m, _p(C), _p(c), _p(F), _p(x), _p(u),
                                               _p(gx), _p(gu), _p(Ks), _p(fac), _p(dx0), _p(dC), _p(dc), _p(dF),
                                               _p(df), flags, stream))
+
+    def lqr_shared_workspace_bytes(self, dtype, T, B, n, m):
+        need = _sz(0)
+        self._check(self.lib.dmpc_lqr_shared_workspace_bytes(dtype_code(dtype), T, B, n, m, ctypes.byref(need)))
+        return int(need.value)
+
+    def lqr_solve_shared(self, dtype, T, B, n, m, x0, C, c, F, F_T, f, x, u, ws, ws_bytes=None, stream=None):
+        """C [T,s,s] and F [F_T,n,s] shared by the batch; ws of lqr_shared_workspace_bytes() bytes."""
+        ws_bytes = ws.nbytes if ws_bytes is None else ws_bytes
+        self._check(self.lib.dmpc_lqr_solve_shared(self.h, dtype_code(dtype), T, B, n, m, _p(x0), _p(C), _p(c), _p(F),
+                                                   int(F_T), _p(f), _p(x), _p(u), _p(ws), int(ws_bytes), stream))
+
+    def lqr_adjoint_shared(self, dtype, T, B, n, m, C, c, F, F_T, x, u, gx, gu, ws, dx0, dC, dc, dF, df,
+                           flags=ADJ_STRICT_REFERENCE, ws_bytes=None, stream=None):
+        ws_bytes = ws.nbytes if ws_bytes is None else ws_bytes
+        self._check(self.lib.dmpc_lqr_adjoint_shared(
+            self.h, dtype_code(dtype), T, B, n, m, _p(C), _p(c), _p(F), int(F_T), _p(x), _p(u), _p(gx), _p(gu), _p(ws),
+            int(ws_bytes), _p(dx0), _p(dC), _p(dc), _p(dF), _p(df), flags, stream))
 
     def pnqp(self, dtype, B, m, H, q, lower, upper, x_init, x, LU, piv, free, iters, flags=None, n_iter=20,
              coupling=COUPLING_ELEMENT, stream=None):

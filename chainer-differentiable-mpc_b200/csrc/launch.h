@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include "lqr_kernels.cuh"
 #include "lqr_adjoint_fused.cuh"
+#include "lqr_shared_kernels.cuh"
 
 namespace dmpc {
 
@@ -22,6 +23,9 @@ template <typename R> int launch_lqr_dtau(const DtauParams<R>& p, cudaStream_t s
 template <typename R> int launch_adjoint_fused(const DtauParams<R>& d, const AdjFusedParams<R>& a, int stage, cudaStream_t st, long long* nlaunch);
 template <typename R> int launch_adjoint_out(const AdjOutParams<R>& p, cudaStream_t st, long long* nlaunch);
 template <typename R> int launch_expand_time_batch(const R* src, R* dst, int count, size_t total, cudaStream_t st, long long* nlaunch);
+// C and F shared by the batch (lqr_shared_launch.cu): the chunked vector sweeps + rollout; the adjoint + reduction
+template <typename R> int launch_lqr_shared_fwd(const LqrSharedParams<R>& p, cudaStream_t st, long long* nlaunch);
+template <typename R> int launch_lqr_shared_adj(const LqrSharedParams<R>& p, cudaStream_t st, long long* nlaunch);
 template <typename R> int launch_reduce_partials(const R* red, int B, int rsz, R* out, cudaStream_t st, long long* nlaunch);
 
 constexpr int kMaxSmem = 227 * 1024;

@@ -1,0 +1,40 @@
+// Launches of the shared-parameter LQR kernels (lqr_shared_kernels.cuh).  Compiled once per dtype (-DDMPC_REAL).
+#include "launch.h"
+
+#ifndef DMPC_REAL
+#define DMPC_REAL double
+#endif
+
+namespace dmpc {
+
+template <typename K, typename P>
+static int shared_launch(K kernel, const P& p, size_t smem, cudaStream_t st, long long* nl) {
+  if (cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return DMPC_ERR_CUDA;
+  kernel<<<(p.B + p.NB - 1) / p.NB, kSharedThreads, smem, st>>>(p);
+  if (nl) ++*nl;
+  return cudaGetLastError() == cudaSuccess ? DMPC_OK : DMPC_ERR_CUDA;
+}
+
+template <typename R>
+int launch_lqr_shared_fwd(const LqrSharedParams<R>& p, cudaStream_t st, long long* nl) {
+  const size_t smem = (size_t)SharedFwdLayout(p.n, p.m, p.NB).total * sizeof(R);
+  return shared_launch(lqr_shared_fwd_kernel<R>, p, smem, st, nl);
+}
+
+template <typename R>
+int launch_lqr_shared_adj(const LqrSharedParams<R>& p, cudaStream_t st, long long* nl) {
+  const size_t smem = (size_t)SharedAdjLayout(p.n, p.m, p.NB).total * sizeof(R);
+  int rc = shared_launch(lqr_shared_adj_kernel<R>, p, smem, st, nl);
+  if (rc) return rc;
+  const int s = p.n + p.m;
+  const size_t total = (size_t)p.T * s * s + (p.dF ? (size_t)p.F_T * p.n * s : 0);
+  const int tpb = 256;
+  lqr_shared_reduce_kernel<R><<<(unsigned)((total + tpb - 1) / tpb), tpb, 0, st>>>(p, (p.B + p.NB - 1) / p.NB);
+  if (nl) ++*nl;
+  return cudaGetLastError() == cudaSuccess ? DMPC_OK : DMPC_ERR_CUDA;
+}
+
+template int launch_lqr_shared_fwd<DMPC_REAL>(const LqrSharedParams<DMPC_REAL>&, cudaStream_t, long long*);
+template int launch_lqr_shared_adj<DMPC_REAL>(const LqrSharedParams<DMPC_REAL>&, cudaStream_t, long long*);
+
+}  // namespace dmpc

@@ -178,6 +178,93 @@ class DiffLqr(FunctionNodeBase):
         return tuple(wrap(g) for g in self.backward_numpy(gx, gu))
 
 
+class DiffLqrShared(FunctionNodeBase):
+    """`DiffLqrShared(T, n_batch, n_state, n_ctrl).apply((x_init, C, c, F, f)) -> (x, u)` for a batch that shares its
+    cost and dynamics matrices: C [T,s,s] and F [T-1 or T,n,s] are one block per time step; x_init [B,n], c [T,B,s] and
+    f [T-1,B,n] (or None) are per element.  Same results as DiffLqr on the broadcast tensors; `backward` returns the
+    gradients in the shapes of the inputs, dC and dF summed over the batch (dmpc_lqr_solve_shared / _adjoint_shared:
+    one Riccati sweep for the whole batch)."""
+
+    def __init__(self, T, n_batch, n_state, n_ctrl, device=0, dtype=np.float64, strict_reference=True, context=None):
+        super().__init__()
+        self.T, self.n_batch, self.n_state, self.n_ctrl = int(T), int(n_batch), int(n_state), int(n_ctrl)
+        self.n_sc = self.n_state + self.n_ctrl
+        self.dtype = np.dtype(dtype)
+        self.strict_reference = strict_reference
+        self._ctx = context if context is not None else _native.default_context(device)
+        self._d = None
+        self._F_T = None
+        self._have_f = False
+
+    def _buffers(self):
+        if self._d is None:
+            T, B, n, m, s, dt, ctx = self.T, self.n_batch, self.n_state, self.n_ctrl, self.n_sc, self.dtype, self._ctx
+            Tm = max(T - 1, 1)
+            shapes = dict(x0=(B, n), C=(T, s, s), c=(T, B, s), F=(T, n, s), f=(Tm, B, n), x=(T, B, n), u=(T, B, m),
+                          gx=(T, B, n), gu=(T, B, m), dx0=(B, n), dC=(T, s, s), dc=(T, B, s), dF=(T, n, s), df=(Tm, B, n),
+                          ws=(ctx.lqr_shared_workspace_bytes(dt, T, B, n, m),))
+            self._d = {k: ctx.empty(v, np.uint8 if k == "ws" else dt) for k, v in shapes.items()}
+        return self._d
+
+    def apply_numpy(self, x_init, C, c, large_f, f=None):
+        T, B, n, m, s, dt = self.T, self.n_batch, self.n_state, self.n_ctrl, self.n_sc, self.dtype
+        x_init, C, c, F = as_f(x_init, dt), as_f(C, dt), as_f(c, dt), as_f(large_f, dt)
+        assert list(x_init.shape) == [B, n]
+        assert list(C.shape) == [T, s, s], "C dim mismatch"
+        assert list(c.shape) == [T, B, s], "c dim mismatch"
+        assert F.shape[0] in (T - 1, T) and list(F.shape[1:]) == [n, s], "F dim mismatch"
+        self._have_f = f is not None and to_xp(f) is not None and T > 1
+        if self._have_f:
+            f = as_f(f, dt)
+            assert list(f.shape) == [T - 1, B, n], " f dim mismatch"
+        self._F_T = F.shape[0]
+        d = self._buffers()
+        ctx = self._ctx
+        d["x0"].upload(x_init); d["C"].upload(C); d["c"].upload(c)
+        Fp = np.zeros((T, n, s), dt)                    # the device buffer has room for F_T = T rows
+        Fp[:self._F_T] = F
+        d["F"].upload(Fp)
+        if self._have_f:
+            d["f"].upload(f)
+        ctx.lqr_solve_shared(dt, T, B, n, m, d["x0"], d["C"], d["c"], d["F"], self._F_T,
+                             d["f"] if self._have_f else None, d["x"], d["u"], d["ws"])
+        x = d["x"].download(sync=False)
+        u = d["u"].download()
+        return x, u
+
+    def backward_numpy(self, grad_x, grad_u):
+        """-> (dx0 [B,n], dC [T,s,s], dc [T,B,s], dF [F_T,n,s], df [T-1,B,n] or None)."""
+        T, B, n, m, s, dt = self.T, self.n_batch, self.n_state, self.n_ctrl, self.n_sc, self.dtype
+        d = self._buffers()
+        ctx = self._ctx
+        gx = None if grad_x is None else d["gx"].upload(as_f(grad_x, dt))
+        gu = None if grad_u is None else d["gu"].upload(as_f(grad_u, dt))
+        ctx.lqr_adjoint_shared(dt, T, B, n, m, d["C"], d["c"], d["F"], self._F_T, d["x"], d["u"], gx, gu, d["ws"],
+                               d["dx0"], d["dC"], d["dc"], d["dF"], d["df"] if self._have_f else None,
+                               _native.ADJ_STRICT_REFERENCE if self.strict_reference else 0)
+        dx0 = d["dx0"].download(sync=False)
+        dC = d["dC"].download(sync=False)
+        dc = d["dc"].download(sync=False)
+        df = d["df"].download(sync=False)[:T - 1] if self._have_f else None
+        dF = d["dF"].download()[:self._F_T]
+        return dx0, dC, dc, dF, df
+
+    # ---- Chainer FunctionNode protocol -------------------------------------------------------
+    def check_type_forward(self, in_types):
+        pass
+
+    def forward(self, inputs):
+        x_init, C, c, large_f, f = inputs
+        self.retain_inputs((0, 1, 2, 3))
+        x, u = self.apply_numpy(x_init, C, c, large_f, f)
+        self.retain_outputs((0, 1))
+        return x, u
+
+    def backward(self, target_input_indexes, grad_outputs):
+        gx, gu = grad_outputs
+        return tuple(None if g is None else wrap(g) for g in self.backward_numpy(to_xp(gx), to_xp(gu)))
+
+
 from _compat import NetLinkBase, Parameter  # noqa: E402
 from util import expand_time_batch  # noqa: E402
 

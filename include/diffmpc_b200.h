@@ -144,6 +144,41 @@ int dmpc_lqr_adjoint(dmpc_handle h, int dtype, int T, int B, int n, int m,
                      int flags, void* stream);
 
 
+/* ---- LQR with C and F shared by the batch (DiffLqr, lqr/differentiable_lqr.py:65-142, on a batch whose C_t, F_t are the
+ *      same for every element: LqrNet / LqrNet_cost_dx, differentiable_lqr.py:186-198, 237-248) --------------------- */
+/*
+ * Shapes: d_C[T,s,s] and d_F[F_T,n,s] (F_T in {T-1, T}; row T-1 is not read) are ONE block per time step, shared by all B
+ * elements; everything per element keeps the reference layout: d_x0[B,n] d_c[T,B,s] d_f[T-1,B,n] (NULL = None)
+ * d_x[T,B,n] d_u[T,B,m].  Results equal dmpc_lqr_solve / dmpc_lqr_adjoint on the broadcast tensors, with the shared
+ * gradients summed over the batch.  C need not be symmetric.
+ * The workspace (dmpc_lqr_shared_workspace_bytes, any alignment) holds the matrices of the one Riccati sweep the whole
+ * batch needs (K_t, Quu_t^-1, Qxu_t, V_t: a few KB to ~100 KB) and the per-chunk partial sums of the adjoint; its size
+ * depends on (dtype, T, B, n, m).  m > 32 and shapes too large for the chunk kernels: DMPC_ERR_UNSUPPORTED.
+ */
+int dmpc_lqr_shared_workspace_bytes(int dtype, int T, int B, int n, int m, size_t* bytes);
+
+/*
+ * LqrRecursion.solve_recursion (lqr_recursion.py:202-209) for the shared batch: the Riccati sweep (:69-158) runs once, at
+ * B = 1, and leaves its matrices in d_ws; the per-element vector sweep (k_t, v_t: :85-120, :152) and the rollout
+ * (:160-200) run for the whole batch.  Writes d_x, d_u (and d_ws, which dmpc_lqr_adjoint_shared reads).
+ */
+int dmpc_lqr_solve_shared(dmpc_handle h, int dtype, int T, int B, int n, int m,
+                          const void* d_x0, const void* d_C, const void* d_c, const void* d_F, int F_T, const void* d_f,
+                          void* d_x, void* d_u, void* d_ws, size_t ws_bytes, void* stream);
+
+/*
+ * DiffLqr.backward (differentiable_lqr.py:78-142) for the shared batch.  Needs d_ws of a dmpc_lqr_solve_shared call on the
+ * same C, F, and its d_x, d_u.  d_gx[T,B,n], d_gu[T,B,m] may be NULL (zeros).
+ * Outputs: per element d_dx0[B,n] d_dc[T,B,s] d_df[T-1,B,n] (nullable); shared d_dC[T,s,s] = sum_b dC_b (:128) and
+ * d_dF[F_T,n,s] = sum_b dF_b (:130-131; row T-1 zero when F_T == T), summed in a fixed order (deterministic).
+ * DMPC_ADJ_STRICT_REFERENCE reproduces quirks Q1 and Q2 as dmpc_lqr_adjoint does.
+ */
+int dmpc_lqr_adjoint_shared(dmpc_handle h, int dtype, int T, int B, int n, int m,
+                            const void* d_C, const void* d_c, const void* d_F, int F_T,
+                            const void* d_x, const void* d_u, const void* d_gx, const void* d_gu,
+                            void* d_ws, size_t ws_bytes,
+                            void* d_dx0, void* d_dC, void* d_dc, void* d_dF, void* d_df, int flags, void* stream);
+
 /* ---- PNQP (replaces PNQP, mpc/pnqp.py:37-201) ---------------------------------------------- */
 /*
  * Batched projected-Newton box QP: min 0.5 x^T H x + q^T x  s.t. lower <= x <= upper.
