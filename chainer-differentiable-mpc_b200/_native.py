@@ -20,6 +20,7 @@ F64, F32 = 0, 1
 LQR_FACTOR, LQR_ROLLOUT, LQR_SAVE_FAC = 1, 2, 4
 ADJ_STRICT_REFERENCE = 1
 ADJ_STAGE_DTAU_ONLY, ADJ_STAGE_OUT_ONLY = 2, 4
+SHARE_C = 1
 COUPLING_ELEMENT, COUPLING_BATCH = 0, 1
 DYN_LINEAR, DYN_PENDULUM = 0, 1
 FLAG_QP_NOT_CONVERGED, FLAG_NONFINITE, FLAG_LS_CAPPED, FLAG_BAD_BOUNDS = 1, 2, 4, 8
@@ -65,6 +66,11 @@ SIGNATURES = {
     "dmpc_lqr_solve_shared": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
     "dmpc_lqr_adjoint_shared": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _sz]
                                 + [_vp] * 5 + [_i, _vp]),
+    "dmpc_lqr_shared_workspace_bytes_ex": (_i, [_i, _i, _i, _i, _i, _i, ctypes.POINTER(_sz)]),
+    "dmpc_lqr_solve_shared_ex": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _sz, _i,
+                                      _vp]),
+    "dmpc_lqr_adjoint_shared_ex": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _sz]
+                                   + [_vp] * 5 + [_i, _i, _vp]),
     "dmpc_boxddp_workspace_bytes": (_i, [_i, _i, _i, _i, _i, ctypes.POINTER(_sz)]),
     "dmpc_boxddp_solve": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _i, _vp, _i, _vp, ctypes.POINTER(_d), _vp,
                                _vp, _vp, _sz] + [_vp] * 7 + [ctypes.POINTER(_i)] * 3 + [_vp]),
@@ -401,23 +407,37 @@ class Context:
                                               _p(gx), _p(gu), _p(Ks), _p(fac), _p(dx0), _p(dC), _p(dc), _p(dF),
                                               _p(df), flags, stream))
 
-    def lqr_shared_workspace_bytes(self, dtype, T, B, n, m):
+    def lqr_shared_workspace_bytes(self, dtype, T, B, n, m, share=None):
+        """share=None: the original entry point; an int (0 or SHARE_C): dmpc_lqr_shared_workspace_bytes_ex."""
         need = _sz(0)
-        self._check(self.lib.dmpc_lqr_shared_workspace_bytes(dtype_code(dtype), T, B, n, m, ctypes.byref(need)))
+        if share is None:
+            self._check(self.lib.dmpc_lqr_shared_workspace_bytes(dtype_code(dtype), T, B, n, m, ctypes.byref(need)))
+        else:
+            self._check(self.lib.dmpc_lqr_shared_workspace_bytes_ex(dtype_code(dtype), T, B, n, m, int(share),
+                                                                    ctypes.byref(need)))
         return int(need.value)
 
-    def lqr_solve_shared(self, dtype, T, B, n, m, x0, C, c, F, F_T, f, x, u, ws, ws_bytes=None, stream=None):
-        """C [T,s,s] and F [F_T,n,s] shared by the batch; ws of lqr_shared_workspace_bytes() bytes."""
+    def lqr_solve_shared(self, dtype, T, B, n, m, x0, C, c, F, F_T, f, x, u, ws, ws_bytes=None, stream=None, share=None):
+        """C [T,s,s] and F [F_T,n,s] shared by the batch (and c [T,s] with share=SHARE_C); ws of
+        lqr_shared_workspace_bytes(..., share) bytes.  share=None calls the original entry point."""
         ws_bytes = ws.nbytes if ws_bytes is None else ws_bytes
-        self._check(self.lib.dmpc_lqr_solve_shared(self.h, dtype_code(dtype), T, B, n, m, _p(x0), _p(C), _p(c), _p(F),
-                                                   int(F_T), _p(f), _p(x), _p(u), _p(ws), int(ws_bytes), stream))
+        a = (self.h, dtype_code(dtype), T, B, n, m, _p(x0), _p(C), _p(c), _p(F), int(F_T), _p(f), _p(x), _p(u), _p(ws),
+             int(ws_bytes))
+        if share is None:
+            self._check(self.lib.dmpc_lqr_solve_shared(*a, stream))
+        else:
+            self._check(self.lib.dmpc_lqr_solve_shared_ex(*a, int(share), stream))
 
     def lqr_adjoint_shared(self, dtype, T, B, n, m, C, c, F, F_T, x, u, gx, gu, ws, dx0, dC, dc, dF, df,
-                           flags=ADJ_STRICT_REFERENCE, ws_bytes=None, stream=None):
+                           flags=ADJ_STRICT_REFERENCE, ws_bytes=None, stream=None, share=None):
+        """share=SHARE_C: c [T,s], dc [T,s] summed over the batch (or None).  share=None: the original entry point."""
         ws_bytes = ws.nbytes if ws_bytes is None else ws_bytes
-        self._check(self.lib.dmpc_lqr_adjoint_shared(
-            self.h, dtype_code(dtype), T, B, n, m, _p(C), _p(c), _p(F), int(F_T), _p(x), _p(u), _p(gx), _p(gu), _p(ws),
-            int(ws_bytes), _p(dx0), _p(dC), _p(dc), _p(dF), _p(df), flags, stream))
+        a = (self.h, dtype_code(dtype), T, B, n, m, _p(C), _p(c), _p(F), int(F_T), _p(x), _p(u), _p(gx), _p(gu), _p(ws),
+             int(ws_bytes), _p(dx0), _p(dC), _p(dc), _p(dF), _p(df), flags)
+        if share is None:
+            self._check(self.lib.dmpc_lqr_adjoint_shared(*a, stream))
+        else:
+            self._check(self.lib.dmpc_lqr_adjoint_shared_ex(*a, int(share), stream))
 
     def pnqp(self, dtype, B, m, H, q, lower, upper, x_init, x, LU, piv, free, iters, flags=None, n_iter=20,
              coupling=COUPLING_ELEMENT, stream=None):

@@ -347,18 +347,22 @@ static int boxddp_impl(dmpc_handle h, int dtype, int T, int B, int n, int m, con
 
 // ------------------------------------------------------------------------------------------------
 // C and F shared by the batch (lqr_shared_kernels.cuh).  Workspace: the zero c block and outputs of the B = 1 Riccati
-// sweep (K_t, k_t, Quu_t^-1 | Qxu_t, V_t | v_t), then one partial record [T][s*s + n*s] per chunk of elements.  The caller's
-// pointer is rounded up to 256 bytes first, so the sweep's 16-byte copies never depend on the caller's alignment.
+// sweep (K_t, k_t, Quu_t^-1 | Qxu_t, V_t | v_t), then one partial record [T][s*s + n*s] per chunk of elements; with
+// DMPC_SHARE_C the records carry sum_b dtau_t as well ([T][s*s + n*s + s]) and a [T,B,s] region follows, where the adjoint
+// parks k' and dtau between its sweeps (dc being [T,s]).  The caller's pointer is rounded up to 256 bytes first, so the
+// sweep's 16-byte copies never depend on the caller's alignment.
 namespace {
-struct SharedWs { size_t c0, Ks, ks, fac, V, part, total; int NB, nchunk; };
-inline SharedWs shared_ws(size_t w, int T, int B, int n, int m) {
+struct SharedWs { size_t c0, Ks, ks, fac, V, part, park, total; int NB, nchunk; };
+inline SharedWs shared_ws(size_t w, int T, int B, int n, int m, int share) {
   SharedWs L; size_t o = 0;
   const size_t s = (size_t)(n + m);
+  const bool c_shared = (share & DMPC_SHARE_C) != 0;
   L.NB = lqr_shared_chunk(w, B, n, m, kMaxSmem);
   L.nchunk = L.NB ? (B + L.NB - 1) / L.NB : 0;
   auto take = [&](size_t bytes) { size_t at = o; o = al256(o + bytes); return at; };
   L.c0 = take(w * T * s); L.Ks = take(w * T * m * n); L.ks = take(w * T * m); L.fac = take(w * T * fac_elems_per_step(n, m));
-  L.V = take(w * T * (size_t)(n * n + n)); L.part = take(w * (size_t)L.nchunk * T * (s * s + n * s));
+  L.V = take(w * T * (size_t)(n * n + n)); L.part = take(w * (size_t)L.nchunk * T * shared_rec_elems(n, m, c_shared));
+  L.park = c_shared ? take(w * (size_t)T * B * s) : 0;
   L.total = o + 256;
   return L;
 }
@@ -367,22 +371,25 @@ inline char* ws_base(void* ws) { return (char*)al256((size_t)ws); }
 
 template <typename R>
 static int lqr_solve_shared_impl(dmpc_handle h, int T, int B, int n, int m, const void* x0, const void* C, const void* c,
-                                 const void* F, int F_T, const void* f, void* x, void* u, void* ws, cudaStream_t st) {
-  const SharedWs W = shared_ws(sizeof(R), T, B, n, m);
+                                 const void* F, int F_T, const void* f, void* x, void* u, void* ws, int share,
+                                 cudaStream_t st) {
+  const SharedWs W = shared_ws(sizeof(R), T, B, n, m, share);
+  const bool c_shared = (share & DMPC_SHARE_C) != 0, roll_only = c_shared && !f;
   char* w = ws_base(ws);
-  CK(cudaMemsetAsync(w + W.c0, 0, sizeof(R) * (size_t)T * (n + m), st));
+  // The sweep runs on a zero c unless c is shared and f is None: then its k_t is every element's k_t.
+  if (!roll_only) CK(cudaMemsetAsync(w + W.c0, 0, sizeof(R) * (size_t)T * (n + m), st));
   LqrParams<R> p;                                    // the matrix sweep: the existing Riccati kernels at B = 1
   memset(&p, 0, sizeof(p));
   p.T = T; p.B = 1; p.n = n; p.m = m; p.flags = LQR_DO_FACTOR | LQR_SAVE_FAC;
-  p.C = (const R*)C; p.c = (const R*)(w + W.c0); p.F = (const R*)F; p.c_scale = R(1);
+  p.C = (const R*)C; p.c = roll_only ? (const R*)c : (const R*)(w + W.c0); p.F = (const R*)F; p.c_scale = R(1);
   p.Ks = (R*)(w + W.Ks); p.ks = (R*)(w + W.ks); p.fac = (R*)(w + W.fac); p.Vsave = (R*)(w + W.V);
   int rc = launch_lqr_solve<R>(p, st, &h->launches);
   if (rc) return fail(h, rc, rc == DMPC_ERR_UNSUPPORTED ? "lqr_solve_shared: no Riccati kernel for this shape" : "lqr_solve_shared: sweep launch failed");
   LqrSharedParams<R> q;
   memset(&q, 0, sizeof(q));
-  q.T = T; q.B = B; q.n = n; q.m = m; q.F_T = F_T; q.NB = W.NB;
+  q.T = T; q.B = B; q.n = n; q.m = m; q.F_T = F_T; q.NB = W.NB; q.c_shared = c_shared;
   q.x0 = (const R*)x0; q.C = (const R*)C; q.c = (const R*)c; q.F = (const R*)F; q.f = (const R*)f;
-  q.Ks = p.Ks; q.fac = p.fac; q.Vsave = p.Vsave; q.x = (R*)x; q.u = (R*)u;
+  q.Ks = p.Ks; q.ks = p.ks; q.fac = p.fac; q.Vsave = p.Vsave; q.x = (R*)x; q.u = (R*)u;
   rc = launch_lqr_shared_fwd<R>(q, st, &h->launches);
   if (rc) h->err = "lqr_solve_shared launch failed";
   return rc;
@@ -391,17 +398,20 @@ static int lqr_solve_shared_impl(dmpc_handle h, int T, int B, int n, int m, cons
 template <typename R>
 static int lqr_adjoint_shared_impl(dmpc_handle h, int T, int B, int n, int m, const void* C, const void* c, const void* F,
                                    int F_T, const void* x, const void* u, const void* gx, const void* gu, void* ws,
-                                   void* dx0, void* dC, void* dc, void* dF, void* df, int flags, cudaStream_t st) {
-  const SharedWs W = shared_ws(sizeof(R), T, B, n, m);
+                                   void* dx0, void* dC, void* dc, void* dF, void* df, int flags, int share,
+                                   cudaStream_t st) {
+  const SharedWs W = shared_ws(sizeof(R), T, B, n, m, share);
+  const bool c_shared = (share & DMPC_SHARE_C) != 0;
   char* w = ws_base(ws);
   LqrSharedParams<R> q;
   memset(&q, 0, sizeof(q));
-  q.T = T; q.B = B; q.n = n; q.m = m; q.F_T = F_T; q.NB = W.NB;
+  q.T = T; q.B = B; q.n = n; q.m = m; q.F_T = F_T; q.NB = W.NB; q.c_shared = c_shared;
   q.flags = (flags & DMPC_ADJ_STRICT_REFERENCE) ? (ADJ_QUIRK_DC | ADJ_QUIRK_DF) : 0;
   q.C = (const R*)C; q.c = (const R*)c; q.F = (const R*)F;
   q.Ks = (const R*)(w + W.Ks); q.fac = (const R*)(w + W.fac); q.Vsave = (const R*)(w + W.V);
   q.x = (R*)x; q.u = (R*)u; q.gx = (const R*)gx; q.gu = (const R*)gu;
   q.dx0 = (R*)dx0; q.dc = (R*)dc; q.df = T > 1 ? (R*)df : nullptr; q.part = (R*)(w + W.part); q.dC = (R*)dC;
+  q.park = c_shared ? (R*)(w + W.park) : (R*)dc;
   q.dF = F_T > 0 ? (R*)dF : nullptr;
   const int rc = launch_lqr_shared_adj<R>(q, st, &h->launches);
   if (rc) h->err = "lqr_adjoint_shared launch failed";
@@ -735,54 +745,74 @@ int dmpc_mpc_step_backward_reduced(dmpc_handle h, int dtype, int T, int B, int n
   return fail(h, DMPC_ERR_UNSUPPORTED, "dtype");
 }
 
-int dmpc_lqr_shared_workspace_bytes(int dtype, int T, int B, int n, int m, size_t* bytes) {
+int dmpc_lqr_shared_workspace_bytes_ex(int dtype, int T, int B, int n, int m, int share, size_t* bytes) {
   if (!bytes || T < 1 || B < 1 || n < 1 || m < 1) return DMPC_ERR_BAD_SHAPE;
   if (dtype != DMPC_F64 && dtype != DMPC_F32) return DMPC_ERR_UNSUPPORTED;
-  if (m > 32) return DMPC_ERR_UNSUPPORTED;
-  const SharedWs W = shared_ws(dtype == DMPC_F64 ? 8 : 4, T, B, n, m);
+  if (m > 32 || (share & ~DMPC_SHARE_C)) return DMPC_ERR_UNSUPPORTED;
+  const SharedWs W = shared_ws(dtype == DMPC_F64 ? 8 : 4, T, B, n, m, share);
   if (!W.NB) return DMPC_ERR_UNSUPPORTED;
   *bytes = W.total;
   return DMPC_OK;
 }
 
+int dmpc_lqr_shared_workspace_bytes(int dtype, int T, int B, int n, int m, size_t* bytes) {
+  return dmpc_lqr_shared_workspace_bytes_ex(dtype, T, B, n, m, 0, bytes);
+}
+
 // common checks of the two shared-parameter calls; 0 or a status
 static int shared_check(dmpc_handle h, int dtype, int T, int B, int n, int m, int F_T, const void* F, const void* ws,
-                        size_t ws_bytes) {
+                        size_t ws_bytes, int share) {
   if (T < 1 || B < 1 || n < 1 || m < 1) return fail(h, DMPC_ERR_BAD_SHAPE, "T,B,n,m must be >= 1");
   if (F_T != T - 1 && F_T != T) return fail(h, DMPC_ERR_BAD_SHAPE, "F must have T-1 or T time rows");
   if ((T > 1 && !F) || !ws) return fail(h, DMPC_ERR_NULL, "lqr shared: F (T > 1) and the workspace are required");
   if (dtype != DMPC_F64 && dtype != DMPC_F32) return fail(h, DMPC_ERR_UNSUPPORTED, "dtype");
   if (m > 32) return fail(h, DMPC_ERR_UNSUPPORTED, "lqr shared: m > 32");
+  if (share & ~DMPC_SHARE_C) return fail(h, DMPC_ERR_UNSUPPORTED, "lqr shared: unknown bit in share");
   size_t need = 0;
-  if (dmpc_lqr_shared_workspace_bytes(dtype, T, B, n, m, &need)) return fail(h, DMPC_ERR_UNSUPPORTED, "lqr shared: shape too large for the chunk kernels");
-  if (ws_bytes < need) return fail(h, DMPC_ERR_BAD_SHAPE, "lqr shared: workspace too small (dmpc_lqr_shared_workspace_bytes)");
+  if (dmpc_lqr_shared_workspace_bytes_ex(dtype, T, B, n, m, share, &need)) return fail(h, DMPC_ERR_UNSUPPORTED, "lqr shared: shape too large for the chunk kernels");
+  if (ws_bytes < need) return fail(h, DMPC_ERR_BAD_SHAPE, "lqr shared: workspace too small (dmpc_lqr_shared_workspace_bytes[_ex])");
   return DMPC_OK;
+}
+
+int dmpc_lqr_solve_shared_ex(dmpc_handle h, int dtype, int T, int B, int n, int m, const void* d_x0, const void* d_C,
+                             const void* d_c, const void* d_F, int F_T, const void* d_f, void* d_x, void* d_u, void* d_ws,
+                             size_t ws_bytes, int share, void* stream) {
+  if (!h) return DMPC_ERR_NULL;
+  if (!d_x0 || !d_C || !d_c || !d_x || !d_u) return fail(h, DMPC_ERR_NULL, "lqr_solve_shared: required buffer is NULL");
+  if (int rc = shared_check(h, dtype, T, B, n, m, F_T, d_F, d_ws, ws_bytes, share)) return rc;
+  if (set_dev(h)) return DMPC_ERR_CUDA;
+  cudaStream_t st = pick(h, stream);
+  if (dtype == DMPC_F64) return lqr_solve_shared_impl<double>(h, T, B, n, m, d_x0, d_C, d_c, d_F, F_T, d_f, d_x, d_u, d_ws, share, st);
+  return lqr_solve_shared_impl<float>(h, T, B, n, m, d_x0, d_C, d_c, d_F, F_T, d_f, d_x, d_u, d_ws, share, st);
 }
 
 int dmpc_lqr_solve_shared(dmpc_handle h, int dtype, int T, int B, int n, int m, const void* d_x0, const void* d_C,
                           const void* d_c, const void* d_F, int F_T, const void* d_f, void* d_x, void* d_u, void* d_ws,
                           size_t ws_bytes, void* stream) {
+  return dmpc_lqr_solve_shared_ex(h, dtype, T, B, n, m, d_x0, d_C, d_c, d_F, F_T, d_f, d_x, d_u, d_ws, ws_bytes, 0, stream);
+}
+
+int dmpc_lqr_adjoint_shared_ex(dmpc_handle h, int dtype, int T, int B, int n, int m, const void* d_C, const void* d_c,
+                               const void* d_F, int F_T, const void* d_x, const void* d_u, const void* d_gx,
+                               const void* d_gu, void* d_ws, size_t ws_bytes, void* d_dx0, void* d_dC, void* d_dc,
+                               void* d_dF, void* d_df, int flags, int share, void* stream) {
   if (!h) return DMPC_ERR_NULL;
-  if (!d_x0 || !d_C || !d_c || !d_x || !d_u) return fail(h, DMPC_ERR_NULL, "lqr_solve_shared: required buffer is NULL");
-  if (int rc = shared_check(h, dtype, T, B, n, m, F_T, d_F, d_ws, ws_bytes)) return rc;
+  const bool dc_nullable = (share & DMPC_SHARE_C) != 0;
+  if (!d_C || !d_c || !d_x || !d_u || !d_dx0 || !d_dC || (!d_dc && !dc_nullable) || (F_T > 0 && !d_dF))
+    return fail(h, DMPC_ERR_NULL, "lqr_adjoint_shared: required buffer is NULL");
+  if (int rc = shared_check(h, dtype, T, B, n, m, F_T, d_F, d_ws, ws_bytes, share)) return rc;
   if (set_dev(h)) return DMPC_ERR_CUDA;
   cudaStream_t st = pick(h, stream);
-  if (dtype == DMPC_F64) return lqr_solve_shared_impl<double>(h, T, B, n, m, d_x0, d_C, d_c, d_F, F_T, d_f, d_x, d_u, d_ws, st);
-  return lqr_solve_shared_impl<float>(h, T, B, n, m, d_x0, d_C, d_c, d_F, F_T, d_f, d_x, d_u, d_ws, st);
+  if (dtype == DMPC_F64) return lqr_adjoint_shared_impl<double>(h, T, B, n, m, d_C, d_c, d_F, F_T, d_x, d_u, d_gx, d_gu, d_ws, d_dx0, d_dC, d_dc, d_dF, d_df, flags, share, st);
+  return lqr_adjoint_shared_impl<float>(h, T, B, n, m, d_C, d_c, d_F, F_T, d_x, d_u, d_gx, d_gu, d_ws, d_dx0, d_dC, d_dc, d_dF, d_df, flags, share, st);
 }
 
 int dmpc_lqr_adjoint_shared(dmpc_handle h, int dtype, int T, int B, int n, int m, const void* d_C, const void* d_c,
                             const void* d_F, int F_T, const void* d_x, const void* d_u, const void* d_gx,
                             const void* d_gu, void* d_ws, size_t ws_bytes, void* d_dx0, void* d_dC, void* d_dc,
                             void* d_dF, void* d_df, int flags, void* stream) {
-  if (!h) return DMPC_ERR_NULL;
-  if (!d_C || !d_c || !d_x || !d_u || !d_dx0 || !d_dC || !d_dc || (F_T > 0 && !d_dF))
-    return fail(h, DMPC_ERR_NULL, "lqr_adjoint_shared: required buffer is NULL");
-  if (int rc = shared_check(h, dtype, T, B, n, m, F_T, d_F, d_ws, ws_bytes)) return rc;
-  if (set_dev(h)) return DMPC_ERR_CUDA;
-  cudaStream_t st = pick(h, stream);
-  if (dtype == DMPC_F64) return lqr_adjoint_shared_impl<double>(h, T, B, n, m, d_C, d_c, d_F, F_T, d_x, d_u, d_gx, d_gu, d_ws, d_dx0, d_dC, d_dc, d_dF, d_df, flags, st);
-  return lqr_adjoint_shared_impl<float>(h, T, B, n, m, d_C, d_c, d_F, F_T, d_x, d_u, d_gx, d_gu, d_ws, d_dx0, d_dC, d_dc, d_dF, d_df, flags, st);
+  return dmpc_lqr_adjoint_shared_ex(h, dtype, T, B, n, m, d_C, d_c, d_F, F_T, d_x, d_u, d_gx, d_gu, d_ws, ws_bytes, d_dx0,
+                                    d_dC, d_dc, d_dF, d_df, flags, 0, stream);
 }
 
 }  // extern "C"

@@ -19,6 +19,14 @@
 //                                                    lambda_{t+1} dtau_t^T)
 //   lqr_shared_reduce_kernel dC_t, dF_t from the partials, summed over the chunks in a fixed order (no atomics)
 //
+// Batch-shared c (c_shared: c is [T,s], the model's one learned block).  c_t is staged once per step and read with a
+// column stride of 0.  With f == nullptr as well, every element has the same k_t, and the B = 1 sweep (run on the real c)
+// already holds it in ks: lqr_shared_rollout_kernel runs only the rollout, reading x0 and writing x, u.  With f given,
+// lqr_shared_fwd_kernel runs its vector sweep on the stride-0 c.  The adjoint then returns dc[T,s] = sum_b dtau_{t,b}
+// (the reference's dc = dtau, summed as the backward of the broadcast would): sweep 3 appends the chunk's sum_b dtau_t to
+// its partial record and the reduce kernel sums those over the chunks in the same fixed order; sweeps 1-2 park k' and
+// dtau in a [T,B,s] region of the workspace instead of in dc.
+//
 // Products: fp64 runs them on the FP64 tensor cores (mma.sync.m8n8k4.f64, 8x8 output tiles spread over the warps);
 // fp32 on FMA.  Both sum in a fixed order, so results are deterministic.
 #pragma once
@@ -32,12 +40,14 @@ constexpr int kSharedThreads = 256;
 template <typename R>
 struct LqrSharedParams {
   int T, B, n, m, F_T, NB, flags;   // flags: ADJ_QUIRK_DC | ADJ_QUIRK_DF
+  int c_shared;     // 1: c is [T,s] and dc is [T,s], summed over the batch
   const R* x0;      // [B,n]
   const R* C;       // [T,s,s]    shared
-  const R* c;       // [T,B,s]
+  const R* c;       // [T,B,s], or [T,s] when c_shared
   const R* F;       // [F_T,n,s]  shared
   const R* f;       // [T-1,B,n] or nullptr
   const R* Ks;      // [T,m,n]            K_t of the B = 1 sweep
+  const R* ks;      // [T,m]              k_t of the B = 1 sweep (the batch's k_t when it ran on a shared c, f == nullptr)
   const R* fac;     // [T,m*m+n*m]        Quu_t^-1 | Qxu_t
   const R* Vsave;   // [T,n*n+n]          V_t | (unused) for t >= 1
   R* x;             // [T,B,n]  forward output / adjoint input
@@ -45,12 +55,26 @@ struct LqrSharedParams {
   const R* gx;      // [T,B,n] or nullptr (zeros)
   const R* gu;      // [T,B,m] or nullptr (zeros)
   R* dx0;           // [B,n]
-  R* dc;            // [T,B,s]
+  R* dc;            // [T,B,s]; c_shared: [T,s] or nullptr
   R* df;            // [T-1,B,n] or nullptr
-  R* part;          // [nchunk][T][s*s + n*s]: P_t | R_t per chunk
+  R* park;          // [T,B,s]  k'_t, then d-tau_t, between the adjoint's sweeps (dc itself unless c_shared)
+  R* part;          // [nchunk][T][shared_rec_elems]: P_t | R_t (| sum_b dtau_t when c_shared) per chunk
   R* dC;            // [T,s,s]
   R* dF;            // [F_T,n,s] or nullptr
 };
+
+// Reals of one partial record (one chunk, one step) of the adjoint.
+__host__ __device__ __forceinline__ int shared_rec_elems(int n, int m, bool c_shared) {
+  const int s = n + m;
+  return s * s + n * s + (c_shared ? s : 0);
+}
+
+// Outputs of lqr_shared_reduce_kernel: dC, then dF (when given), then dc (c_shared, when given).
+template <typename R>
+__host__ __device__ __forceinline__ size_t shared_reduce_outputs(const LqrSharedParams<R>& p) {
+  const size_t s = (size_t)(p.n + p.m);
+  return (size_t)p.T * s * s + (p.dF ? (size_t)p.F_T * p.n * s : 0) + (p.c_shared && p.dc ? (size_t)p.T * s : 0);
+}
 
 // Shared-memory layouts (offsets in reals).  Each kernel has two staging slots (step t and the prefetched next step) and
 // its state blocks.  Every offset is a multiple of 2 reals so 16-byte cp.async stays possible.
@@ -164,8 +188,9 @@ __device__ __forceinline__ void zero_rows(R* dst, int ld, int w, int cnt) {
   for (int o = threadIdx.x; o < cnt * w; o += blockDim.x) { const int e = o / w; dst[e * ld + o - e * w] = R(0); }
 }
 
-template <typename R>
-__global__ void __launch_bounds__(kSharedThreads) lqr_shared_fwd_kernel(const LqrSharedParams<R> p) {
+// kRollOnly: c shared and f == nullptr, so k_t is the B = 1 sweep's ks and the vector sweep is skipped.
+template <typename R, bool kRollOnly>
+__device__ __forceinline__ void lqr_shared_fwd_body(const LqrSharedParams<R>& p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   R* sm = reinterpret_cast<R*>(smem_raw);
   const int n = p.n, m = p.m, s = n + m, T = p.T, NB = p.NB;
@@ -175,46 +200,50 @@ __global__ void __launch_bounds__(kSharedThreads) lqr_shared_fwd_kernel(const Lq
   const SharedFwdLayout L(n, m, NB);
   const CtaGrp g;
   const int fsz = m * m + n * m;
-  R *q = sm + L.q, *v = sm + L.v, *mv = sm + L.mv, *kb = sm + L.kb;
+  int sl = 0;
 
   // ---- vector sweep, t = T-1 .. 0.  Slot of step t: c_t, f_t, F_t, V_{t+1}, Quu_t^-1, Qxu_t.
-  auto stage_bw = [&](int t, int sl) {
-    R* S = sm + sl * L.slot;
-    g_cp_async(g, S + L.oc, p.c + ((size_t)t * B + b0) * s, ne * s);
-    g_cp_async(g, S + L.oQi, p.fac + (size_t)t * fsz, fsz);              
-    if (t < T - 1) {
-      g_cp_async(g, S + L.oF, p.F + (size_t)t * n * s, n * s);
-      if (p.f) {
-        g_cp_async(g, S + L.of, p.f + ((size_t)t * B + b0) * n, ne * n);
-        g_cp_async(g, S + L.oV, p.Vsave + (size_t)(t + 1) * (n * n + n), n * n);
+  if constexpr (!kRollOnly) {
+    R *q = sm + L.q, *v = sm + L.v, *mv = sm + L.mv, *kb = sm + L.kb;
+    const int cbs = p.c_shared ? 0 : s;                                   // column (element) stride of the staged c_t
+    auto stage_bw = [&](int t, int sl) {
+      R* S = sm + sl * L.slot;
+      if (p.c_shared) g_cp_async(g, S + L.oc, p.c + (size_t)t * s, s);
+      else g_cp_async(g, S + L.oc, p.c + ((size_t)t * B + b0) * s, ne * s);
+      g_cp_async(g, S + L.oQi, p.fac + (size_t)t * fsz, fsz);
+      if (t < T - 1) {
+        g_cp_async(g, S + L.oF, p.F + (size_t)t * n * s, n * s);
+        if (p.f) {
+          g_cp_async(g, S + L.of, p.f + ((size_t)t * B + b0) * n, ne * n);
+          g_cp_async(g, S + L.oV, p.Vsave + (size_t)(t + 1) * (n * n + n), n * n);
+        }
       }
-    }
-    cp_async_commit();
-  };
-  stage_bw(T - 1, 0);
-  int sl = 0;
-  for (int t = T - 1; t >= 0; --t) {
-    if (t > 0) { stage_bw(t - 1, sl ^ 1); cp_async_wait<1>(); } else cp_async_wait<0>();
-    __syncthreads();
-    R* S = sm + sl * L.slot;
-    const R* vin = v;
-    if (t < T - 1 && p.f) {                                                // mv = V_{t+1} f_t + v_{t+1}
-      cta_gemm<R>(n, ne, n, mv, 1, n, v, 1, n, S + L.oV, n, 1, S + L.of, 1, n, false);
+      cp_async_commit();
+    };
+    stage_bw(T - 1, 0);
+    for (int t = T - 1; t >= 0; --t) {
+      if (t > 0) { stage_bw(t - 1, sl ^ 1); cp_async_wait<1>(); } else cp_async_wait<0>();
       __syncthreads();
-      vin = mv;
+      R* S = sm + sl * L.slot;
+      const R* vin = v;
+      if (t < T - 1 && p.f) {                                                // mv = V_{t+1} f_t + v_{t+1}
+        cta_gemm<R>(n, ne, n, mv, 1, n, v, 1, n, S + L.oV, n, 1, S + L.of, 1, n, false);
+        __syncthreads();
+        vin = mv;
+      }
+      // q = c_t + F_t^T mv     (t = T-1: q = c_t)
+      cta_gemm<R>(s, ne, t < T - 1 ? n : 0, q, 1, s, S + L.oc, 1, cbs, S + L.oF, 1, s, vin, 1, n, false);
+      __syncthreads();
+      // k_t = -Quu^-1 q_u
+      cta_gemm<R>(m, ne, m, kb, 1, m, nullptr, 0, 0, S + L.oQi, m, 1, q + n, 1, s, true);
+      __syncthreads();
+      // v_t = q_x + Qxu k_t; k_t is parked in the u output until the rollout reads it back
+      if (t > 0) cta_gemm<R>(n, ne, m, v, 1, n, q, 1, s, S + L.oQi + m * m, m, 1, kb, 1, m, false);
+      R* ug = p.u + ((size_t)t * B + b0) * m;
+      for (int o = threadIdx.x; o < ne * m; o += blockDim.x) ug[o] = kb[o];
+      __syncthreads();
+      sl ^= 1;
     }
-    // q = c_t + F_t^T mv     (t = T-1: q = c_t)
-    cta_gemm<R>(s, ne, t < T - 1 ? n : 0, q, 1, s, S + L.oc, 1, s, S + L.oF, 1, s, vin, 1, n, false);
-    __syncthreads();
-    // k_t = -Quu^-1 q_u
-    cta_gemm<R>(m, ne, m, kb, 1, m, nullptr, 0, 0, S + L.oQi, m, 1, q + n, 1, s, true);
-    __syncthreads();
-    // v_t = q_x + Qxu k_t; k_t is parked in the u output until the rollout reads it back
-    if (t > 0) cta_gemm<R>(n, ne, m, v, 1, n, q, 1, s, S + L.oQi + m * m, m, 1, kb, 1, m, false);
-    R* ug = p.u + ((size_t)t * B + b0) * m;
-    for (int o = threadIdx.x; o < ne * m; o += blockDim.x) ug[o] = kb[o];
-    __syncthreads();
-    sl ^= 1;
   }
 
   // ---- rollout, t = 0 .. T-1.  Slot of step t: K_t, F_t, f_t.
@@ -233,8 +262,13 @@ __global__ void __launch_bounds__(kSharedThreads) lqr_shared_fwd_kernel(const Lq
   sl = 0;
   for (int t = 0; t < T; ++t) {
     if (t < T - 1) { stage_fw(t + 1, sl ^ 1); cp_async_wait<1>(); } else cp_async_wait<0>();
-    const R* ug = p.u + ((size_t)t * B + b0) * m;                         // k_t from the sweep (this CTA wrote it)
-    for (int o = threadIdx.x; o < ne * m; o += blockDim.x) { const int e = o / m; tc[e * s + n + o - e * m] = ug[o]; }
+    if constexpr (kRollOnly) {                                            // k_t of the B = 1 sweep, the same for all
+      const R* kg = p.ks + (size_t)t * m;
+      for (int o = threadIdx.x; o < ne * m; o += blockDim.x) { const int e = o / m; tc[e * s + n + o - e * m] = kg[o - e * m]; }
+    } else {
+      const R* ug = p.u + ((size_t)t * B + b0) * m;                       // k_t from the sweep (this CTA wrote it)
+      for (int o = threadIdx.x; o < ne * m; o += blockDim.x) { const int e = o / m; tc[e * s + n + o - e * m] = ug[o]; }
+    }
     __syncthreads();
     R* S = sm + sl * L.slot;
     cta_gemm<R>(m, ne, n, tc + n, 1, s, tc + n, 1, s, S + L.oK, n, 1, tc, 1, s, false);   // u = K x + k
@@ -250,6 +284,18 @@ __global__ void __launch_bounds__(kSharedThreads) lqr_shared_fwd_kernel(const Lq
   }
 }
 
+// Vector sweep + rollout (c per element, or c shared with f given).
+template <typename R>
+__global__ void __launch_bounds__(kSharedThreads) lqr_shared_fwd_kernel(const LqrSharedParams<R> p) {
+  lqr_shared_fwd_body<R, false>(p);
+}
+
+// Rollout only (c shared, f == nullptr): k_t comes from the B = 1 sweep.
+template <typename R>
+__global__ void __launch_bounds__(kSharedThreads) lqr_shared_rollout_kernel(const LqrSharedParams<R> p) {
+  lqr_shared_fwd_body<R, true>(p);
+}
+
 template <typename R>
 __global__ void __launch_bounds__(kSharedThreads) lqr_shared_adj_kernel(const LqrSharedParams<R> p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -262,7 +308,7 @@ __global__ void __launch_bounds__(kSharedThreads) lqr_shared_adj_kernel(const Lq
   const CtaGrp g;
   const int fsz = m * m + n * m;
 
-  // ---- sweep 1, t = T-1 .. 0: q = g_t + F_t^T v'_{t+1};  k'_t = -Quu^-1 q_u;  v'_t = q_x + Qxu k'_t.  k'_t -> dc[t][:, n:]
+  // ---- sweep 1, t = T-1 .. 0: q = g_t + F_t^T v'_{t+1};  k'_t = -Quu^-1 q_u;  v'_t = q_x + Qxu k'_t.  k'_t -> park[t][:, n:]
   {
     R *q = sm + L.q, *v = sm + L.v, *kb = sm + L.kb;
     auto stage1 = [&](int t, int sl) {
@@ -284,14 +330,14 @@ __global__ void __launch_bounds__(kSharedThreads) lqr_shared_adj_kernel(const Lq
       cta_gemm<R>(m, ne, m, kb, 1, m, nullptr, 0, 0, S + L.oQi, m, 1, q + n, 1, s, true);
       __syncthreads();
       if (t > 0) cta_gemm<R>(n, ne, m, v, 1, n, q, 1, s, S + L.oQi + m * m, m, 1, kb, 1, m, false);
-      R* dg = p.dc + ((size_t)t * B + b0) * s;
+      R* dg = p.park + ((size_t)t * B + b0) * s;
       for (int o = threadIdx.x; o < ne * m; o += blockDim.x) { const int e = o / m; dg[e * s + n + o - e * m] = kb[o]; }
       __syncthreads();
       sl ^= 1;
     }
   }
 
-  // ---- sweep 2, t = 0 .. T-1: d-u_t = K_t d-x_t + k'_t;  d-x_{t+1} = F_t d-tau_t  (d-x_0 = 0).  d-tau_t -> dc[t]
+  // ---- sweep 2, t = 0 .. T-1: d-u_t = K_t d-x_t + k'_t;  d-x_{t+1} = F_t d-tau_t  (d-x_0 = 0).  d-tau_t -> park[t]
   {
     R* tc = sm + L.q; R* tn = sm + L.v;                                   // two [NB][s] blocks (q and v|kb of sweep 1)
     auto stage2 = [&](int t, int sl) {
@@ -305,7 +351,7 @@ __global__ void __launch_bounds__(kSharedThreads) lqr_shared_adj_kernel(const Lq
     int sl = 0;
     for (int t = 0; t < T; ++t) {
       if (t < T - 1) { stage2(t + 1, sl ^ 1); cp_async_wait<1>(); } else cp_async_wait<0>();
-      R* dg = p.dc + ((size_t)t * B + b0) * s;
+      R* dg = p.park + ((size_t)t * B + b0) * s;
       for (int o = threadIdx.x; o < ne * m; o += blockDim.x) { const int e = o / m; const int j = n + o - e * m; tc[e * s + j] = dg[e * s + j]; }
       __syncthreads();
       R* S = sm + sl * L.slot;
@@ -324,14 +370,16 @@ __global__ void __launch_bounds__(kSharedThreads) lqr_shared_adj_kernel(const Lq
     R* dt = sm + L.dtau;
     R *lo = sm + L.l0, *ln = sm + L.l1, *dlo = sm + L.dl0, *dln = sm + L.dl1;   // lambda_{t+1} (old), lambda_t (new)
     const bool strict_df = (p.flags & ADJ_QUIRK_DF) != 0;
-    const int rsz = s * s + n * s;
+    const int rsz = shared_rec_elems(n, m, p.c_shared);
+    const int cbs = p.c_shared ? 0 : n;                                   // column (element) stride of the staged c_x
     auto stage3 = [&](int t, int sl) {
       R* S = sm + sl * L.slot;
       g_cp_async(g, S + L.oCx, p.C + (size_t)t * s * s, n * s);          // rows 0..n-1 of C_t
       if (t < T - 1) g_cp_async(g, S + L.oF, p.F + (size_t)t * n * s, n * s);
       stage_rows(S + L.otau, s, p.x + ((size_t)t * B + b0) * n, n, n, ne);
       stage_rows(S + L.otau + n, s, p.u + ((size_t)t * B + b0) * m, m, m, ne);
-      stage_rows(S + L.ocx, n, p.c + ((size_t)t * B + b0) * s, s, n, ne);   // c_t[:, :n]: rows of length n, stride s
+      if (p.c_shared) g_cp_async(g, S + L.ocx, p.c + (size_t)t * s, n);   // c_t[:n], once
+      else stage_rows(S + L.ocx, n, p.c + ((size_t)t * B + b0) * s, s, n, ne);   // c_t[:, :n]: rows of length n, stride s
       if (p.gx) g_cp_async(g, S + L.ogx, p.gx + ((size_t)t * B + b0) * n, ne * n); else zero_rows(S + L.ogx, n, n, ne);
       cp_async_commit();
     };
@@ -339,12 +387,18 @@ __global__ void __launch_bounds__(kSharedThreads) lqr_shared_adj_kernel(const Lq
     int sl = 0;
     for (int t = T - 1; t >= 0; --t) {
       if (t > 0) { stage3(t - 1, sl ^ 1); cp_async_wait<1>(); } else cp_async_wait<0>();
-      const R* dg = p.dc + ((size_t)t * B + b0) * s;
+      const R* dg = p.park + ((size_t)t * B + b0) * s;
       for (int o = threadIdx.x; o < ne * s; o += blockDim.x) dt[o] = dg[o];
       __syncthreads();
       R* S = sm + sl * L.slot;
       const R* tau = S + L.otau;
       R* pt = p.part + ((size_t)blockIdx.x * T + t) * rsz;
+      if (p.c_shared)                                                     // sum_b dtau_t over the chunk, in element order
+        for (int j = threadIdx.x; j < s; j += blockDim.x) {
+          R a = R(0);
+          for (int e = 0; e < ne; ++e) a += dt[e * s + j];
+          pt[s * s + n * s + j] = a;
+        }
       cta_gemm<R>(s, s, ne, pt, s, 1, nullptr, 0, 0, dt, 1, s, tau, s, 1, false);               // P_t = sum dtau tau^T
       if (t < T - 1) {                                                    // R_t = sum dlambda_{t+1} tau^T + lambda_{t+1} dtau^T
         cta_gemm<R>(n, s, ne, pt + s * s, s, 1, nullptr, 0, 0, dlo, 1, n, tau, s, 1, false);
@@ -355,7 +409,7 @@ __global__ void __launch_bounds__(kSharedThreads) lqr_shared_adj_kernel(const Lq
         }
       }
       // lambda_t = c_x + C_x tau_t (+ A_t^T lambda_{t+1}),  d-lambda_t = gx + C_x dtau_t (+ A_t^T dlambda_{t+1})
-      cta_gemm<R>(n, ne, s, ln, 1, n, S + L.ocx, 1, n, S + L.oCx, s, 1, tau, 1, s, false);
+      cta_gemm<R>(n, ne, s, ln, 1, n, S + L.ocx, 1, cbs, S + L.oCx, s, 1, tau, 1, s, false);
       cta_gemm<R>(n, ne, s, dln, 1, n, S + L.ogx, 1, n, S + L.oCx, s, 1, dt, 1, s, false);
       __syncthreads();
       if (t < T - 1) {
@@ -378,12 +432,12 @@ __global__ void __launch_bounds__(kSharedThreads) lqr_shared_adj_kernel(const Lq
   }
 }
 
-// dC_t = 0.5 P_t + P_t^T (ADJ_QUIRK_DC, reference :128) or 0.5 (P_t + P_t^T);  dF_t = R_t (t < T-1), 0 for row T-1.
-// One thread per output, chunks summed in index order: deterministic.
+// dC_t = 0.5 P_t + P_t^T (ADJ_QUIRK_DC, reference :128) or 0.5 (P_t + P_t^T);  dF_t = R_t (t < T-1), 0 for row T-1;
+// c_shared: dc_t = sum_b dtau_t.  One thread per output, chunks summed in index order: deterministic.
 template <typename R>
 __global__ void lqr_shared_reduce_kernel(const LqrSharedParams<R> p, int nchunk) {
-  const int n = p.n, s = n + p.m, T = p.T, rsz = s * s + n * s;
-  const size_t nC = (size_t)T * s * s, total = nC + (p.dF ? (size_t)p.F_T * n * s : 0);
+  const int n = p.n, s = n + p.m, T = p.T, rsz = shared_rec_elems(n, p.m, p.c_shared);
+  const size_t nC = (size_t)T * s * s, nCF = nC + (p.dF ? (size_t)p.F_T * n * s : 0), total = shared_reduce_outputs(p);
   const size_t o = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (o >= total) return;
   if (o < nC) {
@@ -395,13 +449,19 @@ __global__ void lqr_shared_reduce_kernel(const LqrSharedParams<R> p, int nchunk)
       b += pt[j * s + i];
     }
     p.dC[o] = (p.flags & ADJ_QUIRK_DC) ? R(0.5) * a + b : R(0.5) * (a + b);
-  } else {
+  } else if (o < nCF) {
     const size_t r = o - nC;
     const int t = (int)(r / (n * s)), ij = (int)(r - (size_t)t * n * s);
     R a = R(0);
     if (t < T - 1)
       for (int k = 0; k < nchunk; ++k) a += p.part[((size_t)k * T + t) * rsz + s * s + ij];
     p.dF[r] = a;
+  } else {
+    const size_t r = o - nCF;
+    const int t = (int)(r / s), j = (int)(r - (size_t)t * s);
+    R a = R(0);
+    for (int k = 0; k < nchunk; ++k) a += p.part[((size_t)k * T + t) * rsz + s * s + n * s + j];
+    p.dc[r] = a;
   }
 }
 

@@ -18,6 +18,7 @@ static int shared_launch(K kernel, const P& p, size_t smem, cudaStream_t st, lon
 template <typename R>
 int launch_lqr_shared_fwd(const LqrSharedParams<R>& p, cudaStream_t st, long long* nl) {
   const size_t smem = (size_t)SharedFwdLayout(p.n, p.m, p.NB).total * sizeof(R);
+  if (p.c_shared && !p.f) return shared_launch(lqr_shared_rollout_kernel<R>, p, smem, st, nl);   // k_t is the sweep's ks
   return shared_launch(lqr_shared_fwd_kernel<R>, p, smem, st, nl);
 }
 
@@ -26,8 +27,7 @@ int launch_lqr_shared_adj(const LqrSharedParams<R>& p, cudaStream_t st, long lon
   const size_t smem = (size_t)SharedAdjLayout(p.n, p.m, p.NB).total * sizeof(R);
   int rc = shared_launch(lqr_shared_adj_kernel<R>, p, smem, st, nl);
   if (rc) return rc;
-  const int s = p.n + p.m;
-  const size_t total = (size_t)p.T * s * s + (p.dF ? (size_t)p.F_T * p.n * s : 0);
+  const size_t total = shared_reduce_outputs(p);
   const int tpb = 256;
   lqr_shared_reduce_kernel<R><<<(unsigned)((total + tpb - 1) / tpb), tpb, 0, st>>>(p, (p.B + p.NB - 1) / p.NB);
   if (nl) ++*nl;

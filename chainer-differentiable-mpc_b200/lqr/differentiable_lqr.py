@@ -180,10 +180,11 @@ class DiffLqr(FunctionNodeBase):
 
 class DiffLqrShared(FunctionNodeBase):
     """`DiffLqrShared(T, n_batch, n_state, n_ctrl).apply((x_init, C, c, F, f)) -> (x, u)` for a batch that shares its
-    cost and dynamics matrices: C [T,s,s] and F [T-1 or T,n,s] are one block per time step; x_init [B,n], c [T,B,s] and
-    f [T-1,B,n] (or None) are per element.  Same results as DiffLqr on the broadcast tensors; `backward` returns the
-    gradients in the shapes of the inputs, dC and dF summed over the batch (dmpc_lqr_solve_shared / _adjoint_shared:
-    one Riccati sweep for the whole batch)."""
+    cost and dynamics matrices: C [T,s,s] and F [T-1 or T,n,s] are one block per time step; x_init [B,n] and
+    f [T-1,B,n] (or None) are per element; c is per element [T,B,s] or shared [T,s] (chosen by c.ndim).  Same results
+    as DiffLqr on the broadcast tensors; `backward` returns the gradients in the shapes of the inputs, dC, dF (and dc
+    when c is [T,s]) summed over the batch (dmpc_lqr_solve_shared[_ex] / _adjoint_shared[_ex]: one Riccati sweep for
+    the whole batch; with a shared c and f None the forward is that sweep plus the rollout)."""
 
     def __init__(self, T, n_batch, n_state, n_ctrl, device=0, dtype=np.float64, strict_reference=True, context=None):
         super().__init__()
@@ -195,56 +196,76 @@ class DiffLqrShared(FunctionNodeBase):
         self._d = None
         self._F_T = None
         self._have_f = False
+        self._shared_c = False
 
     def _buffers(self):
         if self._d is None:
             T, B, n, m, s, dt, ctx = self.T, self.n_batch, self.n_state, self.n_ctrl, self.n_sc, self.dtype, self._ctx
             Tm = max(T - 1, 1)
-            shapes = dict(x0=(B, n), C=(T, s, s), c=(T, B, s), F=(T, n, s), f=(Tm, B, n), x=(T, B, n), u=(T, B, m),
-                          gx=(T, B, n), gu=(T, B, m), dx0=(B, n), dC=(T, s, s), dc=(T, B, s), dF=(T, n, s), df=(Tm, B, n),
-                          ws=(ctx.lqr_shared_workspace_bytes(dt, T, B, n, m),))
-            self._d = {k: ctx.empty(v, np.uint8 if k == "ws" else dt) for k, v in shapes.items()}
-        return self._d
+            shapes = dict(x0=(B, n), C=(T, s, s), F=(T, n, s), f=(Tm, B, n), x=(T, B, n), u=(T, B, m),
+                          gx=(T, B, n), gu=(T, B, m), dx0=(B, n), dC=(T, s, s), dF=(T, n, s), df=(Tm, B, n))
+            self._d = {k: ctx.empty(v, dt) for k, v in shapes.items()}
+        d = self._d
+        if self._shared_c and "ws_c" not in d:          # c [T,s]: dc [T,s] and the DMPC_SHARE_C workspace
+            T, B, n, m, s, dt, ctx = self.T, self.n_batch, self.n_state, self.n_ctrl, self.n_sc, self.dtype, self._ctx
+            d["c_s"], d["dc_s"] = ctx.empty((T, s), dt), ctx.empty((T, s), dt)
+            d["ws_c"] = ctx.empty((ctx.lqr_shared_workspace_bytes(dt, T, B, n, m, _native.SHARE_C),), np.uint8)
+        if not self._shared_c and "ws" not in d:        # c [T,B,s]
+            T, B, n, m, s, dt, ctx = self.T, self.n_batch, self.n_state, self.n_ctrl, self.n_sc, self.dtype, self._ctx
+            d["c"], d["dc"] = ctx.empty((T, B, s), dt), ctx.empty((T, B, s), dt)
+            d["ws"] = ctx.empty((ctx.lqr_shared_workspace_bytes(dt, T, B, n, m),), np.uint8)
+        return d
+
+    def _mode(self):
+        """(c buffer, dc buffer, workspace, share argument) of the form the last forward used."""
+        d = self._d
+        if self._shared_c:
+            return d["c_s"], d["dc_s"], d["ws_c"], _native.SHARE_C
+        return d["c"], d["dc"], d["ws"], None
 
     def apply_numpy(self, x_init, C, c, large_f, f=None):
         T, B, n, m, s, dt = self.T, self.n_batch, self.n_state, self.n_ctrl, self.n_sc, self.dtype
         x_init, C, c, F = as_f(x_init, dt), as_f(C, dt), as_f(c, dt), as_f(large_f, dt)
         assert list(x_init.shape) == [B, n]
         assert list(C.shape) == [T, s, s], "C dim mismatch"
-        assert list(c.shape) == [T, B, s], "c dim mismatch"
+        assert list(c.shape) in ([T, B, s], [T, s]), "c dim mismatch"
         assert F.shape[0] in (T - 1, T) and list(F.shape[1:]) == [n, s], "F dim mismatch"
         self._have_f = f is not None and to_xp(f) is not None and T > 1
         if self._have_f:
             f = as_f(f, dt)
             assert list(f.shape) == [T - 1, B, n], " f dim mismatch"
         self._F_T = F.shape[0]
+        self._shared_c = c.ndim == 2
         d = self._buffers()
+        c_buf, _, ws, share = self._mode()
         ctx = self._ctx
-        d["x0"].upload(x_init); d["C"].upload(C); d["c"].upload(c)
+        d["x0"].upload(x_init); d["C"].upload(C); c_buf.upload(c)
         Fp = np.zeros((T, n, s), dt)                    # the device buffer has room for F_T = T rows
         Fp[:self._F_T] = F
         d["F"].upload(Fp)
         if self._have_f:
             d["f"].upload(f)
-        ctx.lqr_solve_shared(dt, T, B, n, m, d["x0"], d["C"], d["c"], d["F"], self._F_T,
-                             d["f"] if self._have_f else None, d["x"], d["u"], d["ws"])
+        ctx.lqr_solve_shared(dt, T, B, n, m, d["x0"], d["C"], c_buf, d["F"], self._F_T,
+                             d["f"] if self._have_f else None, d["x"], d["u"], ws, share=share)
         x = d["x"].download(sync=False)
         u = d["u"].download()
         return x, u
 
     def backward_numpy(self, grad_x, grad_u):
-        """-> (dx0 [B,n], dC [T,s,s], dc [T,B,s], dF [F_T,n,s], df [T-1,B,n] or None)."""
+        """-> (dx0 [B,n], dC [T,s,s], dc [T,B,s] (or [T,s], summed over the batch, when c was [T,s]), dF [F_T,n,s],
+        df [T-1,B,n] or None)."""
         T, B, n, m, s, dt = self.T, self.n_batch, self.n_state, self.n_ctrl, self.n_sc, self.dtype
         d = self._buffers()
+        c_buf, dc_buf, ws, share = self._mode()
         ctx = self._ctx
         gx = None if grad_x is None else d["gx"].upload(as_f(grad_x, dt))
         gu = None if grad_u is None else d["gu"].upload(as_f(grad_u, dt))
-        ctx.lqr_adjoint_shared(dt, T, B, n, m, d["C"], d["c"], d["F"], self._F_T, d["x"], d["u"], gx, gu, d["ws"],
-                               d["dx0"], d["dC"], d["dc"], d["dF"], d["df"] if self._have_f else None,
-                               _native.ADJ_STRICT_REFERENCE if self.strict_reference else 0)
+        ctx.lqr_adjoint_shared(dt, T, B, n, m, d["C"], c_buf, d["F"], self._F_T, d["x"], d["u"], gx, gu, ws,
+                               d["dx0"], d["dC"], dc_buf, d["dF"], d["df"] if self._have_f else None,
+                               _native.ADJ_STRICT_REFERENCE if self.strict_reference else 0, share=share)
         dx0 = d["dx0"].download(sync=False)
         dC = d["dC"].download(sync=False)
-        dc = d["dc"].download(sync=False)
+        dc = dc_buf.download(sync=False)
         df = d["df"].download(sync=False)[:T - 1] if self._have_f else None
         dF = d["dF"].download()[:self._F_T]
         return dx0, dC, dc, dF, df
@@ -266,7 +287,7 @@ class DiffLqrShared(FunctionNodeBase):
 
 
 from _compat import NetLinkBase, Parameter  # noqa: E402
-from util import expand_time_batch  # noqa: E402
+from util import expand_batch, expand_time_batch  # noqa: E402
 
 
 def _cat_ab(A, B):
@@ -276,9 +297,21 @@ def _cat_ab(A, B):
     return np.concatenate((A.array, B.array), axis=1)
 
 
+def _batch_invariant(C):
+    """True when C [T,B,...] is a plain array whose entries do not vary along the batch axis: a stride-0 broadcast, or
+    (checked second) a copy of C[:, :1]."""
+    if not isinstance(C, np.ndarray) or C.ndim < 2 or C.shape[1] < 1:
+        return False
+    return C.strides[1] == 0 or np.array_equal(C, np.broadcast_to(C[:, :1], C.shape))
+
+
 class LqrNet(NetLinkBase):
-    """Learn A, B through the LQR layer (reference :145-198; same seeding, :167-171).  `backward_numpy` is the fused
-    path: (T,B)-sum of dF inside the adjoint kernel -> A.grad, B.grad without the [T-1,B,n,s] tensor."""
+    """Learn A, B through the LQR layer (reference :145-198; same seeding, :167-171).  C and c come in as the reference
+    takes them ([T,B,s,s], [T,B,s]).  When C is a plain array that does not vary over the batch (the LQRnet notebook's
+    C = I), the layer is DiffLqrShared on C[:, 0] and the per-element c: one Riccati sweep for the batch, and
+    `backward_numpy` sums dF over t on the host.  Otherwise (C varies per element, or is a Chainer Variable whose
+    per-element dC the caller may read) it is DiffLqr, and `backward_numpy` is its fused path: the (T,B)-sum of dF inside
+    the adjoint kernel -> A.grad, B.grad without the [T-1,B,n,s] tensor."""
 
     def __init__(self, T, n_batch, n_state, n_ctrl, seed):
         super().__init__()
@@ -290,20 +323,33 @@ class LqrNet(NetLinkBase):
             self.A = Parameter(A)
             self.B = Parameter(np.random.randn(n_state, n_ctrl).astype("float"))
         self.lqr_layer = DiffLqr(T, n_batch, n_state, n_ctrl)
+        self.lqr_shared = DiffLqrShared(T, n_batch, n_state, n_ctrl)
+        self._used_shared = False
 
     def forward(self, inputs):
         x_init, C, c, f = inputs
+        self._used_shared = _batch_invariant(C)
+        if self._used_shared:
+            large_f = expand_batch(_cat_ab(self.A, self.B), self.T - 1)             # [T-1, n, s]
+            return self.lqr_shared.apply((x_init, np.ascontiguousarray(C[:, 0]), c, large_f, f))
         large_f = expand_time_batch(_cat_ab(self.A, self.B), self.T - 1, self.n_batch)
         return self.lqr_layer.apply((x_init, C, c, large_f, f))
 
     def backward_numpy(self, grad_x, grad_u):
-        g = self.lqr_layer.backward_reduced_numpy(grad_x, grad_u)      # (dx0, sum dC, sum dc, sum dF, sum df)
-        self.A.grad, self.B.grad = g[3][:, :self.n_state].copy(), g[3][:, self.n_state:].copy()
+        n = self.n_state
+        if self._used_shared:
+            gF = self.lqr_shared.backward_numpy(grad_x, grad_u)[3].sum(0)           # sum over t of dF [T-1, n, s]
+        else:
+            gF = self.lqr_layer.backward_reduced_numpy(grad_x, grad_u)[3]           # (dx0, sum dC, sum dc, sum dF, sum df)
+        self.A.grad, self.B.grad = gF[:, :n].copy(), gF[:, n:].copy()
         return self.A.grad, self.B.grad
 
 
 class LqrNet_cost_dx(NetLinkBase):
-    """Learn A, B, C, c (reference :201-248; C = I + 0.2 randn is NOT symmetric, Q10)."""
+    """Learn A, B, C, c (reference :201-248; C = I + 0.2 randn is NOT symmetric, Q10).  The layer is DiffLqrShared with
+    C [T,s,s], c [T,s] and [A B] [T-1,n,s] broadcast over time only (util.expand_batch, so Chainer sums their gradients
+    over t); x_init and f stay per element.  With f None the forward is one Riccati sweep plus the rollout.
+    `backward_numpy` sums dC, dc and dF over t on the host."""
 
     def __init__(self, T, n_batch, n_state, n_ctrl, seed):
         super().__init__()
@@ -315,17 +361,19 @@ class LqrNet_cost_dx(NetLinkBase):
             self.B = Parameter(np.random.randn(n_state, n_ctrl).astype("float"))
             self.C = Parameter(np.eye(self.n_sc).astype("float") + 0.2 * np.random.randn(self.n_sc, self.n_sc).astype("float"))
             self.c = Parameter(np.random.randn(self.n_sc).astype("float"))
-        self.lqr_layer = DiffLqr(T, n_batch, n_state, n_ctrl)
+        self.lqr_layer = DiffLqrShared(T, n_batch, n_state, n_ctrl)
 
     def forward(self, inputs):
         x_init, f = inputs
-        large_f = expand_time_batch(_cat_ab(self.A, self.B), self.T - 1, self.n_batch)
-        C = expand_time_batch(self.C, self.T, self.n_batch)
-        c = expand_time_batch(self.c, self.T, self.n_batch)
+        large_f = expand_batch(_cat_ab(self.A, self.B), self.T - 1)
+        C = expand_batch(self.C, self.T)
+        c = expand_batch(self.c, self.T)
         return self.lqr_layer.apply((x_init, C, c, large_f, f))
 
     def backward_numpy(self, grad_x, grad_u):
-        g = self.lqr_layer.backward_reduced_numpy(grad_x, grad_u)
-        self.C.grad, self.c.grad = g[1].copy(), g[2].copy()
-        self.A.grad, self.B.grad = g[3][:, :self.n_state].copy(), g[3][:, self.n_state:].copy()
+        g = self.lqr_layer.backward_numpy(grad_x, grad_u)                   # (dx0, dC [T,s,s], dc [T,s], dF, df)
+        n = self.n_state
+        self.C.grad, self.c.grad = g[1].sum(0), g[2].sum(0)
+        gF = g[3].sum(0)
+        self.A.grad, self.B.grad = gF[:, :n].copy(), gF[:, n:].copy()
         return self.A.grad, self.B.grad, self.C.grad, self.c.grad

@@ -179,6 +179,35 @@ int dmpc_lqr_adjoint_shared(dmpc_handle h, int dtype, int T, int B, int n, int m
                             void* d_ws, size_t ws_bytes,
                             void* d_dx0, void* d_dC, void* d_dc, void* d_dF, void* d_df, int flags, void* stream);
 
+/* ---- the same with c shared by the batch as well (LqrNet_cost_dx, differentiable_lqr.py:237-248, and LqrNet on a batch
+ *      whose c does not vary, :186-198: one learned c broadcast over [T, B] with util.expand_time_batch) ----------------- */
+/* bits of `share` */
+enum { DMPC_SHARE_C = 1 };  /* d_c is [T,s], one block per step for every element; d_dc is [T,s] = sum_b dc_b */
+
+/*
+ * The three calls above with one more argument, `share`; share = 0 is exactly the call above.  With DMPC_SHARE_C:
+ *   - d_c[T,s] replaces the [T,B,s] tensor the reference builds with expand_time_batch (the host never broadcasts it);
+ *   - dmpc_lqr_adjoint_shared_ex writes d_dc[T,s] = sum_b dtau_{t,b} (the reference's dc = dtau, :140, summed as the
+ *     backward of the broadcast does), in a fixed order (deterministic).  d_dc may be NULL; no per-element dc is written;
+ *   - with d_f == NULL as well, every element has the same k_t: the one Riccati sweep computes it and the forward only
+ *     rolls the batch out (no per-element vector sweep).  With d_f given, the vector sweep runs on the shared c.
+ * f stays per element (d_f[T-1,B,n]) or NULL.  The workspace size depends on `share` (it holds a [T,B,s] staging region
+ * for the adjoint with DMPC_SHARE_C): size it with dmpc_lqr_shared_workspace_bytes_ex and the same `share`.
+ * Unknown bits in `share`: DMPC_ERR_UNSUPPORTED.
+ */
+int dmpc_lqr_shared_workspace_bytes_ex(int dtype, int T, int B, int n, int m, int share, size_t* bytes);
+
+int dmpc_lqr_solve_shared_ex(dmpc_handle h, int dtype, int T, int B, int n, int m,
+                             const void* d_x0, const void* d_C, const void* d_c, const void* d_F, int F_T, const void* d_f,
+                             void* d_x, void* d_u, void* d_ws, size_t ws_bytes, int share, void* stream);
+
+int dmpc_lqr_adjoint_shared_ex(dmpc_handle h, int dtype, int T, int B, int n, int m,
+                               const void* d_C, const void* d_c, const void* d_F, int F_T,
+                               const void* d_x, const void* d_u, const void* d_gx, const void* d_gu,
+                               void* d_ws, size_t ws_bytes,
+                               void* d_dx0, void* d_dC, void* d_dc, void* d_dF, void* d_df, int flags, int share,
+                               void* stream);
+
 /* ---- PNQP (replaces PNQP, mpc/pnqp.py:37-201) ---------------------------------------------- */
 /*
  * Batched projected-Newton box QP: min 0.5 x^T H x + q^T x  s.t. lower <= x <= upper.
