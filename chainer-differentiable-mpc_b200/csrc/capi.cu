@@ -43,6 +43,13 @@ inline bool adjoint_fused_available(int n, int m) {
   return false;
 }
 inline size_t fac_elems_per_step(int n, int m) { return (size_t)(m * m + n * m); }
+// the per-element Riccati kernels, or the large-system kernels where those do not fit (DESIGN.md §4.8)
+template <typename R>
+int solve_launch(const LqrParams<R>& p, cudaStream_t st, long long* nl) {
+  if (lqr_large_solve_selected<R>(p.n, p.m, p.flags)) return launch_lqr_large_solve<R>(p, st, nl);
+  return launch_lqr_solve<R>(p, st, nl);
+}
+const char* kLargeUnsupported = "shape beyond the per-element kernels' shared memory and the large-system kernels' range (n <= 128, m <= 32)";
 }  // namespace
 
 template <typename R>
@@ -60,8 +67,8 @@ static int lqr_solve_impl(dmpc_handle h, int T, int B, int n, int m, const void*
   p.c_scale = R(1);
   p.x = (R*)x; p.u = (R*)u; p.Ks = (R*)Ks; p.ks = (R*)ks; p.fac = (R*)fac;
   if ((p.flags & LQR_SAVE_FAC) && adjoint_fused_available(n, m)) p.Vsave = (R*)fac + (size_t)T * B * fac_elems_per_step(n, m);
-  int rc = launch_lqr_solve<R>(p, st, &h->launches);
-  if (rc) h->err = "lqr_solve launch failed";
+  int rc = solve_launch<R>(p, st, &h->launches);
+  if (rc) h->err = rc == DMPC_ERR_UNSUPPORTED ? std::string("lqr_solve: ") + kLargeUnsupported : "lqr_solve launch failed";
   return rc;
 }
 
@@ -97,11 +104,14 @@ static int lqr_adjoint_impl(dmpc_handle h, int T, int B, int n, int m, const voi
     }
     return rc;
   }
-  if (!(flags & DMPC_ADJ_STAGE_OUT_ONLY)) {
+  const int stage = (flags & DMPC_ADJ_STAGE_OUT_ONLY) ? 2 : ((flags & DMPC_ADJ_STAGE_DTAU_ONLY) ? 1 : 0);
+  const bool large = lqr_large_adjoint_selected<R>(n, m, partials != nullptr);
+  if (large && !lqr_large_shape_ok(n, m)) return fail(h, DMPC_ERR_UNSUPPORTED, (std::string("lqr_adjoint: ") + kLargeUnsupported).c_str());
+  if (!large && !(flags & DMPC_ADJ_STAGE_OUT_ONLY)) {
     rc = launch_lqr_dtau<R>(d, st, &h->launches);
     if (rc) { h->err = "lqr_dtau launch failed"; return rc; }
   }
-  if (flags & DMPC_ADJ_STAGE_DTAU_ONLY) return rc;
+  if (!large && (flags & DMPC_ADJ_STAGE_DTAU_ONLY)) return rc;
   AdjOutParams<R> a;
   memset(&a, 0, sizeof(a));
   a.T = T; a.B = B; a.n = n; a.m = m; a.F_T = T - 1;
@@ -110,8 +120,14 @@ static int lqr_adjoint_impl(dmpc_handle h, int T, int B, int n, int m, const voi
   a.dtau = (const R*)dc; a.gx = (const R*)gx; a.gu = (const R*)gu;
   a.dx0 = (R*)dx0; a.dC = (R*)dC; a.dc = (R*)dc; a.dF = (R*)dF; a.df = (R*)df;
   if (partials) { a.flags |= ADJ_REDUCE_TB; a.red = (R*)partials; }
-  rc = launch_adjoint_out<R>(a, st, &h->launches);
-  if (rc) { h->err = "adjoint_out launch failed"; return rc; }
+  if (large) {
+    rc = launch_lqr_large_adjoint<R>(a, (const R*)Ks, (const R*)fac, stage, st, &h->launches);
+    if (rc) { h->err = "lqr_adjoint large-system launch failed"; return rc; }
+    if (stage == 1) return rc;
+  } else {
+    rc = launch_adjoint_out<R>(a, st, &h->launches);
+    if (rc) { h->err = "adjoint_out launch failed"; return rc; }
+  }
   if (partials) {
     rc = launch_reduce_partials<R>((const R*)partials, B, adj_red_elems(n, m), (R*)sums, st, &h->launches);
     if (rc) h->err = "reduce_partials launch failed";
@@ -383,7 +399,7 @@ static int lqr_solve_shared_impl(dmpc_handle h, int T, int B, int n, int m, cons
   p.T = T; p.B = 1; p.n = n; p.m = m; p.flags = LQR_DO_FACTOR | LQR_SAVE_FAC;
   p.C = (const R*)C; p.c = roll_only ? (const R*)c : (const R*)(w + W.c0); p.F = (const R*)F; p.c_scale = R(1);
   p.Ks = (R*)(w + W.Ks); p.ks = (R*)(w + W.ks); p.fac = (R*)(w + W.fac); p.Vsave = (R*)(w + W.V);
-  int rc = launch_lqr_solve<R>(p, st, &h->launches);
+  int rc = solve_launch<R>(p, st, &h->launches);
   if (rc) return fail(h, rc, rc == DMPC_ERR_UNSUPPORTED ? "lqr_solve_shared: no Riccati kernel for this shape" : "lqr_solve_shared: sweep launch failed");
   LqrSharedParams<R> q;
   memset(&q, 0, sizeof(q));

@@ -297,6 +297,16 @@ def _cat_ab(A, B):
     return np.concatenate((A.array, B.array), axis=1)
 
 
+def _shared_fits(dtype, T, B, n, m, share=None):
+    """False when the shared path's chunk kernels cannot hold the shape (dmpc_lqr_shared_workspace_bytes[_ex] reports
+    DMPC_ERR_UNSUPPORTED); the per-element path (DiffLqr) runs every n <= 128, m <= 32."""
+    try:
+        _native.default_context().lqr_shared_workspace_bytes(dtype, T, B, n, m, share)
+    except _native.DiffMpcError:
+        return False
+    return True
+
+
 def _batch_invariant(C):
     """True when C [T,B,...] is a plain array whose entries do not vary along the batch axis: a stride-0 broadcast, or
     (checked second) a copy of C[:, :1]."""
@@ -328,7 +338,8 @@ class LqrNet(NetLinkBase):
 
     def forward(self, inputs):
         x_init, C, c, f = inputs
-        self._used_shared = _batch_invariant(C)
+        self._used_shared = _batch_invariant(C) and _shared_fits(np.float64, self.T, self.n_batch, self.n_state,
+                                                                 self.n_ctrl)
         if self._used_shared:
             large_f = expand_batch(_cat_ab(self.A, self.B), self.T - 1)             # [T-1, n, s]
             return self.lqr_shared.apply((x_init, np.ascontiguousarray(C[:, 0]), c, large_f, f))
@@ -361,18 +372,30 @@ class LqrNet_cost_dx(NetLinkBase):
             self.B = Parameter(np.random.randn(n_state, n_ctrl).astype("float"))
             self.C = Parameter(np.eye(self.n_sc).astype("float") + 0.2 * np.random.randn(self.n_sc, self.n_sc).astype("float"))
             self.c = Parameter(np.random.randn(self.n_sc).astype("float"))
-        self.lqr_layer = DiffLqrShared(T, n_batch, n_state, n_ctrl)
+        # shapes beyond the shared path's chunk kernels: host broadcast over [T, B], DiffLqr and its fused reduction
+        self._shared = _shared_fits(np.float64, T, n_batch, n_state, n_ctrl, _native.SHARE_C)
+        self.lqr_layer = (DiffLqrShared if self._shared else DiffLqr)(T, n_batch, n_state, n_ctrl)
 
     def forward(self, inputs):
         x_init, f = inputs
+        if not self._shared:
+            large_f = expand_time_batch(_cat_ab(self.A, self.B), self.T - 1, self.n_batch)
+            C = expand_time_batch(self.C, self.T, self.n_batch)
+            c = expand_time_batch(self.c, self.T, self.n_batch)
+            return self.lqr_layer.apply((x_init, C, c, large_f, f))
         large_f = expand_batch(_cat_ab(self.A, self.B), self.T - 1)
         C = expand_batch(self.C, self.T)
         c = expand_batch(self.c, self.T)
         return self.lqr_layer.apply((x_init, C, c, large_f, f))
 
     def backward_numpy(self, grad_x, grad_u):
-        g = self.lqr_layer.backward_numpy(grad_x, grad_u)                   # (dx0, dC [T,s,s], dc [T,s], dF, df)
         n = self.n_state
+        if not self._shared:
+            g = self.lqr_layer.backward_reduced_numpy(grad_x, grad_u)       # (dx0, sum dC, sum dc, sum dF, sum df)
+            self.C.grad, self.c.grad = g[1].copy(), g[2].copy()
+            self.A.grad, self.B.grad = g[3][:, :n].copy(), g[3][:, n:].copy()
+            return self.A.grad, self.B.grad, self.C.grad, self.c.grad
+        g = self.lqr_layer.backward_numpy(grad_x, grad_u)                   # (dx0, dC [T,s,s], dc [T,s], dF, df)
         self.C.grad, self.c.grad = g[1].sum(0), g[2].sum(0)
         gF = g[3].sum(0)
         self.A.grad, self.B.grad = gF[:, :n].copy(), gF[:, n:].copy()

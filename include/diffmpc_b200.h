@@ -108,7 +108,7 @@ long long dmpc_launch_count(dmpc_handle h);
 /* ---- LQR (replaces LqrRecursion, lqr/lqr_recursion.py:18-209) ------------------------ */
 /* elements (not bytes) of the factor cache written with DMPC_LQR_SAVE_FAC: Quu_t^-1 | Qxu_t per (t,b) [T,B,m*m+n*m], then
  * the value function V_t | v_t per (t,b) [T,B,n*n+n] (written for the shapes whose adjoint runs as two sweeps on
- * lambda_t = V_t x_t + v_t, today n=32/m=8; reserved otherwise).  Opaque to the caller: allocate, pass to lqr_solve, pass
+ * lambda_t = V_t x_t + v_t, today n=32/m=8, and by the large-system kernels; reserved otherwise).  Opaque to the caller: allocate, pass to lqr_solve, pass
  * on to lqr_adjoint. */
 size_t dmpc_lqr_fac_elems(int T, int B, int n, int m);
 
@@ -121,6 +121,11 @@ size_t dmpc_lqr_fac_elems(int T, int B, int n, int m);
  * Alignment: any alignment of the element type is accepted.  The n=32/m=8 tensor-core kernel moves C, c, F, f, Ks, ks and
  * the factor cache with 16-byte asynchronous copies; when one of those pointers is not 16-byte aligned the call is served
  * by the generic kernel instead (same results, slower) - cudaMalloc'ed buffers and torch tensors are always aligned.
+ * Shapes: any T, B >= 1 and 1 <= m <= 32, 1 <= n <= 128 in both dtypes.  Systems whose per-element layout does not fit one
+ * CTA's shared memory (fp64 with SAVE_FAC from n = 64 / 58 / 52 / 38 at m = 1 / 8 / 16 / 32; fp32 from n = 90 / 85 / 78 / 65)
+ * run the tile-parallel kernels of DESIGN.md 4.8, which allocate fp64 scratch stream-ordered on `stream` (up to
+ * 8*(n(n+1) + s(s+1) + 2m(n+1)) bytes per element).  m > 32, or n > 128 where the per-element kernels do not fit:
+ * DMPC_ERR_UNSUPPORTED, nothing launched.
  */
 int dmpc_lqr_solve(dmpc_handle h, int dtype, int T, int B, int n, int m,
                    const void* d_x0, const void* d_C, const void* d_c,
@@ -134,6 +139,9 @@ int dmpc_lqr_solve(dmpc_handle h, int dtype, int T, int B, int n, int m,
  * the inputs: d_dx0[B,n] d_dC[T,B,s,s] d_dc[T,B,s] d_dF[T-1,B,n,s] d_df[T-1,B,n] (nullable).
  * With DMPC_ADJ_STRICT_REFERENCE the reference's dC / df quirks (Q1, Q2) are reproduced;
  * without it the mathematically correct gradients are returned.
+ * Shapes: as dmpc_lqr_solve; the factor cache of either kernel family is accepted.  Where the per-element adjoint kernels
+ * do not fit shared memory the large-system kernels run (fp64 scratch of 16*T*B*n bytes, stream-ordered); outside
+ * n <= 128, m <= 32 at such shapes: DMPC_ERR_UNSUPPORTED, nothing launched.
  */
 int dmpc_lqr_adjoint(dmpc_handle h, int dtype, int T, int B, int n, int m,
                      const void* d_C, const void* d_c, const void* d_F,
@@ -153,7 +161,10 @@ int dmpc_lqr_adjoint(dmpc_handle h, int dtype, int T, int B, int n, int m,
  * gradients summed over the batch.  C need not be symmetric.
  * The workspace (dmpc_lqr_shared_workspace_bytes, any alignment) holds the matrices of the one Riccati sweep the whole
  * batch needs (K_t, Quu_t^-1, Qxu_t, V_t: a few KB to ~100 KB) and the per-chunk partial sums of the adjoint; its size
- * depends on (dtype, T, B, n, m).  m > 32 and shapes too large for the chunk kernels: DMPC_ERR_UNSUPPORTED.
+ * depends on (dtype, T, B, n, m).  m > 32 and shapes too large for the chunk kernels: DMPC_ERR_UNSUPPORTED (at NB = 8 the
+ * chunk kernels hold fp64 n <= 74 / 70 / 64 / 53 and fp32 n <= 109 / 105 / 100 / 88 at m = 1 / 8 / 16 / 32); the one
+ * Riccati sweep runs at any shape dmpc_lqr_solve runs.  The MPC step, dmpc_lqr_active_solve, PNQP and BoxDDP keep their
+ * per-element kernels only and return DMPC_ERR_UNSUPPORTED where those do not fit.
  */
 int dmpc_lqr_shared_workspace_bytes(int dtype, int T, int B, int n, int m, size_t* bytes);
 
@@ -340,6 +351,8 @@ int dmpc_boxddp_solve(dmpc_handle h, int dtype, int T, int B, int n, int m,
  *   d_sums[dmpc_reduced_grad_elems(n,m)] = (sum dC [s,s] | sum dc [s] | sum dF [n,s] | sum df [n]) over (t,b),
  *   summed in a fixed order (deterministic); d_dx0[B,n] stays per element.
  * The result feeds the NCCL all-reduce of the training step directly (a few hundred doubles per rank).
+ * dmpc_lqr_adjoint_reduced covers the shapes of dmpc_lqr_adjoint (its per-element sums need more shared memory, so it moves
+ * to the large-system kernels first: fp64 (64, 8) already does).  dmpc_mpc_step_backward_reduced does not.
  */
 /* util.expand_time_batch on the device (reference util.py:361-377; callers differentiable_lqr.py:186-198,
  * mpc_net.py:78-80, il_env.py:120-129): d_dst[t][b][0..count) = d_src[0..count) for t < T, b < B.  The forward half of the
