@@ -157,7 +157,7 @@ static int mpc_forward_impl(dmpc_handle h, int T, int B, int n, int m, const voi
   p.costs = (R*)costs; p.old_costs = (R*)old_costs; p.alphas = (R*)alphas; p.n_qp = (int*)n_qp;
   p.free_mask = (unsigned char*)free_m; p.n_ls = (int*)n_ls; p.flags = (int*)flags; p.skip = skip;
   int rc = launch_mpc_forward<R>(p, st, &h->launches);
-  if (rc) h->err = rc == DMPC_ERR_UNSUPPORTED ? "mpc_step_forward: unsupported shape / batch coupling needs the batch in one CTA" : "mpc_step_forward launch failed";
+  if (rc) h->err = rc == DMPC_ERR_UNSUPPORTED ? "mpc_step_forward: unsupported shape (n <= 128, m <= 32) or batch coupling (the batch must fit one CTA or cluster, and past the per-element kernels' shared memory only element coupling runs)" : "mpc_step_forward launch failed";
   return rc;
 }
 
@@ -167,6 +167,10 @@ static int mpc_backward_impl(dmpc_handle h, int T, int B, int n, int m, const vo
                              const void* gu, void* wsK, void* wsk, void* wsd, void* act, void* dx0, void* dC,
                              void* dc, void* dF, void* df, cudaStream_t st, void* partials = nullptr,
                              void* sums = nullptr) {
+  // the masked solve and the adjoint each take the large-system kernels where their own per-element kernel does not fit
+  const bool large_adj = lqr_large_adj_out_selected<R>(n, m, partials != nullptr);
+  if ((lqr_large_solve_selected<R>(n, m, LQR_DO_FACTOR | LQR_DO_ROLLOUT | LQR_MASKED) || large_adj) && !lqr_large_shape_ok(n, m))
+    return fail(h, DMPC_ERR_UNSUPPORTED, (std::string("mpc_step_backward: ") + kLargeUnsupported).c_str());
   int rc = launch_active_mask<R>((const R*)u, (const R*)lo, (const R*)hi, (unsigned char*)act, (size_t)T * B * m, st, &h->launches);
   if (rc) { h->err = "active_mask launch failed"; return rc; }
   if (cudaMemsetAsync(dx0, 0, (size_t)B * n * sizeof(R), st) != cudaSuccess) return DMPC_ERR_CUDA;
@@ -178,7 +182,7 @@ static int mpc_backward_impl(dmpc_handle h, int T, int B, int n, int m, const vo
   p.C = (const R*)C; p.c = nullptr; p.cx = (const R*)gx; p.cu = (const R*)gu; p.c_scale = R(-1);   // c := -d_taus (:374)
   p.F = (const R*)F; p.f = nullptr; p.active = (const unsigned char*)act;
   p.Ks = (R*)wsK; p.ks = (R*)wsk; p.tau_out = (R*)wsd;
-  rc = launch_lqr_solve<R>(p, st, &h->launches);
+  rc = solve_launch<R>(p, st, &h->launches);
   if (rc) { h->err = "lqr_active launch failed"; return rc; }
   AdjOutParams<R> a;
   memset(&a, 0, sizeof(a));
@@ -188,8 +192,8 @@ static int mpc_backward_impl(dmpc_handle h, int T, int B, int n, int m, const vo
   a.dtau = (const R*)wsd; a.gx = (const R*)gx; a.gu = (const R*)gu;
   a.dx0 = (R*)dx0; a.dC = (R*)dC; a.dc = (R*)dc; a.dF = (R*)dF; a.df = (R*)df;
   if (partials) { a.flags |= ADJ_REDUCE_TB; a.red = (R*)partials; }
-  rc = launch_adjoint_out<R>(a, st, &h->launches);
-  if (rc) { h->err = "adjoint_out launch failed"; return rc; }
+  rc = large_adj ? launch_lqr_large_adjoint<R>(a, nullptr, nullptr, 2, st, &h->launches) : launch_adjoint_out<R>(a, st, &h->launches);
+  if (rc) { h->err = large_adj ? "mpc_step_backward large-system adjoint launch failed" : "adjoint_out launch failed"; return rc; }
   if (partials) {
     rc = launch_reduce_partials<R>((const R*)partials, B, adj_red_elems(n, m), (R*)sums, st, &h->launches);
     if (rc) h->err = "reduce_partials launch failed";
@@ -207,8 +211,8 @@ static int lqr_active_impl(dmpc_handle h, int T, int B, int n, int m, const void
   p.flags = LQR_DO_FACTOR | LQR_DO_ROLLOUT | LQR_MASKED;
   p.x0 = (const R*)x0; p.C = (const R*)C; p.c = (const R*)c; p.c_scale = R(1); p.F = (const R*)F; p.f = (const R*)f;
   p.active = (const unsigned char*)act; p.x = (R*)x; p.u = (R*)u; p.Ks = (R*)Ks; p.ks = (R*)ks;
-  int rc = launch_lqr_solve<R>(p, st, &h->launches);
-  if (rc) h->err = "lqr_active launch failed";
+  int rc = solve_launch<R>(p, st, &h->launches);
+  if (rc) h->err = rc == DMPC_ERR_UNSUPPORTED ? std::string("lqr_active: ") + kLargeUnsupported : "lqr_active launch failed";
   return rc;
 }
 
@@ -237,7 +241,7 @@ static int traj_impl(dmpc_handle h, int T, int B, int n, int m, int dynamics, co
   for (int i = 0; i < 5; ++i) p.dyn_params[i] = dynp ? (R)dynp[i] : R(0);
   p.x = (R*)x; p.Fout = (R*)Fo; p.fout = (R*)fo; p.skip = skip;
   int rc = launch_traj<R>(p, st, &h->launches);
-  if (rc) h->err = "get_traj launch failed";
+  if (rc) h->err = rc == DMPC_ERR_UNSUPPORTED ? std::string("get_traj: ") + kLargeUnsupported : "get_traj launch failed";
   return rc;
 }
 

@@ -30,12 +30,14 @@ template <typename R> int launch_reduce_partials(const R* red, int B, int rsz, R
 
 constexpr int kMaxSmem = 227 * 1024;
 
-// Systems whose per-element step does not fit one CTA (lqr_large_launch.cu, DESIGN.md §4.8).  *_selected: the
-// per-element kernels would return DMPC_ERR_UNSUPPORTED for shared memory (MASKED calls never select them);
-// the launchers return DMPC_ERR_UNSUPPORTED outside n <= 128, m <= 32 before launching anything.
+// Systems whose per-element step does not fit one CTA (lqr_large_launch.cu, DESIGN.md §4.8, §4.9).  *_selected: the
+// per-element kernels would return DMPC_ERR_UNSUPPORTED for shared memory; the launchers return DMPC_ERR_UNSUPPORTED
+// outside n <= 128, m <= 32 before launching anything.
 inline bool lqr_large_shape_ok(int n, int m) { return n >= 1 && n <= 128 && m >= 1 && m <= 32; }
 template <typename R> bool lqr_large_solve_selected(int n, int m, int lqr_flags);
 template <typename R> bool lqr_large_adjoint_selected(int n, int m, bool reduced);
+// adjoint_out_kernel alone (lambda / d-lambda stage of the MPC step backward)
+template <typename R> bool lqr_large_adj_out_selected(int n, int m, bool reduced);
 template <typename R> int launch_lqr_large_solve(const LqrParams<R>& p, cudaStream_t st, long long* nlaunch);
 // stage: 0 = whole adjoint, 1 = d-tau sweeps only, 2 = lambda recursion + gradients only
 template <typename R> int launch_lqr_large_adjoint(const AdjOutParams<R>& a, const R* Ks, const R* fac, int stage,

@@ -48,6 +48,7 @@ struct LqrParams {
   R* fac;        // [T,B,m*m + n*m]  (Quu^-1 | Qxu) or nullptr
   R* tau_out;    // [T,B,s] or nullptr: rollout also writes [x;u] concatenated
   R* Vsave;      // [T,B,n*n+n] or nullptr: V_t | v_t of the Riccati sweep (t >= 1) for adjoint_fused_kernel
+  const int* skip;  // large-system Q / V steps only (device flag, nullable): non-zero -> the launch is a no-op
 };
 
 // shared-memory layout of one element's region for lqr_solve_kernel (offsets in reals)

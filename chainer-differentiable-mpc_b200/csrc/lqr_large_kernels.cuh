@@ -80,16 +80,23 @@ __device__ __forceinline__ void cta_coldot(int I, int K, FA A, const double* x, 
 
 // ---------------------------------------------------------------------------------------------- forward
 // Q step of time t.  Column j < s of [Q | q] is column j of Q, column s is q.
+// c is p.c, or the split form p.cx | p.cu (NULL parts are zero), times p.c_scale.
 template <typename R>
 __global__ void __launch_bounds__(kLargeThreads) lqr_large_q_kernel(LqrParams<R> p, LargeFwdWs w, int t) {
   extern __shared__ double Wp[];                        // [n][kLargePanel]: W(:, panel)
+  if (p.skip && *p.skip) return;
   const int n = p.n, m = p.m, s = n + m, e = blockIdx.x, j0 = blockIdx.y * kLargePanel;
   const int J = min(kLargePanel, s + 1 - j0);
   const size_t idx = (size_t)t * p.B + e;
   const R* Ct = p.C + idx * s * s;
-  const R* ct = p.c + idx * s;
+  const double cs = (double)p.c_scale;
+  auto cval = [&](int i) -> double {
+    if (p.c) return cs * (double)p.c[idx * s + i];
+    const R* part = i < n ? p.cx : p.cu;
+    return part ? cs * (double)(i < n ? part[idx * n + i] : part[idx * m + i - n]) : 0.0;
+  };
   double* Q = w.Q + (size_t)e * s * (s + 1);
-  auto base = [&](int i, int j) -> double { return j0 + j < s ? (double)Ct[i * s + j0 + j] : (double)ct[i]; };
+  auto base = [&](int i, int j) -> double { return j0 + j < s ? (double)Ct[i * s + j0 + j] : cval(i); };
   auto out = [&](int i, int j, double v) { Q[i * (s + 1) + j0 + j] = v; };
   if (t == p.T - 1) {
     auto zero = [](int, int) -> double { return 0.0; };
@@ -120,17 +127,27 @@ __global__ void __launch_bounds__(kLargeThreads) lqr_large_factor_kernel(LqrPara
   double* H = fsm;
   double* Rhs = fsm + m * m;
   const double* Q = w.Q + (size_t)e * s * ldq;
-  for (int o = threadIdx.x; o < m * m; o += blockDim.x) { const int i = o / m, j = o - i * m; H[o] = Q[(n + i) * ldq + n + j]; }
+  const size_t idx = (size_t)t * p.B + e;
+  // LQR_MASKED (LQR_active, active_constrained_lqr.py:113-126): cross terms of active controls zeroed with 1e-8 on their
+  // diagonal, their rows of Qux and qu zeroed; P below keeps the unmasked Quu, Qux, qu
+  const unsigned char* act = (p.flags & LQR_MASKED) ? p.active + idx * m : nullptr;
+  for (int o = threadIdx.x; o < m * m; o += blockDim.x) {
+    const int i = o / m, j = o - i * m;
+    double hv = Q[(n + i) * ldq + n + j];
+    if (act && (act[i] || act[j])) hv = i == j && act[i] ? 1e-8 : 0.0;
+    H[o] = hv;
+  }
   for (int o = threadIdx.x; o < m * ldr; o += blockDim.x) {
     const int i = o / ldr, j = o - i * ldr;
-    Rhs[o] = j < n ? -Q[(n + i) * ldq + j] : (j == n ? -Q[(n + i) * ldq + s] : (j - n - 1 == i ? 1.0 : 0.0));
+    double rv = j < n ? -Q[(n + i) * ldq + j] : (j == n ? -Q[(n + i) * ldq + s] : (j - n - 1 == i ? 1.0 : 0.0));
+    if (act && j <= n && act[i]) rv = 0.0;
+    Rhs[o] = rv;
   }
   __syncthreads();
   const Grp<kLargeThreads> g;
   g_lu_factor<kLargeThreads, kLargeMaxM>(g, m, H, m, Rhs, ldr, ldr, (int*)nullptr);
   g_back_subst(g, m, H, m, Rhs, ldr, ldr);
   __syncthreads();
-  const size_t idx = (size_t)t * p.B + e;
   double* KK = w.KK + (size_t)e * m * (n + 1);
   double* P = w.P + (size_t)e * m * (n + 1);
   for (int o = threadIdx.x; o < m * (n + 1); o += blockDim.x) {
@@ -153,6 +170,7 @@ __global__ void __launch_bounds__(kLargeThreads) lqr_large_factor_kernel(LqrPara
 // Vdst (nullable): V_t | v_t per (t, b) in the factor-cache layout.
 template <typename R>
 __global__ void __launch_bounds__(kLargeThreads) lqr_large_v_kernel(LqrParams<R> p, LargeFwdWs w, R* Vdst, int t) {
+  if (p.skip && *p.skip) return;
   const int n = p.n, m = p.m, s = n + m, e = blockIdx.x, j0 = blockIdx.y * kLargePanel, ldq = s + 1;
   const int J = min(kLargePanel, n + 1 - j0);
   const double* Q = w.Q + (size_t)e * s * ldq;
@@ -171,7 +189,8 @@ __global__ void __launch_bounds__(kLargeThreads) lqr_large_v_kernel(LqrParams<R>
              });
 }
 
-// Rollout: one CTA per element over the horizon.
+// Rollout: one CTA per element over the horizon.  LQR_MASKED: u of active controls is zero
+// (active_constrained_lqr.py:175); tau_out (nullable) gets [x; u].
 template <typename R>
 __global__ void __launch_bounds__(kLargeThreads) lqr_large_rollout_kernel(LqrParams<R> p) {
   extern __shared__ double rsm[];
@@ -184,11 +203,14 @@ __global__ void __launch_bounds__(kLargeThreads) lqr_large_rollout_kernel(LqrPar
     const size_t idx = (size_t)t * p.B + e;
     const R* Kt = p.Ks + idx * m * n;
     const R* kt = p.ks + idx * m;
+    const unsigned char* act = (p.flags & LQR_MASKED) ? p.active + idx * m : nullptr;
     cta_rowdot(m, n, [&](int i, int k) -> double { return (double)Kt[i * n + k]; }, xu,
-               [&](int i) -> double { return (double)kt[i]; }, [&](int i, double v) { xu[n + i] = v; });
+               [&](int i) -> double { return (double)kt[i]; },
+               [&](int i, double v) { xu[n + i] = act && act[i] ? 0.0 : v; });
     __syncthreads();
-    for (int o = threadIdx.x; o < n; o += blockDim.x) p.x[idx * n + o] = (R)xu[o];
-    for (int o = threadIdx.x; o < m; o += blockDim.x) p.u[idx * m + o] = (R)xu[n + o];
+    if (p.x) for (int o = threadIdx.x; o < n; o += blockDim.x) p.x[idx * n + o] = (R)xu[o];
+    if (p.u) for (int o = threadIdx.x; o < m; o += blockDim.x) p.u[idx * m + o] = (R)xu[n + o];
+    if (p.tau_out) for (int o = threadIdx.x; o < s; o += blockDim.x) p.tau_out[idx * s + o] = (R)xu[o];
     if (t < T - 1) {
       const R* Ft = p.F + idx * n * s;
       const R* ft = p.f ? p.f + idx * n : nullptr;
@@ -202,8 +224,8 @@ __global__ void __launch_bounds__(kLargeThreads) lqr_large_rollout_kernel(LqrPar
 }
 
 // ---------------------------------------------------------------------------------------------- adjoint
-// One CTA per element; the same three recursions as lqr_dtau_kernel + adjoint_out_kernel (ADJ_NEGATE / ADJ_NEG_RHS
-// are not used by the LQR adjoint):
+// One CTA per element; the same three recursions as lqr_dtau_kernel + adjoint_out_kernel (the MPC step backward runs
+// sweep 3 only, on the masked solve's dtau, with ADJ_NEGATE / ADJ_NEG_RHS as in adjoint_out_kernel):
 //   sweep 1 (t down): q = [gx | gu] + F_t^T v';  k' = -Quu^-1 q_u;  v' = q_x + Qxu k'      (k' parked in dtau[t, n:])
 //   sweep 2 (t up):   du = K_t dx + k';  dtau_t = [dx; du];  dx' = F_t dtau_t
 //   sweep 3 (t down): lambda_t = c_t[:n] + C_t[:n,:] tau_t + F_t[:, :n]^T lambda_{t+1}, d-lambda the same on dtau and gx
@@ -274,7 +296,10 @@ __global__ void __launch_bounds__(kLargeThreads) lqr_large_adj_kernel(AdjOutPara
     cta_rowdot(n, s, [&](int i, int k) -> double { return (double)Ct[i * s + k]; }, dx,
                [&](int i) -> double { return (double)ct[i]; }, [&](int i, double v) { tmp[i] = v; });
     cta_rowdot(n, s, [&](int i, int k) -> double { return (double)Ct[i * s + k]; }, dt,
-               [&](int i) -> double { return a.gx ? (double)a.gx[idx * n + i] : 0.0; }, [&](int i, double v) { tmp2[i] = v; });
+               [&](int i) -> double {
+                 const double gv = a.gx ? (double)a.gx[idx * n + i] : 0.0;
+                 return (a.flags & ADJ_NEG_RHS) ? -gv : gv;
+               }, [&](int i, double v) { tmp2[i] = v; });
     __syncthreads();
     const R* Ft = a.F + idx * n * s;
     const int Kf = t < T - 1 ? n : 0;
@@ -290,37 +315,44 @@ __global__ void __launch_bounds__(kLargeThreads) lqr_large_adj_kernel(AdjOutPara
       dl[o] = dt[o];
       w.lam[idx * n + o] = q[o];
       w.dlam[idx * n + o] = dt[o];
-      if (t == 0) a.dx0[(size_t)e * n + o] = (R)dt[o];
+      if (t == 0) a.dx0[(size_t)e * n + o] = (R)((a.flags & ADJ_NEGATE) ? -dt[o] : dt[o]);
     }
     __syncthreads();
   }
 }
 
-// dC_t, dF_t (t < T-1), df_t (t < T-1) per (t, b); dc_t is dtau_t itself (the caller's dc buffer).
+// dC_t, dF_t (t < T-1), df_t (t < T-1, nullable) per (t, b).  dc_t is dtau_t: the LQR adjoint's dtau is the caller's dc
+// buffer; ADJ_NEGATE (MPC step) writes dc = -dtau and negates every gradient, and F with T rows (F_T == T) gets a zero
+// row T-1 of dF (mpc_step.py:428).
 template <typename R>
 __global__ void __launch_bounds__(kLargeThreads) lqr_large_outer_kernel(AdjOutParams<R> a, LargeAdjWs w) {
   const int n = a.n, m = a.m, s = n + m, e = blockIdx.x, t = blockIdx.y, T = a.T, B = a.B;
   const size_t idx = (size_t)t * B + e;
   const bool quirk_c = (a.flags & ADJ_QUIRK_DC) != 0, quirk_f = (a.flags & ADJ_QUIRK_DF) != 0;
+  const double sgn = (a.flags & ADJ_NEGATE) ? -1.0 : 1.0;
   auto tau = [&](int j) -> double { return j < n ? (double)a.x[idx * n + j] : (double)a.u[idx * m + j - n]; };
   const R* dt = a.dtau + idx * s;
   R* dC = a.dC + idx * s * s;
   for (int o = threadIdx.x; o < s * s; o += blockDim.x) {
     const int i = o / s, j = o - i * s;
     const double x = (double)dt[i] * tau(j), y = tau(i) * (double)dt[j];
-    dC[o] = (R)(quirk_c ? 0.5 * x + y : 0.5 * (x + y));
+    dC[o] = (R)(quirk_c ? 0.5 * x + y : sgn * (0.5 * (x + y)));
   }
-  if (t >= T - 1) return;
+  if (a.dc != a.dtau) for (int o = threadIdx.x; o < s; o += blockDim.x) a.dc[idx * s + o] = (R)(sgn * (double)dt[o]);
+  if (t >= T - 1) {
+    if (a.F_T == T && a.dF) for (int o = threadIdx.x; o < n * s; o += blockDim.x) a.dF[idx * n * s + o] = R(0);
+    return;
+  }
   const double* ln = w.lam + (idx + B) * n;
   const double* dln = w.dlam + (idx + B) * n;
   R* dF = a.dF + idx * n * s;
   for (int o = threadIdx.x; o < n * s; o += blockDim.x) {
     const int i = o / s, j = o - i * s;
-    dF[o] = (R)(dln[i] * tau(j) + ln[i] * (double)dt[j]);
+    dF[o] = (R)(sgn * (dln[i] * tau(j) + ln[i] * (double)dt[j]));
   }
   if (a.df) {
     const double* src = quirk_f ? w.dlam + idx * n : dln;
-    for (int o = threadIdx.x; o < n; o += blockDim.x) a.df[idx * n + o] = (R)src[o];
+    for (int o = threadIdx.x; o < n; o += blockDim.x) a.df[idx * n + o] = (R)(sgn * src[o]);
   }
 }
 
@@ -331,7 +363,8 @@ __global__ void __launch_bounds__(kLargeThreads) lqr_large_red_kernel(AdjOutPara
   const int n = a.n, m = a.m, s = n + m, e = blockIdx.x, j0 = blockIdx.y * kLargePanel, T = a.T, B = a.B;
   const int J = min(kLargePanel, s - j0);
   const bool quirk_c = (a.flags & ADJ_QUIRK_DC) != 0, quirk_f = (a.flags & ADJ_QUIRK_DF) != 0;
-  const double c1 = 0.5, c2 = quirk_c ? 1.0 : 0.5;
+  const double sgn = (a.flags & ADJ_NEGATE) ? -1.0 : 1.0;    // ADJ_NEGATE never comes with the quirks
+  const double c1 = sgn * 0.5, c2 = quirk_c ? 1.0 : sgn * 0.5;
   auto tau = [&](int t, int j) -> double {
     const size_t idx = (size_t)t * B + e;
     return j < n ? (double)a.x[idx * n + j] : (double)a.u[idx * m + j - n];
@@ -351,17 +384,17 @@ __global__ void __launch_bounds__(kLargeThreads) lqr_large_red_kernel(AdjOutPara
   large_gemm(n, J, 2 * T1,
              [&](int i, int k) -> double { return k < T1 ? dlam(k + 1, i) : lam(k - T1 + 1, i); },
              [&](int k, int j) -> double { return k < T1 ? tau(k, j0 + j) : dt(k - T1, j0 + j); },
-             zero, [&](int i, int j, double v) { out[s * s + s + i * s + j0 + j] = (R)v; });
+             zero, [&](int i, int j, double v) { out[s * s + s + i * s + j0 + j] = (R)(sgn * v); });
   if (blockIdx.y != 0) return;
   for (int o = threadIdx.x; o < s + n; o += blockDim.x) {
     double acc = 0.0;
     if (o < s) {
       for (int t = 0; t < T; ++t) acc += dt(t, o);
-      out[s * s + o] = (R)acc;
+      out[s * s + o] = (R)(sgn * acc);
     } else {
       const int i = o - s;
       for (int t = 0; t < T1; ++t) acc += quirk_f ? dlam(t, i) : dlam(t + 1, i);
-      out[s * s + s + n * s + i] = (R)acc;
+      out[s * s + s + n * s + i] = (R)(sgn * acc);
     }
   }
 }

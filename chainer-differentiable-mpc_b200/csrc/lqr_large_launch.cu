@@ -10,9 +10,9 @@ namespace dmpc {
 
 // A call takes these kernels only where the per-element kernels cannot run it for shared memory: the same layout
 // functions and the same kMaxSmem test as do_launch (one element per CTA at s > 24; smaller systems always fit).
+// LQR_MASKED calls (the MPC step backward, LQR_active) are selected by the same test.
 template <typename R>
 bool lqr_large_solve_selected(int n, int m, int flags) {
-  if (flags & LQR_MASKED) return false;
   const LqrLayout L = lqr_layout<R>(n, m, (flags & LQR_SAVE_FAC) != 0, !(flags & LQR_DO_FACTOR));
   return m > 32 || (size_t)L.stride * sizeof(R) > (size_t)kMaxSmem;
 }
@@ -22,6 +22,13 @@ template <typename R>
 bool lqr_large_adjoint_selected(int n, int m, bool reduced) {
   return (size_t)dtau_layout<R>(n, m).stride * sizeof(R) > (size_t)kMaxSmem ||
          (size_t)adj_layout<R>(n, m, reduced).stride * sizeof(R) > (size_t)kMaxSmem;
+}
+
+// The lambda / d-lambda stage alone (the MPC step backward, whose dtau comes from the masked solve): adjoint_out_kernel's
+// layout test.
+template <typename R>
+bool lqr_large_adj_out_selected(int n, int m, bool reduced) {
+  return (size_t)adj_layout<R>(n, m, reduced).stride * sizeof(R) > (size_t)kMaxSmem;
 }
 
 namespace {
@@ -93,6 +100,7 @@ int launch_lqr_large_adjoint(const AdjOutParams<R>& a, const R* Ks, const R* fac
 
 template bool lqr_large_solve_selected<DMPC_REAL>(int, int, int);
 template bool lqr_large_adjoint_selected<DMPC_REAL>(int, int, bool);
+template bool lqr_large_adj_out_selected<DMPC_REAL>(int, int, bool);
 template int launch_lqr_large_solve<DMPC_REAL>(const LqrParams<DMPC_REAL>&, cudaStream_t, long long*);
 template int launch_lqr_large_adjoint<DMPC_REAL>(const AdjOutParams<DMPC_REAL>&, const DMPC_REAL*, const DMPC_REAL*, int, cudaStream_t, long long*);
 

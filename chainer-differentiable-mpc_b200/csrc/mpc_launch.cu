@@ -177,6 +177,8 @@ int launch_mpc_forward<Rr>(const MpcFwdParams<Rr>& p, cudaStream_t st, long long
     return launch_elems(mpc_forward_kernel<Rr, 0, 0, 32, false>, p, 32, sb, p.B, false, st, nl);
   }
   if (batch) return DMPC_ERR_UNSUPPORTED;
+  // one element per CTA does not fit shared memory (launch_elems' test): the host-stepped large-system kernels
+  if (sb > kMpcMaxSmem) return launch_mpc_large_forward<Rr>(p, st, nl);
   return launch_elems(mpc_forward_kernel<Rr, 0, 0, 256, false>, p, 256, sb, p.B, false, st, nl);
 }
 
@@ -207,7 +209,7 @@ int launch_active_mask<Rr>(const Rr* u, const Rr* lo, const Rr* hi, unsigned cha
 
 template <>
 int launch_traj<Rr>(const TrajParams<Rr>& p, cudaStream_t st, long long* nl) {
-  if (p.n + p.m > 64) return DMPC_ERR_UNSUPPORTED;
+  if (p.n + p.m > 64) return launch_traj_large<Rr>(p, st, nl);     // traj_kernel keeps [x; u] in registers
   const int tpb = 64;
   traj_kernel<Rr, 64><<<(p.B + tpb - 1) / tpb, tpb, 0, st>>>(p);
   if (nl) ++*nl;

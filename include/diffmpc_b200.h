@@ -163,8 +163,8 @@ int dmpc_lqr_adjoint(dmpc_handle h, int dtype, int T, int B, int n, int m,
  * batch needs (K_t, Quu_t^-1, Qxu_t, V_t: a few KB to ~100 KB) and the per-chunk partial sums of the adjoint; its size
  * depends on (dtype, T, B, n, m).  m > 32 and shapes too large for the chunk kernels: DMPC_ERR_UNSUPPORTED (at NB = 8 the
  * chunk kernels hold fp64 n <= 74 / 70 / 64 / 53 and fp32 n <= 109 / 105 / 100 / 88 at m = 1 / 8 / 16 / 32); the one
- * Riccati sweep runs at any shape dmpc_lqr_solve runs.  The MPC step, dmpc_lqr_active_solve, PNQP and BoxDDP keep their
- * per-element kernels only and return DMPC_ERR_UNSUPPORTED where those do not fit.
+ * Riccati sweep runs at any shape dmpc_lqr_solve runs.  The MPC step, its backward, dmpc_lqr_active_solve, dmpc_get_traj
+ * (LinDx) and BoxDDP (LinDx) run every n <= 128, m <= 32 as well (DESIGN.md §4.9); dmpc_pnqp stays at m <= 32.
  */
 int dmpc_lqr_shared_workspace_bytes(int dtype, int T, int B, int n, int m, size_t* bytes);
 
@@ -256,6 +256,10 @@ int dmpc_pnqp(dmpc_handle h, int dtype, int B, int m,
  * (line-search passes run: the accepted pass, or max_ls_trials on an element whose line search hit the cap - that one
  * carries DMPC_FLAG_LS_CAPPED and its alpha is the one of the last pass); d_flags[B] int32 (dmpc_elem_flag bits).
  * max_ls_trials caps the per-element line search (the reference's loop has no effective cap, Q5).
+ * Shapes: any T, B >= 1 and 1 <= m <= 32, 1 <= n <= 128 in both dtypes.  Systems whose per-element layout does not fit one
+ * CTA's shared memory (fp64 from n = 57 at m = 8) run on host-stepped large-system kernels (DESIGN.md §4.9): element
+ * coupling and DMPC_DYN_LINEAR only (DMPC_COUPLING_BATCH there returns DMPC_ERR_UNSUPPORTED), every product in fp64, fp32
+ * tensors widened on load and rounded once on store; outside the range DMPC_ERR_UNSUPPORTED, nothing launched.
  */
 int dmpc_mpc_step_forward(dmpc_handle h, int dtype, int T, int B, int n, int m,
                           const void* d_C, const void* d_c, const void* d_F, int F_T, const void* d_f,
@@ -274,6 +278,8 @@ int dmpc_mpc_step_forward(dmpc_handle h, int dtype, int T, int B, int n, int m,
  * (d_active doubles as an output: the active set used).
  * Outputs: d_dx0[B,n] d_dC[T,B,s,s] d_dc[T,B,s] d_dF[F_T,B,n,s] (row T-1 zero-filled when F_T == T, Q8)
  * d_df[T-1,B,n] (NULL when f_hat is None).
+ * Shapes: as dmpc_mpc_step_forward.  The masked solve and the adjoint each take the large-system kernels where their own
+ * per-element kernel does not fit (DESIGN.md §4.9); outside n <= 128, m <= 32 DMPC_ERR_UNSUPPORTED, nothing launched.
  */
 int dmpc_mpc_step_backward(dmpc_handle h, int dtype, int T, int B, int n, int m,
                            const void* d_C, const void* d_c, const void* d_F, int F_T,
@@ -285,6 +291,7 @@ int dmpc_mpc_step_backward(dmpc_handle h, int dtype, int T, int B, int n, int m,
 /*
  * LQR_active.solve_recursion (mpc/active_constrained_lqr.py:195-202) on its own:
  * d_active[T,B,m] uint8 = u_zero_Index.  Same tensors as dmpc_lqr_solve.
+ * Shapes: as dmpc_lqr_solve (the large-system kernels apply the masks where the per-element layout does not fit).
  */
 int dmpc_lqr_active_solve(dmpc_handle h, int dtype, int T, int B, int n, int m,
                           const void* d_x0, const void* d_C, const void* d_c, const void* d_F, int F_T,
@@ -296,6 +303,8 @@ int dmpc_lqr_active_solve(dmpc_handle h, int dtype, int T, int B, int n, int m,
 /*
  * Roll x_{t+1} = dyn(x_t, u_t) from d_x0 under d_u[T,B,m] -> d_x[T,B,n].  For DMPC_DYN_PENDULUM
  * (n=3, m=1) d_Fout[T-1,B,3,4] / d_fout[T-1,B,3] (nullable) receive the analytic linearisation.
+ * Shapes: DMPC_DYN_LINEAR at any n <= 128, m <= 32 (past n + m = 64 one CTA per element, with the row-dot order and
+ * rounding of the large-system line search, so get_traj of its accepted controls reproduces its trajectory bit for bit).
  */
 int dmpc_get_traj(dmpc_handle h, int dtype, int T, int B, int n, int m, int dynamics,
                   const void* d_x0, const void* d_u, const void* d_F, const void* d_f,
@@ -318,6 +327,8 @@ int dmpc_get_traj(dmpc_handle h, int dtype, int T, int B, int n, int m, int dyna
  *            *h_n_iter, *h_status (DMPC_BOXDDP_*), *h_flags (OR of the per-element DMPC_FLAG_* over all steps)
  *   d_ws   : caller-owned workspace of dmpc_boxddp_workspace_bytes() bytes
  * Returns DMPC_ERR_NONFINITE where the reference's NaN asserts would fire (mpc_step.py:284-285).
+ * Shapes: those of dmpc_mpc_step_forward; with DMPC_DYN_LINEAR every n <= 128, m <= 32 (element coupling past the
+ * per-element kernels, DESIGN.md §4.9).
  */
 typedef struct {
   double eps;               /* box_ddp.py:27 eps */
@@ -352,7 +363,8 @@ int dmpc_boxddp_solve(dmpc_handle h, int dtype, int T, int B, int n, int m,
  *   summed in a fixed order (deterministic); d_dx0[B,n] stays per element.
  * The result feeds the NCCL all-reduce of the training step directly (a few hundred doubles per rank).
  * dmpc_lqr_adjoint_reduced covers the shapes of dmpc_lqr_adjoint (its per-element sums need more shared memory, so it moves
- * to the large-system kernels first: fp64 (64, 8) already does).  dmpc_mpc_step_backward_reduced does not.
+ * to the large-system kernels first: fp64 (64, 8) already does).  dmpc_mpc_step_backward_reduced covers the shapes of
+ * dmpc_mpc_step_backward the same way.
  */
 /* util.expand_time_batch on the device (reference util.py:361-377; callers differentiable_lqr.py:186-198,
  * mpc_net.py:78-80, il_env.py:120-129): d_dst[t][b][0..count) = d_src[0..count) for t < T, b < B.  The forward half of the
