@@ -31,24 +31,14 @@ inline int cuda_fail(dmpc_handle h, cudaError_t e, const char* where) {
 }
 #define CK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return cuda_fail(h, e_, #call); } while (0)
 inline int set_dev(dmpc_handle h) { return cudaSetDevice(h->device) == cudaSuccess ? 0 : DMPC_ERR_CUDA; }
-// Shapes whose adjoint runs as two sweeps on the V_t, v_t saved by the forward (lqr_adjoint_fused.cuh).
-// DMPC_ADJ_UNFUSED=1 selects the three-sweep kernels for A/B runs.
-inline bool adjoint_fused_available(int n, int m) {
-  static int off = -1;
-  if (off < 0) { const char* e = getenv("DMPC_ADJ_UNFUSED"); off = (e && e[0] == '1') ? 1 : 0; }
-  if (off) return false;
-#define X(N_, M_) if (n == N_ && m == M_) return true;
-  DMPC_FUSED_SHAPES(X)
-#undef X
-  return false;
+// fn(double{}) or fn(float{}): the typed implementation of an entry point
+template <class Fn>
+int by_dtype(dmpc_handle h, int dtype, Fn fn) {
+  if (dtype == DMPC_F64) return fn(double{});
+  if (dtype == DMPC_F32) return fn(float{});
+  return fail(h, DMPC_ERR_UNSUPPORTED, "dtype");
 }
 inline size_t fac_elems_per_step(int n, int m) { return (size_t)(m * m + n * m); }
-// the per-element Riccati kernels, or the large-system kernels where those do not fit (DESIGN.md §4.8)
-template <typename R>
-int solve_launch(const LqrParams<R>& p, cudaStream_t st, long long* nl) {
-  if (lqr_large_solve_selected<R>(p.n, p.m, p.flags)) return launch_lqr_large_solve<R>(p, st, nl);
-  return launch_lqr_solve<R>(p, st, nl);
-}
 const char* kLargeUnsupported = "shape beyond the per-element kernels' shared memory and the large-system kernels' range (n <= 128, m <= 32)";
 }  // namespace
 
@@ -66,8 +56,8 @@ static int lqr_solve_impl(dmpc_handle h, int T, int B, int n, int m, const void*
   p.x0 = (const R*)x0; p.C = (const R*)C; p.c = (const R*)c; p.F = (const R*)F; p.f = (const R*)f;
   p.c_scale = R(1);
   p.x = (R*)x; p.u = (R*)u; p.Ks = (R*)Ks; p.ks = (R*)ks; p.fac = (R*)fac;
-  if ((p.flags & LQR_SAVE_FAC) && adjoint_fused_available(n, m)) p.Vsave = (R*)fac + (size_t)T * B * fac_elems_per_step(n, m);
-  int rc = solve_launch<R>(p, st, &h->launches);
+  if ((p.flags & LQR_SAVE_FAC) && adjoint_fused_available<R>(n, m)) p.Vsave = (R*)fac + (size_t)T * B * fac_elems_per_step(n, m);
+  int rc = launch_lqr_solve<R>(p, st, &h->launches);
   if (rc) h->err = rc == DMPC_ERR_UNSUPPORTED ? std::string("lqr_solve: ") + kLargeUnsupported : "lqr_solve launch failed";
   return rc;
 }
@@ -82,59 +72,30 @@ static int lqr_adjoint_impl(dmpc_handle h, int T, int B, int n, int m, const voi
   d.T = T; d.B = B; d.n = n; d.m = m;
   d.F = (const R*)F; d.gx = (const R*)gx; d.gu = (const R*)gu; d.Ks = (const R*)Ks; d.fac = (const R*)fac;
   d.dc = (R*)dc;
-  int rc = DMPC_OK;
-  if ((partials || df) && adjoint_fused_available(n, m)) {
-    // two sweeps.  Full gradients: v'_t is parked in the df output buffer (row t-1) and in dx0 (t = 0) between them.
-    // Fused (T,B)-reduction: dc is a workspace, v'_t travels in its first n entries, nothing but dx0 and the per-element
-    // partial sums is written.
-    d.vp = partials ? nullptr : (R*)df; d.dx0 = (R*)dx0;
-    AdjFusedParams<R> a;
-    memset(&a, 0, sizeof(a));
-    a.T = T; a.B = B; a.n = n; a.m = m;
-    a.flags = (flags & DMPC_ADJ_STRICT_REFERENCE) ? (ADJ_QUIRK_DC | ADJ_QUIRK_DF) : 0;
-    a.F = (const R*)F; a.Ks = (const R*)Ks; a.Vv = (const R*)fac + (size_t)T * B * fac_elems_per_step(n, m);
-    a.x = (const R*)x; a.u = (const R*)u; a.vp = (const R*)df; a.dx0 = (const R*)dx0;
-    a.dc = (R*)dc; a.dC = (R*)dC; a.dF = (R*)dF; a.df = (R*)df; a.red = (R*)partials;
-    const int stage = (flags & DMPC_ADJ_STAGE_OUT_ONLY) ? 2 : ((flags & DMPC_ADJ_STAGE_DTAU_ONLY) ? 1 : 0);
-    rc = launch_adjoint_fused<R>(d, a, stage, st, &h->launches);
-    if (rc) { h->err = "adjoint_fused launch failed"; return rc; }
-    if (partials && stage != 1) {
-      rc = launch_reduce_partials<R>((const R*)partials, B, adj_red_elems(n, m), (R*)sums, st, &h->launches);
-      if (rc) h->err = "reduce_partials launch failed";
-    }
-    return rc;
-  }
-  const int stage = (flags & DMPC_ADJ_STAGE_OUT_ONLY) ? 2 : ((flags & DMPC_ADJ_STAGE_DTAU_ONLY) ? 1 : 0);
-  const bool large = lqr_large_adjoint_selected<R>(n, m, partials != nullptr);
-  if (large && !lqr_large_shape_ok(n, m)) return fail(h, DMPC_ERR_UNSUPPORTED, (std::string("lqr_adjoint: ") + kLargeUnsupported).c_str());
-  if (!large && !(flags & DMPC_ADJ_STAGE_OUT_ONLY)) {
-    rc = launch_lqr_dtau<R>(d, st, &h->launches);
-    if (rc) { h->err = "lqr_dtau launch failed"; return rc; }
-  }
-  if (!large && (flags & DMPC_ADJ_STAGE_DTAU_ONLY)) return rc;
+  // two-sweep adjoint only.  Full gradients: v'_t is parked in the df output buffer (row t-1) and in dx0 (t = 0) between
+  // the sweeps.  Fused (T,B)-reduction: dc is a workspace, v'_t travels in its first n entries, nothing but dx0 and the
+  // per-element partial sums is written.
+  d.vp = partials ? nullptr : (R*)df; d.dx0 = (R*)dx0;
+  const int qflags = (flags & DMPC_ADJ_STRICT_REFERENCE) ? (ADJ_QUIRK_DC | ADJ_QUIRK_DF) : 0;
+  AdjFusedParams<R> f;
+  memset(&f, 0, sizeof(f));
+  f.T = T; f.B = B; f.n = n; f.m = m; f.flags = qflags;
+  f.F = (const R*)F; f.Ks = (const R*)Ks; f.Vv = (const R*)fac + (size_t)T * B * fac_elems_per_step(n, m);
+  f.x = (const R*)x; f.u = (const R*)u; f.vp = (const R*)df; f.dx0 = (const R*)dx0;
+  f.dc = (R*)dc; f.dC = (R*)dC; f.dF = (R*)dF; f.df = (R*)df; f.red = (R*)partials;
   AdjOutParams<R> a;
   memset(&a, 0, sizeof(a));
-  a.T = T; a.B = B; a.n = n; a.m = m; a.F_T = T - 1;
-  a.flags = (flags & DMPC_ADJ_STRICT_REFERENCE) ? (ADJ_QUIRK_DC | ADJ_QUIRK_DF) : 0;
+  a.T = T; a.B = B; a.n = n; a.m = m; a.F_T = T - 1; a.flags = qflags;
   a.C = (const R*)C; a.c = (const R*)c; a.F = (const R*)F; a.x = (const R*)x; a.u = (const R*)u;
   a.dtau = (const R*)dc; a.gx = (const R*)gx; a.gu = (const R*)gu;
   a.dx0 = (R*)dx0; a.dC = (R*)dC; a.dc = (R*)dc; a.dF = (R*)dF; a.df = (R*)df;
   if (partials) { a.flags |= ADJ_REDUCE_TB; a.red = (R*)partials; }
-  if (large) {
-    rc = launch_lqr_large_adjoint<R>(a, (const R*)Ks, (const R*)fac, stage, st, &h->launches);
-    if (rc) { h->err = "lqr_adjoint large-system launch failed"; return rc; }
-    if (stage == 1) return rc;
-  } else {
-    rc = launch_adjoint_out<R>(a, st, &h->launches);
-    if (rc) { h->err = "adjoint_out launch failed"; return rc; }
-  }
-  if (partials) {
-    rc = launch_reduce_partials<R>((const R*)partials, B, adj_red_elems(n, m), (R*)sums, st, &h->launches);
-    if (rc) h->err = "reduce_partials launch failed";
-  }
+  const int stage = (flags & DMPC_ADJ_STAGE_OUT_ONLY) ? 2 : ((flags & DMPC_ADJ_STAGE_DTAU_ONLY) ? 1 : 0);
+  const char* failed = nullptr;
+  const int rc = launch_lqr_adjoint<R>(d, f, a, stage, (R*)sums, st, &h->launches, &failed);
+  if (rc) h->err = failed ? failed : std::string("lqr_adjoint: ") + kLargeUnsupported;
   return rc;
 }
-
 
 template <typename R>
 static int mpc_forward_impl(dmpc_handle h, int T, int B, int n, int m, const void* C, const void* c, const void* F,
@@ -167,10 +128,12 @@ static int mpc_backward_impl(dmpc_handle h, int T, int B, int n, int m, const vo
                              const void* gu, void* wsK, void* wsk, void* wsd, void* act, void* dx0, void* dC,
                              void* dc, void* dF, void* df, cudaStream_t st, void* partials = nullptr,
                              void* sums = nullptr) {
-  // the masked solve and the adjoint each take the large-system kernels where their own per-element kernel does not fit
-  const bool large_adj = lqr_large_adj_out_selected<R>(n, m, partials != nullptr);
-  if ((lqr_large_solve_selected<R>(n, m, LQR_DO_FACTOR | LQR_DO_ROLLOUT | LQR_MASKED) || large_adj) && !lqr_large_shape_ok(n, m))
-    return fail(h, DMPC_ERR_UNSUPPORTED, (std::string("mpc_step_backward: ") + kLargeUnsupported).c_str());
+  // The masked solve and the adjoint each take the large-system kernels where their own per-element kernel does not fit.
+  // Outside the large-system range (n <= 128, m <= 32) at least the masked solve would not run: at m > 32 it is sent to
+  // the large-system kernels, and at n > 128 one element's lqr_layout exceeds kMaxSmem in either dtype (at (129, 1):
+  // 465 KiB in fp32, 929 KiB in fp64, against 227 KiB).  Refusing those shapes here launches nothing, not even
+  // active_mask_kernel.
+  if (!lqr_large_shape_ok(n, m)) return fail(h, DMPC_ERR_UNSUPPORTED, (std::string("mpc_step_backward: ") + kLargeUnsupported).c_str());
   int rc = launch_active_mask<R>((const R*)u, (const R*)lo, (const R*)hi, (unsigned char*)act, (size_t)T * B * m, st, &h->launches);
   if (rc) { h->err = "active_mask launch failed"; return rc; }
   if (cudaMemsetAsync(dx0, 0, (size_t)B * n * sizeof(R), st) != cudaSuccess) return DMPC_ERR_CUDA;
@@ -182,7 +145,7 @@ static int mpc_backward_impl(dmpc_handle h, int T, int B, int n, int m, const vo
   p.C = (const R*)C; p.c = nullptr; p.cx = (const R*)gx; p.cu = (const R*)gu; p.c_scale = R(-1);   // c := -d_taus (:374)
   p.F = (const R*)F; p.f = nullptr; p.active = (const unsigned char*)act;
   p.Ks = (R*)wsK; p.ks = (R*)wsk; p.tau_out = (R*)wsd;
-  rc = solve_launch<R>(p, st, &h->launches);
+  rc = launch_lqr_solve<R>(p, st, &h->launches);
   if (rc) { h->err = "lqr_active launch failed"; return rc; }
   AdjOutParams<R> a;
   memset(&a, 0, sizeof(a));
@@ -192,12 +155,9 @@ static int mpc_backward_impl(dmpc_handle h, int T, int B, int n, int m, const vo
   a.dtau = (const R*)wsd; a.gx = (const R*)gx; a.gu = (const R*)gu;
   a.dx0 = (R*)dx0; a.dC = (R*)dC; a.dc = (R*)dc; a.dF = (R*)dF; a.df = (R*)df;
   if (partials) { a.flags |= ADJ_REDUCE_TB; a.red = (R*)partials; }
-  rc = large_adj ? launch_lqr_large_adjoint<R>(a, nullptr, nullptr, 2, st, &h->launches) : launch_adjoint_out<R>(a, st, &h->launches);
-  if (rc) { h->err = large_adj ? "mpc_step_backward large-system adjoint launch failed" : "adjoint_out launch failed"; return rc; }
-  if (partials) {
-    rc = launch_reduce_partials<R>((const R*)partials, B, adj_red_elems(n, m), (R*)sums, st, &h->launches);
-    if (rc) h->err = "reduce_partials launch failed";
-  }
+  const char* failed = nullptr;
+  rc = launch_adjoint_out<R>(a, (R*)sums, st, &h->launches, &failed);
+  if (rc) h->err = failed;
   return rc;
 }
 
@@ -211,7 +171,7 @@ static int lqr_active_impl(dmpc_handle h, int T, int B, int n, int m, const void
   p.flags = LQR_DO_FACTOR | LQR_DO_ROLLOUT | LQR_MASKED;
   p.x0 = (const R*)x0; p.C = (const R*)C; p.c = (const R*)c; p.c_scale = R(1); p.F = (const R*)F; p.f = (const R*)f;
   p.active = (const unsigned char*)act; p.x = (R*)x; p.u = (R*)u; p.Ks = (R*)Ks; p.ks = (R*)ks;
-  int rc = solve_launch<R>(p, st, &h->launches);
+  int rc = launch_lqr_solve<R>(p, st, &h->launches);
   if (rc) h->err = rc == DMPC_ERR_UNSUPPORTED ? std::string("lqr_active: ") + kLargeUnsupported : "lqr_active launch failed";
   return rc;
 }
@@ -254,7 +214,6 @@ namespace {
 struct BoxWs {
   size_t x_nom, u_a, u_b, x_new, Ks, ks, u_first, objs, costs, old, alphas, du, n_qp, free_m, n_ls, flags, mask, dynp, status, ctl, total;
 };
-inline size_t al256(size_t v) { return (v + 255) & ~(size_t)255; }
 inline BoxWs box_ws(size_t w, int T, int B, int n, int m) {
   BoxWs L; size_t o = 0;
   auto take = [&](size_t bytes) { size_t at = o; o = al256(o + bytes); return at; };
@@ -403,7 +362,7 @@ static int lqr_solve_shared_impl(dmpc_handle h, int T, int B, int n, int m, cons
   p.T = T; p.B = 1; p.n = n; p.m = m; p.flags = LQR_DO_FACTOR | LQR_SAVE_FAC;
   p.C = (const R*)C; p.c = roll_only ? (const R*)c : (const R*)(w + W.c0); p.F = (const R*)F; p.c_scale = R(1);
   p.Ks = (R*)(w + W.Ks); p.ks = (R*)(w + W.ks); p.fac = (R*)(w + W.fac); p.Vsave = (R*)(w + W.V);
-  int rc = solve_launch<R>(p, st, &h->launches);
+  int rc = launch_lqr_solve<R>(p, st, &h->launches);
   if (rc) return fail(h, rc, rc == DMPC_ERR_UNSUPPORTED ? "lqr_solve_shared: no Riccati kernel for this shape" : "lqr_solve_shared: sweep launch failed");
   LqrSharedParams<R> q;
   memset(&q, 0, sizeof(q));
@@ -551,9 +510,7 @@ int dmpc_lqr_solve(dmpc_handle h, int dtype, int T, int B, int n, int m, const v
   if (!(flags & (DMPC_LQR_FACTOR | DMPC_LQR_ROLLOUT))) return fail(h, DMPC_ERR_UNSUPPORTED, "nothing to do");
   if (set_dev(h)) return DMPC_ERR_CUDA;
   cudaStream_t st = pick(h, stream);
-  if (dtype == DMPC_F64) return lqr_solve_impl<double>(h, T, B, n, m, d_x0, d_C, d_c, d_F, d_f, d_x, d_u, d_Ks, d_ks, d_fac, flags, st);
-  if (dtype == DMPC_F32) return lqr_solve_impl<float>(h, T, B, n, m, d_x0, d_C, d_c, d_F, d_f, d_x, d_u, d_Ks, d_ks, d_fac, flags, st);
-  return fail(h, DMPC_ERR_UNSUPPORTED, "dtype");
+  return by_dtype(h, dtype, [&](auto r) { return lqr_solve_impl<decltype(r)>(h, T, B, n, m, d_x0, d_C, d_c, d_F, d_f, d_x, d_u, d_Ks, d_ks, d_fac, flags, st); });
 }
 
 int dmpc_lqr_adjoint(dmpc_handle h, int dtype, int T, int B, int n, int m, const void* d_C, const void* d_c,
@@ -566,9 +523,7 @@ int dmpc_lqr_adjoint(dmpc_handle h, int dtype, int T, int B, int n, int m, const
     return fail(h, DMPC_ERR_NULL, "lqr_adjoint: required buffer is NULL");
   if (set_dev(h)) return DMPC_ERR_CUDA;
   cudaStream_t st = pick(h, stream);
-  if (dtype == DMPC_F64) return lqr_adjoint_impl<double>(h, T, B, n, m, d_C, d_c, d_F, d_x, d_u, d_gx, d_gu, d_Ks, d_fac, d_dx0, d_dC, d_dc, d_dF, d_df, flags, st);
-  if (dtype == DMPC_F32) return lqr_adjoint_impl<float>(h, T, B, n, m, d_C, d_c, d_F, d_x, d_u, d_gx, d_gu, d_Ks, d_fac, d_dx0, d_dC, d_dc, d_dF, d_df, flags, st);
-  return fail(h, DMPC_ERR_UNSUPPORTED, "dtype");
+  return by_dtype(h, dtype, [&](auto r) { return lqr_adjoint_impl<decltype(r)>(h, T, B, n, m, d_C, d_c, d_F, d_x, d_u, d_gx, d_gu, d_Ks, d_fac, d_dx0, d_dC, d_dc, d_dF, d_df, flags, st); });
 }
 
 int dmpc_pnqp(dmpc_handle h, int dtype, int B, int m, const void* d_H, const void* d_q, const void* d_lower,
@@ -579,9 +534,7 @@ int dmpc_pnqp(dmpc_handle h, int dtype, int B, int m, const void* d_H, const voi
   if (!d_H || !d_q || !d_lower || !d_upper || !d_x || !d_free || !d_iters) return fail(h, DMPC_ERR_NULL, "pnqp: required buffer is NULL");
   if (set_dev(h)) return DMPC_ERR_CUDA;
   cudaStream_t st = pick(h, stream);
-  if (dtype == DMPC_F64) return pnqp_impl<double>(h, B, m, d_H, d_q, d_lower, d_upper, d_x_init, n_iter, coupling, d_x, d_LU, d_piv, d_free, d_iters, d_flags, st);
-  if (dtype == DMPC_F32) return pnqp_impl<float>(h, B, m, d_H, d_q, d_lower, d_upper, d_x_init, n_iter, coupling, d_x, d_LU, d_piv, d_free, d_iters, d_flags, st);
-  return fail(h, DMPC_ERR_UNSUPPORTED, "dtype");
+  return by_dtype(h, dtype, [&](auto r) { return pnqp_impl<decltype(r)>(h, B, m, d_H, d_q, d_lower, d_upper, d_x_init, n_iter, coupling, d_x, d_LU, d_piv, d_free, d_iters, d_flags, st); });
 }
 
 int dmpc_mpc_step_forward(dmpc_handle h, int dtype, int T, int B, int n, int m, const void* d_C, const void* d_c,
@@ -603,9 +556,7 @@ int dmpc_mpc_step_forward(dmpc_handle h, int dtype, int T, int B, int n, int m, 
   if (dynamics != DMPC_DYN_LINEAR && dynamics != DMPC_DYN_PENDULUM) return fail(h, DMPC_ERR_UNSUPPORTED, "dynamics selector");
   if (set_dev(h)) return DMPC_ERR_CUDA;
   cudaStream_t st = pick(h, stream);
-  if (dtype == DMPC_F64) return mpc_forward_impl<double>(h, T, B, n, m, d_C, d_c, d_F, F_T, d_f, d_x_nom, d_u_nom, d_lower, d_upper, d_tC, d_tc, dynamics, d_tF, d_tf, h_dyn_params, ls_decay, max_ls_trials, need_expand, coupling, d_x, d_u, d_Ks, d_ks, d_u_first, d_objs, d_costs, d_old_costs, d_alphas, d_n_qp, d_free, d_n_ls, d_flags, st);
-  if (dtype == DMPC_F32) return mpc_forward_impl<float>(h, T, B, n, m, d_C, d_c, d_F, F_T, d_f, d_x_nom, d_u_nom, d_lower, d_upper, d_tC, d_tc, dynamics, d_tF, d_tf, h_dyn_params, ls_decay, max_ls_trials, need_expand, coupling, d_x, d_u, d_Ks, d_ks, d_u_first, d_objs, d_costs, d_old_costs, d_alphas, d_n_qp, d_free, d_n_ls, d_flags, st);
-  return fail(h, DMPC_ERR_UNSUPPORTED, "dtype");
+  return by_dtype(h, dtype, [&](auto r) { return mpc_forward_impl<decltype(r)>(h, T, B, n, m, d_C, d_c, d_F, F_T, d_f, d_x_nom, d_u_nom, d_lower, d_upper, d_tC, d_tc, dynamics, d_tF, d_tf, h_dyn_params, ls_decay, max_ls_trials, need_expand, coupling, d_x, d_u, d_Ks, d_ks, d_u_first, d_objs, d_costs, d_old_costs, d_alphas, d_n_qp, d_free, d_n_ls, d_flags, st); });
 }
 
 int dmpc_mpc_step_backward(dmpc_handle h, int dtype, int T, int B, int n, int m, const void* d_C, const void* d_c,
@@ -621,9 +572,7 @@ int dmpc_mpc_step_backward(dmpc_handle h, int dtype, int T, int B, int n, int m,
     return fail(h, DMPC_ERR_NULL, "mpc_step_backward: required buffer is NULL");
   if (set_dev(h)) return DMPC_ERR_CUDA;
   cudaStream_t st = pick(h, stream);
-  if (dtype == DMPC_F64) return mpc_backward_impl<double>(h, T, B, n, m, d_C, d_c, d_F, F_T, d_x, d_u, d_lower, d_upper, d_gx, d_gu, d_ws_Ks, d_ws_ks, d_ws_dtau, d_active, d_dx0, d_dC, d_dc, d_dF, d_df, st);
-  if (dtype == DMPC_F32) return mpc_backward_impl<float>(h, T, B, n, m, d_C, d_c, d_F, F_T, d_x, d_u, d_lower, d_upper, d_gx, d_gu, d_ws_Ks, d_ws_ks, d_ws_dtau, d_active, d_dx0, d_dC, d_dc, d_dF, d_df, st);
-  return fail(h, DMPC_ERR_UNSUPPORTED, "dtype");
+  return by_dtype(h, dtype, [&](auto r) { return mpc_backward_impl<decltype(r)>(h, T, B, n, m, d_C, d_c, d_F, F_T, d_x, d_u, d_lower, d_upper, d_gx, d_gu, d_ws_Ks, d_ws_ks, d_ws_dtau, d_active, d_dx0, d_dC, d_dc, d_dF, d_df, st); });
 }
 
 int dmpc_lqr_active_solve(dmpc_handle h, int dtype, int T, int B, int n, int m, const void* d_x0, const void* d_C,
@@ -635,9 +584,7 @@ int dmpc_lqr_active_solve(dmpc_handle h, int dtype, int T, int B, int n, int m, 
   if (!d_x0 || !d_C || !d_c || (T > 1 && !d_F) || !d_active || !d_x || !d_u || !d_Ks || !d_ks) return fail(h, DMPC_ERR_NULL, "lqr_active: required buffer is NULL");
   if (set_dev(h)) return DMPC_ERR_CUDA;
   cudaStream_t st = pick(h, stream);
-  if (dtype == DMPC_F64) return lqr_active_impl<double>(h, T, B, n, m, d_x0, d_C, d_c, d_F, d_f, d_active, d_x, d_u, d_Ks, d_ks, st);
-  if (dtype == DMPC_F32) return lqr_active_impl<float>(h, T, B, n, m, d_x0, d_C, d_c, d_F, d_f, d_active, d_x, d_u, d_Ks, d_ks, st);
-  return fail(h, DMPC_ERR_UNSUPPORTED, "dtype");
+  return by_dtype(h, dtype, [&](auto r) { return lqr_active_impl<decltype(r)>(h, T, B, n, m, d_x0, d_C, d_c, d_F, d_f, d_active, d_x, d_u, d_Ks, d_ks, st); });
 }
 
 int dmpc_get_traj(dmpc_handle h, int dtype, int T, int B, int n, int m, int dynamics, const void* d_x0,
@@ -651,9 +598,7 @@ int dmpc_get_traj(dmpc_handle h, int dtype, int T, int B, int n, int m, int dyna
   if ((d_Fout == nullptr) != (d_fout == nullptr)) return fail(h, DMPC_ERR_NULL, "Fout and fout go together");
   if (set_dev(h)) return DMPC_ERR_CUDA;
   cudaStream_t st = pick(h, stream);
-  if (dtype == DMPC_F64) return traj_impl<double>(h, T, B, n, m, dynamics, d_x0, d_u, d_F, d_f, h_dyn_params, d_x, d_Fout, d_fout, st);
-  if (dtype == DMPC_F32) return traj_impl<float>(h, T, B, n, m, dynamics, d_x0, d_u, d_F, d_f, h_dyn_params, d_x, d_Fout, d_fout, st);
-  return fail(h, DMPC_ERR_UNSUPPORTED, "dtype");
+  return by_dtype(h, dtype, [&](auto r) { return traj_impl<decltype(r)>(h, T, B, n, m, dynamics, d_x0, d_u, d_F, d_f, h_dyn_params, d_x, d_Fout, d_fout, st); });
 }
 
 int dmpc_boxddp_workspace_bytes(int dtype, int T, int B, int n, int m, size_t* bytes) {
@@ -683,8 +628,7 @@ int dmpc_boxddp_solve(dmpc_handle h, int dtype, int T, int B, int n, int m, cons
   if (ws_bytes < need) return fail(h, DMPC_ERR_BAD_SHAPE, "boxddp: workspace too small (dmpc_boxddp_workspace_bytes)");
   if (set_dev(h)) return DMPC_ERR_CUDA;
   cudaStream_t st = pick(h, stream);
-  if (dtype == DMPC_F64) return boxddp_impl<double>(h, dtype, T, B, n, m, d_x_init, d_C, d_c, d_lower, d_upper, dynamics, d_F, F_T, d_f, h_dyn_params, d_u_init, opts, d_ws, d_x_best, d_u_best, d_costs_best, d_du_best, d_du_last, d_F_lin, d_f_lin, h_n_iter, h_status, h_flags, st);
-  return boxddp_impl<float>(h, dtype, T, B, n, m, d_x_init, d_C, d_c, d_lower, d_upper, dynamics, d_F, F_T, d_f, h_dyn_params, d_u_init, opts, d_ws, d_x_best, d_u_best, d_costs_best, d_du_best, d_du_last, d_F_lin, d_f_lin, h_n_iter, h_status, h_flags, st);
+  return by_dtype(h, dtype, [&](auto r) { return boxddp_impl<decltype(r)>(h, dtype, T, B, n, m, d_x_init, d_C, d_c, d_lower, d_upper, dynamics, d_F, F_T, d_f, h_dyn_params, d_u_init, opts, d_ws, d_x_best, d_u_best, d_costs_best, d_du_best, d_du_last, d_F_lin, d_f_lin, h_n_iter, h_status, h_flags, st); });
 }
 
 int dmpc_expand_time_batch(dmpc_handle h, int dtype, int T, int B, int count, const void* d_src, void* d_dst, void* stream) {
@@ -694,9 +638,10 @@ int dmpc_expand_time_batch(dmpc_handle h, int dtype, int T, int B, int count, co
   if (set_dev(h)) return DMPC_ERR_CUDA;
   cudaStream_t st = pick(h, stream);
   const size_t total = (size_t)T * B * count;
-  if (dtype == DMPC_F64) return launch_expand_time_batch<double>((const double*)d_src, (double*)d_dst, count, total, st, &h->launches);
-  if (dtype == DMPC_F32) return launch_expand_time_batch<float>((const float*)d_src, (float*)d_dst, count, total, st, &h->launches);
-  return fail(h, DMPC_ERR_UNSUPPORTED, "dtype");
+  return by_dtype(h, dtype, [&](auto r) {
+    using R = decltype(r);
+    return launch_expand_time_batch<R>((const R*)d_src, (R*)d_dst, count, total, st, &h->launches);
+  });
 }
 
 static int warmstart_impl(dmpc_handle h, int dtype, int T, int B, int m, int n_samples, void* d_cache, const int* d_idx,
@@ -709,15 +654,12 @@ static int warmstart_impl(dmpc_handle h, int dtype, int T, int B, int m, int n_s
   const size_t total = (size_t)T * B * m;
   const int tpb = 256;
   const unsigned grid = (unsigned)((total + tpb - 1) / tpb);
-  if (dtype == DMPC_F64) {
-    if (put) warmstart_kernel<double, true><<<grid, tpb, 0, st>>>(T, B, m, n_samples, (double*)d_cache, d_idx, (double*)d_u);
-    else warmstart_kernel<double, false><<<grid, tpb, 0, st>>>(T, B, m, n_samples, (double*)d_cache, d_idx, (double*)d_u);
-  } else if (dtype == DMPC_F32) {
-    if (put) warmstart_kernel<float, true><<<grid, tpb, 0, st>>>(T, B, m, n_samples, (float*)d_cache, d_idx, (float*)d_u);
-    else warmstart_kernel<float, false><<<grid, tpb, 0, st>>>(T, B, m, n_samples, (float*)d_cache, d_idx, (float*)d_u);
-  } else return fail(h, DMPC_ERR_UNSUPPORTED, "dtype");
-  ++h->launches;
-  return cudaGetLastError() == cudaSuccess ? DMPC_OK : fail(h, DMPC_ERR_CUDA, "warmstart launch failed");
+  return by_dtype(h, dtype, [&](auto r) {
+    using R = decltype(r);
+    const int rc = launch(put ? warmstart_kernel<R, true> : warmstart_kernel<R, false>, grid, tpb, 0, st, &h->launches, T, B, m,
+                          n_samples, (R*)d_cache, d_idx, (R*)d_u);
+    return rc ? fail(h, rc, "warmstart launch failed") : DMPC_OK;
+  });
 }
 
 int dmpc_warmstart_take(dmpc_handle h, int dtype, int T, int B, int m, int n_samples, const void* d_cache, const int32_t* d_idx,
@@ -742,9 +684,7 @@ int dmpc_lqr_adjoint_reduced(dmpc_handle h, int dtype, int T, int B, int n, int 
     return fail(h, DMPC_ERR_NULL, "lqr_adjoint_reduced: required buffer is NULL");
   if (set_dev(h)) return DMPC_ERR_CUDA;
   cudaStream_t st = pick(h, stream);
-  if (dtype == DMPC_F64) return lqr_adjoint_impl<double>(h, T, B, n, m, d_C, d_c, d_F, d_x, d_u, d_gx, d_gu, d_Ks, d_fac, d_dx0, nullptr, d_ws_dtau, nullptr, nullptr, flags, st, d_ws_partials, d_sums);
-  if (dtype == DMPC_F32) return lqr_adjoint_impl<float>(h, T, B, n, m, d_C, d_c, d_F, d_x, d_u, d_gx, d_gu, d_Ks, d_fac, d_dx0, nullptr, d_ws_dtau, nullptr, nullptr, flags, st, d_ws_partials, d_sums);
-  return fail(h, DMPC_ERR_UNSUPPORTED, "dtype");
+  return by_dtype(h, dtype, [&](auto r) { return lqr_adjoint_impl<decltype(r)>(h, T, B, n, m, d_C, d_c, d_F, d_x, d_u, d_gx, d_gu, d_Ks, d_fac, d_dx0, nullptr, d_ws_dtau, nullptr, nullptr, flags, st, d_ws_partials, d_sums); });
 }
 
 int dmpc_mpc_step_backward_reduced(dmpc_handle h, int dtype, int T, int B, int n, int m, const void* d_C, const void* d_c,
@@ -760,9 +700,7 @@ int dmpc_mpc_step_backward_reduced(dmpc_handle h, int dtype, int T, int B, int n
     return fail(h, DMPC_ERR_NULL, "mpc_step_backward_reduced: required buffer is NULL");
   if (set_dev(h)) return DMPC_ERR_CUDA;
   cudaStream_t st = pick(h, stream);
-  if (dtype == DMPC_F64) return mpc_backward_impl<double>(h, T, B, n, m, d_C, d_c, d_F, F_T, d_x, d_u, d_lower, d_upper, d_gx, d_gu, d_ws_Ks, d_ws_ks, d_ws_dtau, d_active, d_dx0, nullptr, nullptr, nullptr, nullptr, st, d_ws_partials, d_sums);
-  if (dtype == DMPC_F32) return mpc_backward_impl<float>(h, T, B, n, m, d_C, d_c, d_F, F_T, d_x, d_u, d_lower, d_upper, d_gx, d_gu, d_ws_Ks, d_ws_ks, d_ws_dtau, d_active, d_dx0, nullptr, nullptr, nullptr, nullptr, st, d_ws_partials, d_sums);
-  return fail(h, DMPC_ERR_UNSUPPORTED, "dtype");
+  return by_dtype(h, dtype, [&](auto r) { return mpc_backward_impl<decltype(r)>(h, T, B, n, m, d_C, d_c, d_F, F_T, d_x, d_u, d_lower, d_upper, d_gx, d_gu, d_ws_Ks, d_ws_ks, d_ws_dtau, d_active, d_dx0, nullptr, nullptr, nullptr, nullptr, st, d_ws_partials, d_sums); });
 }
 
 int dmpc_lqr_shared_workspace_bytes_ex(int dtype, int T, int B, int n, int m, int share, size_t* bytes) {
@@ -802,8 +740,7 @@ int dmpc_lqr_solve_shared_ex(dmpc_handle h, int dtype, int T, int B, int n, int 
   if (int rc = shared_check(h, dtype, T, B, n, m, F_T, d_F, d_ws, ws_bytes, share)) return rc;
   if (set_dev(h)) return DMPC_ERR_CUDA;
   cudaStream_t st = pick(h, stream);
-  if (dtype == DMPC_F64) return lqr_solve_shared_impl<double>(h, T, B, n, m, d_x0, d_C, d_c, d_F, F_T, d_f, d_x, d_u, d_ws, share, st);
-  return lqr_solve_shared_impl<float>(h, T, B, n, m, d_x0, d_C, d_c, d_F, F_T, d_f, d_x, d_u, d_ws, share, st);
+  return by_dtype(h, dtype, [&](auto r) { return lqr_solve_shared_impl<decltype(r)>(h, T, B, n, m, d_x0, d_C, d_c, d_F, F_T, d_f, d_x, d_u, d_ws, share, st); });
 }
 
 int dmpc_lqr_solve_shared(dmpc_handle h, int dtype, int T, int B, int n, int m, const void* d_x0, const void* d_C,
@@ -823,8 +760,7 @@ int dmpc_lqr_adjoint_shared_ex(dmpc_handle h, int dtype, int T, int B, int n, in
   if (int rc = shared_check(h, dtype, T, B, n, m, F_T, d_F, d_ws, ws_bytes, share)) return rc;
   if (set_dev(h)) return DMPC_ERR_CUDA;
   cudaStream_t st = pick(h, stream);
-  if (dtype == DMPC_F64) return lqr_adjoint_shared_impl<double>(h, T, B, n, m, d_C, d_c, d_F, F_T, d_x, d_u, d_gx, d_gu, d_ws, d_dx0, d_dC, d_dc, d_dF, d_df, flags, share, st);
-  return lqr_adjoint_shared_impl<float>(h, T, B, n, m, d_C, d_c, d_F, F_T, d_x, d_u, d_gx, d_gu, d_ws, d_dx0, d_dC, d_dc, d_dF, d_df, flags, share, st);
+  return by_dtype(h, dtype, [&](auto r) { return lqr_adjoint_shared_impl<decltype(r)>(h, T, B, n, m, d_C, d_c, d_F, F_T, d_x, d_u, d_gx, d_gu, d_ws, d_dx0, d_dC, d_dc, d_dF, d_df, flags, share, st); });
 }
 
 int dmpc_lqr_adjoint_shared(dmpc_handle h, int dtype, int T, int B, int n, int m, const void* d_C, const void* d_c,

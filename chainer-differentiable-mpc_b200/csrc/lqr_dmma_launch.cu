@@ -17,14 +17,12 @@ int launch_lqr_solve_dmma(const LqrParams<R>& p, cudaStream_t st, long long* nl)
     constexpr int WPC = 4;
     const size_t smem = (size_t)WPC * WarpCfg::TOTAL * sizeof(double);
     auto kern = lqr_factor_dmma_warp_kernel<WPC, R>;
-    if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return DMPC_ERR_CUDA;
+    if (set_smem(kern, smem)) return DMPC_ERR_CUDA;
     static int n_sm = 0;
     if (n_sm == 0) { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev); }
     int grid = (p.B + WPC - 1) / WPC;                            // persistent: at most the 2 resident CTAs per SM
     if (grid > 2 * n_sm) grid = 2 * n_sm;
-    kern<<<grid, WPC * 32, smem, st>>>(p);                       // the rollout (if requested) is fused in
-    if (nl) ++*nl;
-    return cudaGetLastError() == cudaSuccess ? DMPC_OK : DMPC_ERR_CUDA;
+    return launch(kern, grid, WPC * 32, smem, st, nl, p);         // the rollout (if requested) is fused in
   }
   if (p.flags & LQR_DO_ROLLOUT) return launch_lqr_rollout_32_8<R>(p, st, nl);   // rollout-only: compact generic launch
   return DMPC_OK;

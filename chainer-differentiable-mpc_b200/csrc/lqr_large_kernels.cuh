@@ -16,6 +16,7 @@
 // Every product runs in fp64 on mma.m8n8k4.f64 (DMMA); fp32 tensors are widened on load and rounded once on store.
 // Scratch (V | v, Q | q, [K | k], P, lambda, d-lambda) is fp64 and per element.
 #pragma once
+#include "launch.h"
 #include "lqr_kernels.cuh"
 #include "lqr_shared_kernels.cuh"
 
@@ -397,6 +398,32 @@ __global__ void __launch_bounds__(kLargeThreads) lqr_large_red_kernel(AdjOutPara
       out[s * s + s + n * s + i] = (R)(sgn * acc);
     }
   }
+}
+
+// ---- host: the Riccati steps of the large-system LQR solve and MPC step forward
+
+inline size_t large_fwd_ws_bytes(int B, int n, int m) {
+  const size_t s = (size_t)(n + m);
+  return sizeof(double) * B * ((size_t)n * (n + 1) + s * (s + 1) + 2 * (size_t)m * (n + 1));
+}
+
+// Per t = T-1 ... 0: lqr_large_q_kernel, then factor(w, t) (the factor step, which launches one kernel), then for t >= 1
+// lqr_large_v_kernel, which also writes V_t | v_t to Vdst when it is not null.  `ws` holds large_fwd_ws_bytes.
+// factor's kernel has its shared-memory limit set by the caller.
+template <typename R, typename Factor>
+int large_riccati_steps(const LqrParams<R>& q, double* ws, R* Vdst, Factor factor, cudaStream_t st, long long* nl) {
+  const int n = q.n, s = n + q.m, B = q.B;
+  const size_t nV = (size_t)n * (n + 1), nQ = (size_t)s * (s + 1), nK = (size_t)q.m * (n + 1);
+  const LargeFwdWs w{ws, ws + (size_t)B * nV, ws + (size_t)B * (nV + nQ), ws + (size_t)B * (nV + nQ + nK)};
+  const size_t smq = sizeof(double) * n * kLargePanel;
+  int rc = set_smem(lqr_large_q_kernel<R>, smq);
+  const dim3 gq(B, (s + 1 + kLargePanel - 1) / kLargePanel), gv(B, (n + 1 + kLargePanel - 1) / kLargePanel);
+  for (int t = q.T - 1; t >= 0 && !rc; --t) {
+    rc = launch(lqr_large_q_kernel<R>, gq, kLargeThreads, smq, st, nl, q, w, t);
+    if (!rc) rc = factor(w, t);
+    if (!rc && t > 0) rc = launch(lqr_large_v_kernel<R>, gv, kLargeThreads, 0, st, nl, q, w, Vdst, t);
+  }
+  return rc;
 }
 
 }  // namespace dmpc

@@ -32,12 +32,8 @@ static int do_launch(K kernel, const P& p, int G, size_t stride_bytes, int B, cu
   while (G <= 32 && tpb > 32 && (B + epb - 1) / epb < 148 * 2) { tpb /= 2; epb = tpb / G; }
   const size_t smem = (size_t)epb * stride_bytes;
   if (smem > (size_t)kMaxSmem) return DMPC_ERR_UNSUPPORTED;
-  cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e != cudaSuccess) return DMPC_ERR_CUDA;
-  const int grid = (B + epb - 1) / epb;
-  kernel<<<grid, tpb, smem, st>>>(p);
-  if (nl) ++*nl;
-  return cudaGetLastError() == cudaSuccess ? DMPC_OK : DMPC_ERR_CUDA;
+  if (set_smem(kernel, smem)) return DMPC_ERR_CUDA;
+  return launch(kernel, (B + epb - 1) / epb, tpb, smem, st, nl, p);
 }
 
 static bool dmma_enabled() {
@@ -75,6 +71,29 @@ static bool lqr_tpe_adj_enabled() {
   return v == 1 && lqr_tpe_enabled();
 }
 
+#define DMPC_FUSED_SHAPES(X) X(32, 8)
+
+template <typename R>
+bool adjoint_fused_available(int n, int m) {
+  static int off = -1;
+  if (off < 0) { const char* e = getenv("DMPC_ADJ_UNFUSED"); off = (e && e[0] == '1') ? 1 : 0; }
+  if (off) return false;
+#define X(N_, M_) if (n == N_ && m == M_) return true;
+  DMPC_FUSED_SHAPES(X)
+#undef X
+  return false;
+}
+
+// s <= 6: one thread per element, registers only (lqr_tpe_kernel.cuh); `warp_reals` of shared memory per warp
+template <typename K, template <typename> class P, typename R>
+static int tpe_launch(K kernel, const P<R>& p, int warp_reals, cudaStream_t st, long long* nl) {
+  const int tpb = p.B >= 148 * 64 * 2 ? 64 : 32;            // small batches: more, smaller CTAs so the grid covers the SMs
+  const int epw = tpe_elems_per_warp(p.B);
+  const size_t sm = (size_t)(tpb / 32) * warp_reals * sizeof(R);
+  if (set_smem(kernel, sm)) return DMPC_ERR_CUDA;
+  return launch(kernel, (p.B + epw * (tpb / 32) - 1) / (epw * (tpb / 32)), tpb, sm, st, nl, p, epw);
+}
+
 template <typename R>
 int launch_lqr_rollout_32_8(const LqrParams<R>& p, cudaStream_t st, long long* nl) {
   LqrParams<R> q = p;
@@ -93,30 +112,21 @@ int launch_lqr_solve(const LqrParams<R>& p, cudaStream_t st, long long* nl) {
   const bool aligned = al16(p.C) && al16(p.c) && al16(p.F) && al16(p.f) && al16(p.Ks) && al16(p.ks) && al16(p.fac) && al16(p.Vsave);
   if (p.n == 32 && p.m == 8 && !(p.flags & LQR_MASKED) && p.c && p.c_scale == R(1) && dmma_enabled() && aligned)
     return launch_lqr_solve_dmma<R>(p, st, nl);
-  // s <= 6: one thread per element, registers only (lqr_tpe_kernel.cuh); DMPC_LQR_GROUP=1 keeps the group kernel (A/B)
+  // DMPC_LQR_GROUP=1 keeps the group kernel (A/B)
   if (lqr_tpe_enabled()) {
-    const int tpb = p.B >= 148 * 64 * 2 ? 64 : 32;            // small batches: more, smaller CTAs so the grid covers the SMs
-    const int epw = tpe_elems_per_warp(p.B);
-    const int grid = (p.B + epw * (tpb / 32) - 1) / (epw * (tpb / 32));
-#define X(N_, M_)                                                                                            \
-    if (p.n == N_ && p.m == M_) {                                                                            \
-      auto k = lqr_tpe_kernel<R, N_, M_, 64, 2, 3>;                                                          \
-      const size_t sm = (size_t)(tpb / 32) * tpe_lqr_warp_reals(N_, M_, 2, 3) * sizeof(R);                   \
-      if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm) != cudaSuccess) return DMPC_ERR_CUDA; \
-      k<<<grid, tpb, sm, st>>>(p, epw);                                                                        \
-      if (nl) ++*nl;                                                                                         \
-      return cudaGetLastError() == cudaSuccess ? DMPC_OK : DMPC_ERR_CUDA;                                    \
-    }
+#define X(N_, M_) if (p.n == N_ && p.m == M_) return tpe_launch(lqr_tpe_kernel<R, N_, M_, 64, 2, 3>, p, tpe_lqr_warp_reals(N_, M_, 2, 3), st, nl);
     X(2, 1) X(3, 1) X(4, 2)
 #undef X
   }
   const bool compact = !(p.flags & LQR_DO_FACTOR);
   const LqrLayout L = lqr_layout<R>(p.n, p.m, (p.flags & LQR_SAVE_FAC) != 0, compact);
   const size_t sb = (size_t)L.stride * sizeof(R);
+  // one element per CTA does not fit (do_launch's test; s > 24 runs one element per CTA, smaller systems always fit) or
+  // m > 32: the host-stepped large-system kernels (lqr_large_launch.cu), masked solves included
+  if (p.m > 32 || sb > (size_t)kMaxSmem) return launch_lqr_large_solve<R>(p, st, nl);
 #define X(N_, M_, G_) if (si.specialised && p.n == N_ && p.m == M_) return do_launch(lqr_solve_kernel<R, N_, M_, G_>, p, G_, sb, p.B, st, nl);
   DMPC_SHAPES(X)
 #undef X
-  if (p.m > 32) return DMPC_ERR_UNSUPPORTED;
   switch (si.G) {
     case 8: return do_launch(lqr_solve_kernel<R, 0, 0, 8>, p, 8, sb, p.B, st, nl);
     case 16: return do_launch(lqr_solve_kernel<R, 0, 0, 16>, p, 16, sb, p.B, st, nl);
@@ -126,21 +136,10 @@ int launch_lqr_solve(const LqrParams<R>& p, cudaStream_t st, long long* nl) {
 }
 
 template <typename R>
-int launch_lqr_dtau(const DtauParams<R>& p, cudaStream_t st, long long* nl) {
+static int launch_lqr_dtau(const DtauParams<R>& p, cudaStream_t st, long long* nl) {
   const ShapeInfo si = pick_shape_impl(p.n, p.m);
-  if (lqr_tpe_enabled()) {                                    // s <= 6: thread per element (lqr_tpe_kernel.cuh)
-    const int tpb = p.B >= 148 * 64 * 2 ? 64 : 32;
-    const int epw = tpe_elems_per_warp(p.B);
-    const int grid = (p.B + epw * (tpb / 32) - 1) / (epw * (tpb / 32));
-#define X(N_, M_)                                                                                            \
-    if (p.n == N_ && p.m == M_) {                                                                            \
-      auto k = lqr_dtau_tpe_kernel<R, N_, M_, 64, 3>;                                                        \
-      const size_t sm = (size_t)(tpb / 32) * tpe_dtau_warp_reals(N_, M_, 3) * sizeof(R);                     \
-      if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm) != cudaSuccess) return DMPC_ERR_CUDA; \
-      k<<<grid, tpb, sm, st>>>(p, epw);                                                                        \
-      if (nl) ++*nl;                                                                                         \
-      return cudaGetLastError() == cudaSuccess ? DMPC_OK : DMPC_ERR_CUDA;                                    \
-    }
+  if (lqr_tpe_enabled()) {
+#define X(N_, M_) if (p.n == N_ && p.m == M_) return tpe_launch(lqr_dtau_tpe_kernel<R, N_, M_, 64, 3>, p, tpe_dtau_warp_reals(N_, M_, 3), st, nl);
     X(2, 1) X(3, 1) X(4, 2)
 #undef X
   }
@@ -158,9 +157,9 @@ int launch_lqr_dtau(const DtauParams<R>& p, cudaStream_t st, long long* nl) {
 }
 
 // Two-sweep adjoint: sweep 1 (lqr_dtau_kernel<FUSED>) then adjoint_fused_kernel, one CTA per element each.
-
+// stage as launch_lqr_adjoint's; DMPC_ERR_UNSUPPORTED when the shape has no instantiation
 template <typename R>
-int launch_adjoint_fused(const DtauParams<R>& d, const AdjFusedParams<R>& a, int stage, cudaStream_t st, long long* nl) {
+static int launch_adjoint_fused(const DtauParams<R>& d, const AdjFusedParams<R>& a, int stage, cudaStream_t st, long long* nl) {
 #define X(N_, M_)                                                                                                     \
   if (d.n == N_ && d.m == M_) {                                                                                       \
     const DtauLayout L1 = dtau_layout<R>(N_, M_);                                                                     \
@@ -176,23 +175,13 @@ int launch_adjoint_fused(const DtauParams<R>& d, const AdjFusedParams<R>& a, int
   return DMPC_ERR_UNSUPPORTED;
 }
 
+// adjoint_out_kernel / adjoint_out_tpe_kernel
 template <typename R>
-int launch_adjoint_out(const AdjOutParams<R>& p, cudaStream_t st, long long* nl) {
+static int launch_adjoint_out_group(const AdjOutParams<R>& p, cudaStream_t st, long long* nl) {
   const ShapeInfo si = pick_shape_impl(p.n, p.m);
   const bool red = (p.flags & ADJ_REDUCE_TB) != 0;
   if (!red && lqr_tpe_adj_enabled()) {                        // s <= 6, materialised gradients: thread per element
-    const int tpb = p.B >= 148 * 64 * 2 ? 64 : 32;
-    const int epw = tpe_elems_per_warp(p.B);
-    const int grid = (p.B + epw * (tpb / 32) - 1) / (epw * (tpb / 32));
-#define X(N_, M_)                                                                                            \
-    if (p.n == N_ && p.m == M_) {                                                                            \
-      auto k = adjoint_out_tpe_kernel<R, N_, M_, 64>;                                                        \
-      const size_t sm = (size_t)(tpb / 32) * tpe_adj_warp_reals(N_, M_) * sizeof(R);                         \
-      if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm) != cudaSuccess) return DMPC_ERR_CUDA; \
-      k<<<grid, tpb, sm, st>>>(p, epw);                                                                        \
-      if (nl) ++*nl;                                                                                         \
-      return cudaGetLastError() == cudaSuccess ? DMPC_OK : DMPC_ERR_CUDA;                                    \
-    }
+#define X(N_, M_) if (p.n == N_ && p.m == M_) return tpe_launch(adjoint_out_tpe_kernel<R, N_, M_, 64>, p, tpe_adj_warp_reals(N_, M_), st, nl);
     X(2, 1) X(3, 1) X(4, 2)
 #undef X
   }
@@ -214,12 +203,56 @@ int launch_adjoint_out(const AdjOutParams<R>& p, cudaStream_t st, long long* nl)
 #undef Y
 }
 
+// The last step of the (T,B)-reduced adjoint: the per-element partial records a.red summed into `sums`.
 template <typename R>
-int launch_reduce_partials(const R* red, int B, int rsz, R* out, cudaStream_t st, long long* nl) {
-  const int wpb = 4;
-  reduce_partials_kernel<R><<<(rsz + wpb - 1) / wpb, wpb * 32, 0, st>>>(red, B, rsz, out);
-  if (nl) ++*nl;
-  return cudaGetLastError() == cudaSuccess ? DMPC_OK : DMPC_ERR_CUDA;
+static int reduce_partials(const AdjOutParams<R>& a, R* sums, cudaStream_t st, long long* nl, const char** failed) {
+  if (!a.red) return DMPC_OK;
+  *failed = "reduce_partials launch failed";
+  const int wpb = 4, rsz = adj_red_elems(a.n, a.m);
+  return launch(reduce_partials_kernel<R>, (rsz + wpb - 1) / wpb, wpb * 32, 0, st, nl, (const R*)a.red, a.B, rsz, sums);
+}
+
+// The per-element kernels run where one element's layout fits one CTA's shared memory (do_launch's test).  (The
+// compile-time shapes' reduced adjoint keeps its sums in registers; all of them fit either way.)
+template <typename R>
+static bool fits(int stride) { return (size_t)stride * sizeof(R) <= (size_t)kMaxSmem; }
+
+template <typename R>
+int launch_lqr_adjoint(const DtauParams<R>& d, const AdjFusedParams<R>& f, const AdjOutParams<R>& a, int stage, R* sums,
+                       cudaStream_t st, long long* nl, const char** failed) {
+  int rc;
+  if ((a.red || a.df) && adjoint_fused_available<R>(a.n, a.m)) {
+    *failed = "adjoint_fused launch failed";
+    rc = launch_adjoint_fused<R>(d, f, stage, st, nl);
+  } else if (!fits<R>(dtau_layout<R>(a.n, a.m).stride) || !fits<R>(adj_layout<R>(a.n, a.m, a.red != nullptr).stride)) {
+    // m > 32 alone does not select these: the per-element adjoint kernels have no limit on m
+    if (!lqr_large_shape_ok(a.n, a.m)) { *failed = nullptr; return DMPC_ERR_UNSUPPORTED; }
+    *failed = "lqr_adjoint large-system launch failed";
+    rc = launch_lqr_large_adjoint<R>(a, d.Ks, d.fac, stage, st, nl);
+  } else {
+    *failed = "lqr_dtau launch failed";
+    rc = stage == 2 ? DMPC_OK : launch_lqr_dtau<R>(d, st, nl);
+    if (!rc && stage != 1) {
+      *failed = "adjoint_out launch failed";
+      rc = launch_adjoint_out_group<R>(a, st, nl);
+    }
+  }
+  if (rc || stage == 1) return rc;
+  return reduce_partials<R>(a, sums, st, nl, failed);
+}
+
+template <typename R>
+int launch_adjoint_out(const AdjOutParams<R>& p, R* sums, cudaStream_t st, long long* nl, const char** failed) {
+  int rc;
+  if (fits<R>(adj_layout<R>(p.n, p.m, p.red != nullptr).stride)) {
+    *failed = "adjoint_out launch failed";
+    rc = launch_adjoint_out_group<R>(p, st, nl);
+  } else {
+    *failed = "mpc_step_backward large-system adjoint launch failed";
+    rc = launch_lqr_large_adjoint<R>(p, nullptr, nullptr, 2, st, nl);
+  }
+  if (rc) return rc;
+  return reduce_partials<R>(p, sums, st, nl, failed);
 }
 
 template <typename R>
@@ -227,17 +260,15 @@ int launch_expand_time_batch(const R* src, R* dst, int count, size_t total, cuda
   const int tpb = 256;
   size_t blocks = (total + tpb - 1) / tpb;
   if (blocks > 148 * 32) blocks = 148 * 32;               // grid-stride: 32 CTAs per SM keep the store queues full
-  expand_time_batch_kernel<R><<<(unsigned)blocks, tpb, 0, st>>>(src, dst, count, total);
-  if (nl) ++*nl;
-  return cudaGetLastError() == cudaSuccess ? DMPC_OK : DMPC_ERR_CUDA;
+  return launch(expand_time_batch_kernel<R>, (unsigned)blocks, tpb, 0, st, nl, src, dst, count, total);
 }
 
+template bool adjoint_fused_available<DMPC_REAL>(int, int);
 template int launch_expand_time_batch<DMPC_REAL>(const DMPC_REAL*, DMPC_REAL*, int, size_t, cudaStream_t, long long*);
-template int launch_reduce_partials<DMPC_REAL>(const DMPC_REAL*, int, int, DMPC_REAL*, cudaStream_t, long long*);
 template int launch_lqr_rollout_32_8<DMPC_REAL>(const LqrParams<DMPC_REAL>&, cudaStream_t, long long*);
 template int launch_lqr_solve<DMPC_REAL>(const LqrParams<DMPC_REAL>&, cudaStream_t, long long*);
-template int launch_lqr_dtau<DMPC_REAL>(const DtauParams<DMPC_REAL>&, cudaStream_t, long long*);
-template int launch_adjoint_fused<DMPC_REAL>(const DtauParams<DMPC_REAL>&, const AdjFusedParams<DMPC_REAL>&, int, cudaStream_t, long long*);
-template int launch_adjoint_out<DMPC_REAL>(const AdjOutParams<DMPC_REAL>&, cudaStream_t, long long*);
+template int launch_lqr_adjoint<DMPC_REAL>(const DtauParams<DMPC_REAL>&, const AdjFusedParams<DMPC_REAL>&,
+                                           const AdjOutParams<DMPC_REAL>&, int, DMPC_REAL*, cudaStream_t, long long*, const char**);
+template int launch_adjoint_out<DMPC_REAL>(const AdjOutParams<DMPC_REAL>&, DMPC_REAL*, cudaStream_t, long long*, const char**);
 
 }  // namespace dmpc

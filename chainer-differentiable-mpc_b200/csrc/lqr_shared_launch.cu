@@ -9,10 +9,8 @@ namespace dmpc {
 
 template <typename K, typename P>
 static int shared_launch(K kernel, const P& p, size_t smem, cudaStream_t st, long long* nl) {
-  if (cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return DMPC_ERR_CUDA;
-  kernel<<<(p.B + p.NB - 1) / p.NB, kSharedThreads, smem, st>>>(p);
-  if (nl) ++*nl;
-  return cudaGetLastError() == cudaSuccess ? DMPC_OK : DMPC_ERR_CUDA;
+  if (set_smem(kernel, smem)) return DMPC_ERR_CUDA;
+  return launch(kernel, (p.B + p.NB - 1) / p.NB, kSharedThreads, smem, st, nl, p);
 }
 
 template <typename R>
@@ -29,9 +27,7 @@ int launch_lqr_shared_adj(const LqrSharedParams<R>& p, cudaStream_t st, long lon
   if (rc) return rc;
   const size_t total = shared_reduce_outputs(p);
   const int tpb = 256;
-  lqr_shared_reduce_kernel<R><<<(unsigned)((total + tpb - 1) / tpb), tpb, 0, st>>>(p, (p.B + p.NB - 1) / p.NB);
-  if (nl) ++*nl;
-  return cudaGetLastError() == cudaSuccess ? DMPC_OK : DMPC_ERR_CUDA;
+  return launch(lqr_shared_reduce_kernel<R>, (unsigned)((total + tpb - 1) / tpb), tpb, 0, st, nl, p, (p.B + p.NB - 1) / p.NB);
 }
 
 template int launch_lqr_shared_fwd<DMPC_REAL>(const LqrSharedParams<DMPC_REAL>&, cudaStream_t, long long*);

@@ -202,18 +202,14 @@ template <>
 int launch_active_mask<Rr>(const Rr* u, const Rr* lo, const Rr* hi, unsigned char* out, size_t count, cudaStream_t st,
                            long long* nl) {
   const int tpb = 256;
-  active_mask_kernel<Rr><<<(unsigned)((count + tpb - 1) / tpb), tpb, 0, st>>>(u, lo, hi, out, count);
-  if (nl) ++*nl;
-  return cudaGetLastError() == cudaSuccess ? DMPC_OK : DMPC_ERR_CUDA;
+  return launch(active_mask_kernel<Rr>, (unsigned)((count + tpb - 1) / tpb), tpb, 0, st, nl, u, lo, hi, out, count);
 }
 
 template <>
 int launch_traj<Rr>(const TrajParams<Rr>& p, cudaStream_t st, long long* nl) {
   if (p.n + p.m > 64) return launch_traj_large<Rr>(p, st, nl);     // traj_kernel keeps [x; u] in registers
   const int tpb = 64;
-  traj_kernel<Rr, 64><<<(p.B + tpb - 1) / tpb, tpb, 0, st>>>(p);
-  if (nl) ++*nl;
-  return cudaGetLastError() == cudaSuccess ? DMPC_OK : DMPC_ERR_CUDA;
+  return launch(traj_kernel<Rr, 64>, (p.B + tpb - 1) / tpb, tpb, 0, st, nl, p);
 }
 
 }  // namespace dmpc

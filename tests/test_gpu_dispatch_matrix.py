@@ -1,4 +1,4 @@
-"""GPU: every kernel the launchers (csrc/lqr_launch.cu, csrc/mpc_launch.cu, csrc/capi.cu) can select, against the fp64 oracle.
+"""GPU: every kernel the launchers (csrc/lqr_launch.cu, csrc/mpc_launch.cu) can select, against the fp64 oracle.
 
 Each case names the kernel it is meant to reach and proves it: the call runs under torch.profiler (CUDA activity), which
 records every kernel of the process, including the ones launched through the C ABI, and the case asserts a substring of
@@ -18,9 +18,9 @@ Launcher branch -> case that reaches it (kernel asserted from the profiler trace
                       thread-per-element (2,1) (3,1) (4,2)  default  *-pathtpe*, epw8 / epw16 / epw_auto
                       specialised group <N,M,G>             lqr_group, active at (32,8), mpcb at (32,8), *-pathfused*
                       runtime group G = 8 / 16 / 32 / 256   default  lqr-*-pathgroup* (m > n included), active, mpcb
-  launch_lqr_dtau     tpe / specialised / runtime G         as above (adjoint of every lqr case)
-  launch_adjoint_out  tpe (full) / specialised / runtime    as above; reduced: *-reduced*; adj_group
-  launch_adjoint_fused + adjoint_fused_available            (32,8) full and reduced: *-pathdmma*, *-pathfused*; off: adj_unfused
+  launch_lqr_adjoint  lqr_dtau: tpe / specialised / runtime G   as above (adjoint of every lqr case)
+                      adjoint_out: tpe (full) / specialised / runtime   as above; reduced: *-reduced*; adj_group
+                      two sweeps where adjoint_fused_available  (32,8) full and reduced: *-pathdmma*, *-pathfused*; off: adj_unfused
   launch_mpc_forward  tpe (m = 1) / specialised / runtime   default mpcf cases, mpc_group (linear and pendulum <3,1,4>)
   launch_mpc_tpe      4 lanes with / without stash, 1 lane   default mpcf (stash threshold asserted), mpc_no_spec, mpc_no_stash
 MPC step forward contract (mpcf keys, every kernel above in both couplings where the launcher has them):
